@@ -23,6 +23,11 @@ every number.
 --deliver (config 2, end-to-end leg): full (Q,3,224,224 fp32, the reference's return value) | channel_mean
   ((Q,224,224): what evaluation.py:134,411,503 reduces every heat-map to) | fp16.
 
+--dump-outputs DIR: after the timed steps, write what the timed call returned in its last step as DIR/<name>.npy
+  (float32; float64 and integer arrays as float64), at most 64,000,000 bytes in all: an array too large for its share is
+  written as a fixed, seeded sample of its elements plus the sampled flat positions (<name>_index.npy).  Inputs are seeded,
+  so two builds run with the same arguments can be compared file by file.  Under torchrun: rank 0's shard.
+
 Without --config the N = 1 run also measures configs 3, 4, 5, the mixed / fp32-accurate modes, the ResNet101 variant and
 the gradient-family explainers of config 2 briefly and attaches them under "also" (each with its own parity figures), so that one driver run covers every configuration.
 Under torchrun (N > 1) each rank works on its own shard (requests are independent: no collective on the data path;
@@ -36,6 +41,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True          # bench.py writes nothing into the tree, not even __pycache__ of what it imports
 ROOT = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.join(ROOT, "lrp-imagecaptioning-pytorch_b200")
 for p in (PKG, os.path.join(ROOT, "tests")):
@@ -76,7 +82,11 @@ def parse(argv=None):
                     help="run 1 warm-up + 1 step and exit (the command line captured under ncu for profiles/)")
     ap.add_argument("--cpu-words", type=int, default=19, help="words per image of the bounded CPU sample")
     ap.add_argument("--cpu-images", type=int, default=4, help="images of the bounded CPU sample (about 10-30 s of host work)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (at most 64 MB in all)")
     a = ap.parse_args(argv)
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     a.also = (a.config == 0) and not a.no_also
     if a.config == 0:
         a.config = 2
@@ -202,6 +212,26 @@ def bind_to_gpu_numa_node(index):
         return sorted(os.sched_getaffinity(0))
     except Exception as e:      # affinity is an optimisation only
         return f"unavailable: {e!r}"
+
+
+def write_outputs(dirname, arrays, budget=64_000_000, seed=0):
+    """Writes each tensor of `arrays` (name -> tensor) as <dirname>/<name>.npy: float64 and integer tensors as float64
+    (integers are exact below 2**53), the others as float32.  The files, .npy headers included, stay within `budget`
+    bytes: every array gets an equal share; one larger than its share is written as the elements at a fixed, seeded set
+    of flat positions, which go to <name>_index.npy (float64), so that the same arguments always select the same elements."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    share = budget // len(arrays) - 1024                # 1024: room for the headers of the array's two files
+    for name, t in arrays.items():
+        t = t.detach()
+        t = t.double() if t.dtype == torch.float64 or not t.is_floating_point() else t.float()
+        flat = t.reshape(-1)
+        if flat.numel() * flat.element_size() > share:
+            k = share // (flat.element_size() + 8)
+            idx = torch.unique(torch.randint(0, flat.numel(), (k,), generator=torch.Generator().manual_seed(seed)))
+            np.save(os.path.join(dirname, name + "_index.npy"), idx.double().numpy())
+            t = flat[idx.to(flat.device)]
+        np.save(os.path.join(dirname, name + ".npy"), t.cpu().numpy())
 
 
 def _oracle():
@@ -487,6 +517,8 @@ def run_config2(args, ctx, brief=False):
     sampler = ClockSampler(ctx.local) if rank == 0 else None
     ms = ctx.timed(lambda: step(imgs_d, toks_d), steps)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:          # before the end-to-end leg overwrites `heat`
+        write_outputs(args.dump_outputs, {"heatmaps": last["out"][0], "word_relevance": last["out"][1]})
     # the chain's share of the TIMED (graph-replayed) step: chain_ms_in_step = ms_per_step - (the other phases)
     others = phase_ms["encoder_forward_gains"] + phase_ms["explainer_forward"] + phase_ms["decoder_relevance"]
     chain_in_step = max(ms / steps - others, phase_ms["encoder_relevance_chain"])
@@ -707,6 +739,12 @@ def run_config3(args, ctx, brief=False):
     ms = ctx.timed(step, steps)
     clocks = sampler.stop() if sampler else None
     calls = {k: _lib.CALLS[k] - calls0.get(k, 0) for k in _lib.CALLS}
+    if args.dump_outputs and rank == 0:
+        r_feat, r_words, req_img, req_t, caps = last["r"]
+        cap_len = max(len(c) for c in caps)
+        captions = torch.tensor([[int(w) for w in c] + [-1] * (cap_len - len(c)) for c in caps])  # -1: past the end
+        write_outputs(args.dump_outputs, {"feature_relevance": r_feat, "word_relevance": r_words,
+                                          "request_image": req_img, "request_word": req_t, "captions": captions})
     for _ in range(2):
         step_e2e()
     ms_e2e = ctx.timed(step_e2e, steps)
@@ -831,6 +869,8 @@ def run_config4(args, ctx, brief=False):
     ms = ctx.timed(step, steps)
     clocks = sampler.stop() if sampler else None
     calls = {k: _lib.CALLS[k] - calls0.get(k, 0) for k in _lib.CALLS}
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, {"heatmaps": last["rel"]})
     for _ in range(2):
         step_e2e()
     ms_e2e = ctx.timed(step_e2e, steps)
@@ -896,6 +936,7 @@ def build_config5(args, dev, seed, B):
     import synth
     from models import gridTDmodel as G
     V, H, E, T = args.vocab, 512, 512, 20
+    torch.manual_seed(seed)                     # the training step's dropout masks: the same in every run
     model = G.GridTDModel(E, H, V, "vgg16")
     model.load_state_dict(synth.gridtd_decoder_state(1, V, H, E), strict=False)       # same weights on every rank
     model.img_encoder.encoder.load_state_dict(synth.vgg_state(2))
@@ -924,9 +965,10 @@ def run_config5(args, ctx, brief=False):
     imgs_h, caps_h = imgs.pin_memory(), caps.pin_memory()
     imgs_d, caps_d = imgs_h.to(dev), caps_h.to(dev)
     loss_h = torch.empty(3).pin_memory()
+    last = {}
 
     def step():
-        st.step(imgs_d, caps_d, caplens)
+        last["loss"] = st.step(imgs_d, caps_d, caplens)
 
     def step_e2e():
         l = st.step(imgs_h.to(dev, non_blocking=True), caps_h.to(dev, non_blocking=True), caplens)
@@ -940,6 +982,8 @@ def run_config5(args, ctx, brief=False):
     ms = ctx.timed(step, steps)
     clocks = sampler.stop() if sampler else None
     calls = {k: _lib.CALLS[k] - calls0.get(k, 0) for k in _lib.CALLS}
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, {"losses": torch.stack(last["loss"])})     # (total, cross-entropy, LRP-weighted)
     ms_e2e = ctx.timed(step_e2e, steps)
     ms_nosync = None
     if st.distributed:
@@ -1162,10 +1206,12 @@ def run_gradient(args, ctx, brief=True):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        heat, _ = pipe.explain(imgs_d, toks_d, out=heat)
+        heat, r_words = pipe.explain(imgs_d, toks_d, out=heat)
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / args.steps
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {"heatmaps": heat, "word_relevance": r_words})
     out = {"metric": method + "_explanations_per_s", "value": round(Q / ms * 1e3, 1), "unit": UNIT, "ms_per_step": round(ms, 3),
            "dtype": "bf16" if args.precision == "bf16" else "bf16x3", "config": {"workload": f"config2 with the {method} "
            f"explainer: {B} images x {T} words, VGG16 224x224, precision {args.precision}, inputs resident in HBM"}}
@@ -1212,10 +1258,11 @@ def run_ours(args):
                                  ("config2_gradient_bf16", 2, dict(method="gradient", precision="bf16", steps=4)),
                                  ("config2_guided_bf16", 2, dict(method="guided", precision="bf16", steps=4))):
             a2 = argparse.Namespace(**vars(args))
-            a2.config, a2.also, a2.warmup = cfg, False, 3
+            a2.config, a2.also, a2.warmup, a2.dump_outputs = cfg, False, 3, None
             a2.images = {2: 64, 3: 64, 4: 512, 5: 128}[cfg]
             for k, v in extra.items():
                 setattr(a2, k, v)
+            a2.steps = min(a2.steps, args.steps)
             try:
                 torch.cuda.empty_cache()
                 r = (run_gradient if name.startswith("config2_g") else RUNNERS[cfg])(a2, ctx, brief=True)

@@ -1,16 +1,24 @@
-"""CPU, build container only: the oracle against the UNMODIFIED reference executed live (oracle/check_vs_reference.py,
-fresh seeds).  Skips itself where /root/reference is not mounted (the GPU box) — there the committed fixtures in
-tests/golden, generated by the same shim (oracle/make_golden.py), are the pin."""
+"""CPU: the oracle against the UNMODIFIED original project on the cases of oracle/check_vs_reference.py (fresh seeds and
+shapes that the fixtures of oracle/make_golden.py do not use).  Every run compares the oracle with the expected outputs
+stored in tests/golden/live_check.npz; where ref_shim finds the original, the script also runs it live and checks both
+the oracle and the stored outputs against it."""
 import os
 import subprocess
 import sys
 
 import pytest
 
+import check_vs_reference as C
+import ref_shim
 from conftest import ROOT
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/LRPtools"), reason="/root/reference is not mounted")
+def test_oracle_matches_stored_live_check_outputs():
+    inp, expected, source = C.load_fixture()
+    C.compare(C.oracle_outputs(inp), expected, f"oracle vs stored ({source})")
+
+
+@pytest.mark.skipif(not ref_shim.reference_available(), reason="the original project is not available to ref_shim")
 def test_oracle_matches_live_reference():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "oracle", "check_vs_reference.py")], capture_output=True,
                        text=True, timeout=600)
