@@ -1939,15 +1939,9 @@ static int make_map_out(CUtensorMap* map, const void* base, uint64_t rows, uint6
 
 template <int EPI>
 static int launch_tc(const CUtensorMap& ma, const CUtensorMap& mb, const TcParams& p, int grid, cudaStream_t st) {
-  static std::once_flag once;
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [] {
-    attr_err = cudaFuncSetAttribute(tc_conv_kernel<EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_BYTES);
-  });
-  if (attr_err != cudaSuccess) {
-    set_error("cudaFuncSetAttribute(max dynamic smem) failed: %s", cudaGetErrorString(attr_err));
-    return LRPX_E_CUDA;
-  }
+  static std::atomic<uint64_t> attr_done;
+  const int rc = ensure_smem_attr(tc_conv_kernel<EPI>, TC_SMEM_BYTES, attr_done);
+  if (rc != LRPX_OK) return rc;
   tc_conv_kernel<EPI><<<grid, TC_THREADS, TC_SMEM_BYTES, st>>>(ma, mb, p);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) {
@@ -1978,15 +1972,9 @@ static int launch_tc_slab(const CUtensorMap& ma0, const CUtensorMap& ma1, const 
 template <int EPI, bool PAIR>
 static int launch_tc_slab_impl(const CUtensorMap& ma0, const CUtensorMap& ma1, const CUtensorMap& mb, const CUtensorMap& mbh,
                                const CUtensorMap& mo, const TcParams& p, int grid, cudaStream_t st) {
-  static std::once_flag once;
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [] {
-    attr_err = cudaFuncSetAttribute(tc_conv_slab_kernel<EPI, PAIR>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_BYTES);
-  });
-  if (attr_err != cudaSuccess) {
-    set_error("cudaFuncSetAttribute(max dynamic smem) failed: %s", cudaGetErrorString(attr_err));
-    return LRPX_E_CUDA;
-  }
+  static std::atomic<uint64_t> attr_done;
+  const int rc = ensure_smem_attr(tc_conv_slab_kernel<EPI, PAIR>, TC_SMEM_BYTES, attr_done);
+  if (rc != LRPX_OK) return rc;
   if (p.cluster == 2) {
     // GPCs with an odd number of SMs cannot host a pair on their last SM: a persistent grid must not exceed the
     // number of clusters that are co-resident, or the left-over pair would run after everyone else

@@ -31,7 +31,10 @@ __global__ void __launch_bounds__(256) sgemm_nn_kernel(const float* __restrict__
   __shared__ float As[TBK][TBM + 4];
   __shared__ float Bs[TBK][TBN];
   const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
-  const int m0 = blockIdx.y * TBM, n0 = blockIdx.x * TBN;
+  // 1-D grid, column tiles fastest: M / 64 row tiles exceed the 65 535 blocks of a grid's y dimension at Q * P rows
+  const int ntn = (N + TBN - 1) / TBN;
+  const int mt = blockIdx.x / ntn;
+  const int m0 = mt * TBM, n0 = (blockIdx.x - mt * ntn) * TBN;
   float acc[4][4] = {};
   for (int k0 = 0; k0 < K; k0 += TBK) {
 #pragma unroll
@@ -98,7 +101,7 @@ __global__ void __launch_bounds__(256) sgemm_nn_kernel(const float* __restrict__
 template <int EPI>
 static int sgemm(const float* A, const float* B, float* C, int M, int N, int K, const GemmEpi& e, cudaStream_t st) {
   if (M == 0) return LRPX_OK;
-  dim3 grid(ceil_div(N, 64), ceil_div(M, 64));
+  const unsigned grid = (unsigned)ceil_div(N, 64) * (unsigned)ceil_div(M, 64);
   sgemm_nn_kernel<EPI><<<grid, 256, 0, st>>>(A, B, C, M, N, K, K, N, N, e);
   cudaError_t err = cudaGetLastError();
   if (err != cudaSuccess) {

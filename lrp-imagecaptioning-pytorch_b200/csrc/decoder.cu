@@ -160,7 +160,7 @@ __global__ void grid_avg_kernel(lrpx_gridtd_args a, GridWs w) {
 }
 // wproj[q][p][h] = A * (sum_i alpha_i[p] * uctx_i[h]) / stab(A_pre)     (:1091-1095 then :1125-1128)
 __global__ void grid_attn_kernel(lrpx_gridtd_args a, GridWs w) {
-  int q = blockIdx.y, p = blockIdx.x;
+  const int q = blockIdx.x / a.P, p = blockIdx.x - q * a.P;          // one block per (request, pixel)
   int b = a.req_img[q], t = a.req_t[q];
   const float* al = a.alpha + (size_t)b * a.T * a.P + p;
   size_t o0 = ((size_t)b * a.P + p) * a.H;
@@ -431,7 +431,7 @@ __global__ void aoa_post_kernel(lrpx_aoa_args a, AoaWs w, int i) {
 // wval = r_val / stab(value), r_val = value * alpha[head][p] * uval   (:1112-1113, :1141-1144)
 // addq = r_glob / stab(glob) / P                                     (:1136-1139)
 __global__ void aoa_val_kernel(lrpx_aoa_args a, AoaWs w) {
-  int q = blockIdx.y, p = blockIdx.x;
+  const int q = blockIdx.x / a.P, p = blockIdx.x - q * a.P;          // one block per (request, pixel)
   int b = a.req_img[q], t = a.req_t[q], head = a.req_head[q];
   float al = a.alpha[(((size_t)b * a.T + t) * a.num_head + head) * a.P + p];
   size_t o0 = ((size_t)b * a.P + p) * a.H;
@@ -774,17 +774,17 @@ int lrpx_gridtd_decoder_lrp_f32(const lrpx_gridtd_args* a, void* workspace, size
       const size_t n4 = (size_t)a->B * a->P * H / 4;
       grid_attn_gain_kernel<<<(unsigned)((n4 + 255) / 256 < 4096 ? (n4 + 255) / 256 : 4096), 256, 0, st>>>(a->A, a->A_pre, w.gA, n4);
     }
-    static bool attr_done = false;
-    if (!attr_done) {
-      cudaFuncSetAttribute(grid_attn_rows_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
-      cudaFuncSetAttribute(grid_attn_rows_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
-      attr_done = true;
+    static std::atomic<uint64_t> attr_done[2];
+    if (w3_proj) {
+      RUN(ensure_smem_attr(grid_attn_rows_kernel<true>, 160 * 1024, attr_done[1]));
+      grid_attn_rows_kernel<true><<<Q, at, att_smem, st>>>(*a, w);
+    } else {
+      RUN(ensure_smem_attr(grid_attn_rows_kernel<false>, 160 * 1024, attr_done[0]));
+      grid_attn_rows_kernel<false><<<Q, at, att_smem, st>>>(*a, w);
     }
-    if (w3_proj) grid_attn_rows_kernel<true><<<Q, at, att_smem, st>>>(*a, w);
-    else grid_attn_rows_kernel<false><<<Q, at, att_smem, st>>>(*a, w);
     RUN(gemm_any<GE_FEAT>(w.wproj, a->W_proj, w3_proj, w.a3, a->r_feat, Q * a->P, a->C, H, fe, st, w3_proj != nullptr));
   } else {
-    grid_attn_kernel<<<dim3(a->P, Q), nt, 0, st>>>(*a, w);
+    grid_attn_kernel<<<(unsigned)Q * a->P, nt, 0, st>>>(*a, w);
     RUN(gemm_any<GE_FEAT>(w.wproj, a->W_proj, w3_proj, w.a3, a->r_feat, Q * a->P, a->C, H, fe, st));
   }
   words_norm_kernel<<<Q, 32, 0, st>>>(a->r_words, a->req_t, T);
@@ -829,7 +829,7 @@ int lrpx_aoa_decoder_lrp_f32(const lrpx_aoa_args* a, void* workspace, size_t wor
     RUN(gemm_any<GE_STORE>(w.u, a->W_g, w3_g, w.a3, w.v, Q, E + 2 * H, H, none, st));
     aoa_post_kernel<<<Q, 256, 0, st>>>(*a, w, i);
   }
-  aoa_val_kernel<<<dim3(a->P, Q), nt, 0, st>>>(*a, w);
+  aoa_val_kernel<<<(unsigned)Q * a->P, nt, 0, st>>>(*a, w);
   GemmEpi pe{a->A, a->A_pre, w.addq, a->req_img, a->P};
   RUN(gemm_any<GE_AOA_PROJ>(w.wval, a->W_v, w3_v, w.a3, w.w2, Q * a->P, H, H, pe, st));
   GemmEpi fe{a->feat, nullptr, nullptr, a->req_img, a->P};

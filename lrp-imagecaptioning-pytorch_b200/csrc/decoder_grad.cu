@@ -17,6 +17,8 @@
 #include "lrpx_common.cuh"
 #include "dec_gemm.cuh"
 
+#include <algorithm>
+
 namespace lrpx {
 
 #define RUN(x)                         \
@@ -219,7 +221,7 @@ template <bool SPLIT>
 __global__ void ggrad_attn_slow_kernel(const float* __restrict__ alpha, const float* __restrict__ uctx,
                                        const int32_t* __restrict__ req_img, const int32_t* __restrict__ req_t,
                                        float* __restrict__ dproj, __nv_bfloat16* __restrict__ a3, int T, int P, int H) {
-  const int q = blockIdx.y, p = blockIdx.x;
+  const int q = blockIdx.x / P, p = blockIdx.x - q * P;            // one block per (request, pixel)
   const int b = req_img[q], t = req_t[q];
   const float* al = alpha + (size_t)b * T * P + p;
   for (int h = threadIdx.x; h < H; h += blockDim.x) {
@@ -250,8 +252,10 @@ static size_t ggrad_carve(const lrpx_gridtd_grad_args* a, float* base, GGradWs* 
   t.dproj = take(Q * a->P * H);
   if (a->flags & LRPX_DEC_TC_GEMM) {
     auto take16 = [&](size_t n) { return reinterpret_cast<__nv_bfloat16*>(take((n + 1) / 2)); };
-    const size_t big = Q * a->P * 2 * H, small = Q * 2 * E;
-    t.a3 = take16(big > small ? big : small);
+    // a3 takes the split operand of every GEMM but the fused step GEMMs: the projector (Q*P x H), the global
+    // projection (Q x E) and, when the step kernels do not split (fused_split off), the step GEMMs (Q x 4H)
+    const size_t kmax = std::max({(size_t)a->P * H, E, 4 * H});
+    t.a3 = take16(Q * 2 * kmax);
     t.a3u = take16(Q * 2 * 4 * H);
     t.w3_2 = take16(3 * H * 3 * 4 * H);
     t.w3_1 = take16((H + 2 * E) * 3 * 4 * H);
@@ -295,7 +299,7 @@ __global__ void agrad_init_kernel(lrpx_aoa_grad_args a, AGradWs w) {
 // d_h[t+1] += d_B @ W_gate  (:1470);  d_value[p] = d_context (.) alpha[head][p] on the chosen head (gradient_mha :1415-1433)
 __global__ void agrad_ctx_kernel(lrpx_aoa_grad_args a, AGradWs w, const float* __restrict__ v_ctx,
                                  const float* __restrict__ v_gate, __nv_bfloat16* a3) {
-  const int q = blockIdx.y, p = blockIdx.x, H = a.H;
+  const int q = blockIdx.x / a.P, p = blockIdx.x - q * a.P, H = a.H;     // one block per (request, pixel)
   const int b = a.req_img[q], t = a.req_t[q], head = a.req_head[q];
   const int dk = H / a.num_head;
   const float al = a.alpha[(((size_t)b * a.T + t) * a.num_head + head) * a.P + p];
@@ -429,7 +433,7 @@ __global__ void dgrad_post_kernel(lrpx_adaptive_grad_args a, DGradWs w, int i) {
 // d_feat[q][p][c] = (d_glob @ W_glob)[c] / P + alpha_t[p] * (d_context @ W_proj)[c]     (:1011-1015)
 __global__ void dgrad_out_kernel(lrpx_adaptive_grad_args a, const float* __restrict__ avg /* (Q,C) */,
                                  const float* __restrict__ y /* (Q,C) */) {
-  const int q = blockIdx.y, p = blockIdx.x;
+  const int q = blockIdx.x / a.P, p = blockIdx.x - q * a.P;          // one block per (request, pixel)
   const int b = a.req_img[q], t = a.req_t[q];
   const float al = a.alpha[((size_t)b * a.T + t) * a.P + p];
   float* dst = a.d_feat + ((size_t)q * a.P + p) * a.C;
@@ -453,7 +457,9 @@ static size_t dgrad_carve(const lrpx_adaptive_grad_args* a, float* base, DGradWs
   t.y = take(Q * C);
   if (a->flags & LRPX_DEC_TC_GEMM) {
     auto take16 = [&](size_t n) { return reinterpret_cast<__nv_bfloat16*>(take((n + 1) / 2)); };
-    t.a3 = take16(Q * 2 * 4 * H);
+    // a3 takes the split operand of every GEMM: the step GEMM (Q x 4H), the global projection (Q x E), the projector
+    // (Q x H)
+    t.a3 = take16(Q * 2 * std::max({4 * H, E, H}));
     t.w3_g = take16((2 * E + H) * 3 * 4 * H);
     t.w3_glob = take16(C * 3 * E);
     t.w3_proj = take16(C * 3 * H);
@@ -577,18 +583,19 @@ int lrpx_gridtd_decoder_grad_f32(const lrpx_gridtd_grad_args* a, void* workspace
   ggrad_avg_kernel<<<Q, 128, 0, st>>>(*a, w);
   const size_t att_smem = (size_t)T * (((P + 3) & ~3) + H) * sizeof(float);
   if (att_smem <= 200 * 1024) {
-    static bool attr_done = false;
-    if (!attr_done) {
-      cudaFuncSetAttribute(ggrad_attn_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-      cudaFuncSetAttribute(ggrad_attn_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-      attr_done = true;
-    }
+    static std::atomic<uint64_t> attr_done[2];
     const int at = H / 4 >= 512 ? 512 : ((H / 4 + 31) & ~31);
-    if (w3_proj) ggrad_attn_kernel<true><<<Q, at, att_smem, st>>>(a->alpha, w.uctx, a->req_img, a->req_t, w.dproj, w.a3, T, P, H);
-    else ggrad_attn_kernel<false><<<Q, at, att_smem, st>>>(a->alpha, w.uctx, a->req_img, a->req_t, w.dproj, w.a3, T, P, H);
+    if (w3_proj) {
+      RUN(ensure_smem_attr(ggrad_attn_kernel<true>, 200 * 1024, attr_done[1]));
+      ggrad_attn_kernel<true><<<Q, at, att_smem, st>>>(a->alpha, w.uctx, a->req_img, a->req_t, w.dproj, w.a3, T, P, H);
+    } else {
+      RUN(ensure_smem_attr(ggrad_attn_kernel<false>, 200 * 1024, attr_done[0]));
+      ggrad_attn_kernel<false><<<Q, at, att_smem, st>>>(a->alpha, w.uctx, a->req_img, a->req_t, w.dproj, w.a3, T, P, H);
+    }
   } else {          // long captions x wide hidden state: alpha and d_context rows do not fit one block's shared memory
-    if (w3_proj) ggrad_attn_slow_kernel<true><<<dim3(P, Q), nt, 0, st>>>(a->alpha, w.uctx, a->req_img, a->req_t, w.dproj, w.a3, T, P, H);
-    else ggrad_attn_slow_kernel<false><<<dim3(P, Q), nt, 0, st>>>(a->alpha, w.uctx, a->req_img, a->req_t, w.dproj, w.a3, T, P, H);
+    const unsigned qp = (unsigned)Q * P;
+    if (w3_proj) ggrad_attn_slow_kernel<true><<<qp, nt, 0, st>>>(a->alpha, w.uctx, a->req_img, a->req_t, w.dproj, w.a3, T, P, H);
+    else ggrad_attn_slow_kernel<false><<<qp, nt, 0, st>>>(a->alpha, w.uctx, a->req_img, a->req_t, w.dproj, w.a3, T, P, H);
   }
   GemmEpi fe{a->feat, nullptr, w.coefavg, a->req_img, P};
   if (guided) RUN(gemm_any<GE_ADD_MASK>(w.dproj, a->W_proj, w3_proj, w.a3, a->d_feat, Q * P, C, H, fe, st, w3_proj != nullptr));
@@ -632,7 +639,7 @@ int lrpx_aoa_decoder_grad_f32(const lrpx_aoa_grad_args* a, void* workspace, size
   float* v_gate = w.v + (size_t)Q * H;      // (Q,H)   (v holds Q*(E+2H) floats)
   RUN(gemm_any<GE_STORE>(w.uA, a->W_aoa, w3_aoa, w.a3, v_ctx, Q, H, H, none, st));
   RUN(gemm_any<GE_STORE>(w.uB, a->W_gate, w3_gate, w.a3, v_gate, Q, H, H, none, st));
-  agrad_ctx_kernel<<<dim3(P, Q), nt, 0, st>>>(*a, w, v_ctx, v_gate, w3_v ? w.a3 : nullptr);
+  agrad_ctx_kernel<<<(unsigned)Q * P, nt, 0, st>>>(*a, w, v_ctx, v_gate, w3_v ? w.a3 : nullptr);
   // the value projection's input gradient is formed first: its split operand occupies a3 until that GEMM has run
   GemmEpi ge{nullptr, nullptr, w.d_glob, a->req_img, P};
   // d_glob is known only after the LSTM chain: run the chain on the CUDA-core/tensor-core step GEMMs with their own
@@ -683,7 +690,7 @@ int lrpx_adaptive_decoder_grad_f32(const lrpx_adaptive_grad_args* a, void* works
   }
   RUN(gemm_any<GE_STORE>(w.d_glob, a->W_glob, w3_glob, w.a3, w.v, Q, C, E, none, st));      // d_average_img_feature
   RUN(gemm_any<GE_STORE>(w.dctx, a->W_proj, w3_proj, w.a3, w.y, Q, C, H, none, st));        // d_context @ W_proj
-  dgrad_out_kernel<<<dim3(a->P, Q), 256, 0, st>>>(*a, w.v, w.y);
+  dgrad_out_kernel<<<(unsigned)Q * a->P, 256, 0, st>>>(*a, w.v, w.y);
   words_norm_kernel<<<Q, 32, 0, st>>>(a->r_words, a->req_t, T);
   LRPX_CHECK_LAUNCH();
   return LRPX_OK;

@@ -399,22 +399,25 @@ extern "C" int lrpx_lstm_step_f32(const lrpx_lstm_step_args* a, void* stream) {
   // barriers, one 87 KB chunk of look-ahead).  LRPX_LSTM_KC = 64 | 128 select the other variants.
   static const int kc = [] { const char* e = getenv("LRPX_LSTM_KC"); const int v = e ? atoi(e) : 256;
                              return (v == 64 || v == 128) ? v : 256; }();
-  auto launch = [&](auto kernel, int KC, int STAGES, bool* done) {
+  auto launch = [&](auto kernel, int KC, int STAGES, std::atomic<uint64_t>& done) {
     const size_t smem = (size_t)(STAGES * (LS_ROWS * (KC + 4) + a->G * LS_U * (KC + 4)) + LS_SLICES * 32 * LS_RPT * a->G) * sizeof(float);
-    if (!*done) { cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); *done = true; }
-    kernel<<<a->H / LS_U, 256, smem, st>>>(*a);
+    const int rc = ensure_smem_attr(kernel, (int)smem, done);
+    if (rc == LRPX_OK) kernel<<<a->H / LS_U, 256, smem, st>>>(*a);
+    return rc;
   };
-  static bool attr_done[6] = {false, false, false, false, false, false};
+  static std::atomic<uint64_t> attr_done[6];
+  int rc;
   if (kc == 128) {
-    if (a->G == 5) launch(lstm_step_kernel<5, 128, 3>, 128, 3, &attr_done[0]);
-    else launch(lstm_step_kernel<4, 128, 3>, 128, 3, &attr_done[1]);
+    if (a->G == 5) rc = launch(lstm_step_kernel<5, 128, 3>, 128, 3, attr_done[0]);
+    else rc = launch(lstm_step_kernel<4, 128, 3>, 128, 3, attr_done[1]);
   } else if (kc == 256) {
-    if (a->G == 5) launch(lstm_step_kernel<5, 256, 2>, 256, 2, &attr_done[4]);
-    else launch(lstm_step_kernel<4, 256, 2>, 256, 2, &attr_done[5]);
+    if (a->G == 5) rc = launch(lstm_step_kernel<5, 256, 2>, 256, 2, attr_done[4]);
+    else rc = launch(lstm_step_kernel<4, 256, 2>, 256, 2, attr_done[5]);
   } else {
-    if (a->G == 5) launch(lstm_step_kernel<5, 64, 4>, 64, 4, &attr_done[2]);
-    else launch(lstm_step_kernel<4, 64, 4>, 64, 4, &attr_done[3]);
+    if (a->G == 5) rc = launch(lstm_step_kernel<5, 64, 4>, 64, 4, attr_done[2]);
+    else rc = launch(lstm_step_kernel<4, 64, 4>, 64, 4, attr_done[3]);
   }
+  if (rc != LRPX_OK) return rc;
   LRPX_CHECK_LAUNCH();
   return LRPX_OK;
 }

@@ -5,6 +5,7 @@
 #include <stdint.h>
 #include <stdio.h>
 #include <stdarg.h>
+#include <atomic>
 #include "../../include/lrpx.h"
 
 namespace lrpx {
@@ -41,5 +42,23 @@ __device__ __forceinline__ float stab(float z) {
 
 static inline int ceil_div(long long a, long long b) { return (int)((a + b - 1) / b); }
 static inline cudaStream_t as_stream(void* s) { return reinterpret_cast<cudaStream_t>(s); }
+
+// Dynamic shared memory above 48 KB needs cudaFuncSetAttribute, which applies to the CURRENT device only: set it once
+// per (kernel, device).  `done` is the caller's static bit set of the devices already set up for `kernel` (devices
+// from 64 on are set up on every call).
+template <class Kernel>
+static int ensure_smem_attr(Kernel kernel, int bytes, std::atomic<uint64_t>& done) {
+  int dev = 0;
+  cudaError_t e = cudaGetDevice(&dev);
+  const uint64_t bit = (e == cudaSuccess && dev < 64) ? (uint64_t)1 << dev : 0;
+  if (bit && (done.load(std::memory_order_acquire) & bit)) return LRPX_OK;
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+  if (e != cudaSuccess) {
+    set_error("cudaFuncSetAttribute(max dynamic shared memory %d) failed: %s", bytes, cudaGetErrorString(e));
+    return LRPX_E_CUDA;
+  }
+  done.fetch_or(bit, std::memory_order_release);
+  return LRPX_OK;
+}
 
 }  // namespace lrpx

@@ -352,15 +352,24 @@ def _check_requests(B, T, V, req_img, req_t, req_word, req_head=None, num_head=0
 DEC_W3_READY = 4          # LRPX_DEC_W3_READY
 
 
-def _decoder_workspace(ws_cache, kind, dims, nbytes, dev, tc_gemm):
+def weight_stamp(tensors):
+    """(data pointer, in-place version counter) of each tensor: changes when a tensor is replaced or updated in place
+    (``load_state_dict``, an optimizer step, ``p.add_()``).  Caches of prepared weight copies are keyed on it."""
+    return tuple((t.data_ptr(), t._version) for t in tensors)
+
+
+def _decoder_workspace(ws_cache, kind, dims, nbytes, dev, tc_gemm, weights=None):
     """Workspace of one LRP-decoder call -> (ws, extra flags, key to store it under after a successful call).
-    ``ws_cache`` (a dict owned by the caller, living exactly as long as the caller's ``weights`` dict stays unchanged —
-    BatchExplainer keeps one next to its weights) makes the workspace persistent per argument shape, so the split bf16
-    copies of the weight matrices written by the first call are reused (LRPX_DEC_W3_READY: four conversion kernels less
-    per call).  Entries are never evicted — a captured CUDA graph may point into them — and at most four shapes are kept;
-    nothing allocated during a stream capture is cached."""
+    ``ws_cache`` (a dict owned by the caller — BatchExplainer keeps one next to its weights) makes the workspace
+    persistent per argument shape and weights, so the split bf16 copies of the weight matrices written by the first call
+    are reused (LRPX_DEC_W3_READY: four conversion kernels less per call).  With ``weights`` (the decoder entry points
+    always pass theirs) the key also holds the weights' ``weight_stamp``: other weight tensors, or the same ones updated
+    in place, get a workspace of their own.  Entries are never evicted — a captured CUDA graph may point into them — and
+    at most four are kept; nothing allocated during a stream capture is cached."""
     ws = None
     key = (kind, dims, nbytes)
+    if weights is not None:
+        key += (weight_stamp(weights[k] for k in sorted(weights)),)
     if ws_cache is not None and tc_gemm:
         ws = ws_cache.get(key)
         if ws is not None:
@@ -397,7 +406,7 @@ def gridtd_decoder_lrp(state: dict, weights: dict, req_img, req_t, req_word, wan
     f.update(r_feat=r_feat, r_words=r_words, r_words_raw=r_raw)
     _fill_args(a, f, keep)
     nbytes = lib().lrpx_gridtd_decoder_workspace_bytes(C.byref(a))
-    ws, extra, store = _decoder_workspace(ws_cache, "gridtd", (B, T, H, E, P, Cc, V, Q), nbytes, dev, tc_gemm)
+    ws, extra, store = _decoder_workspace(ws_cache, "gridtd", (B, T, H, E, P, Cc, V, Q), nbytes, dev, tc_gemm, weights)
     a.flags |= extra
     check(lib().lrpx_gridtd_decoder_lrp_f32(C.byref(a), _ptr(ws), nbytes, _stream()), "lrpx_gridtd_decoder_lrp_f32")
     if store is not None:
@@ -427,7 +436,7 @@ def aoa_decoder_lrp(state: dict, weights: dict, num_head, req_img, req_t, req_wo
     f.update(r_feat=r_feat, r_words=r_words, r_words_raw=r_raw)
     _fill_args(a, f, keep)
     nbytes = lib().lrpx_aoa_decoder_workspace_bytes(C.byref(a))
-    ws, extra, store = _decoder_workspace(ws_cache, "aoa", (B, T, H, E, P, Cc, V, Q, num_head), nbytes, dev, tc_gemm)
+    ws, extra, store = _decoder_workspace(ws_cache, "aoa", (B, T, H, E, P, Cc, V, Q, num_head), nbytes, dev, tc_gemm, weights)
     a.flags |= extra
     check(lib().lrpx_aoa_decoder_lrp_f32(C.byref(a), _ptr(ws), nbytes, _stream()), "lrpx_aoa_decoder_lrp_f32")
     if store is not None:
@@ -459,7 +468,7 @@ def adaptive_decoder_lrp(state: dict, weights: dict, req_img, req_t, req_word, w
     f.update(r_feat=r_feat, r_words=r_words, r_words_raw=r_raw)
     _fill_args(a, f, keep)
     nbytes = lib().lrpx_adaptive_decoder_workspace_bytes(C.byref(a))
-    ws, extra, store = _decoder_workspace(ws_cache, "adaptive", (B, T, H, E, P, Cc, V, Q), nbytes, dev, tc_gemm)
+    ws, extra, store = _decoder_workspace(ws_cache, "adaptive", (B, T, H, E, P, Cc, V, Q), nbytes, dev, tc_gemm, weights)
     a.flags |= extra
     check(lib().lrpx_adaptive_decoder_lrp_f32(C.byref(a), _ptr(ws), nbytes, _stream()), "lrpx_adaptive_decoder_lrp_f32")
     if store is not None:

@@ -27,14 +27,15 @@ class BatchExplainer:
             raise ValueError("BatchExplainer drives the tensor-core chain: it needs a VGG-style encoder and "
                              "precision='fp32' (fp32-accurate mode) or 'bf16'")
         self.ex = explainer
-        self.eng = explainer.engine()
         # gradient-family explainers (models/_gradient.py): same pipeline, the decoder-gradient kernels and the chain's
         # 'gradient' / 'guided' rule instead of the relevance ones
         self.is_gradient = hasattr(explainer, "_grad_weights")
         if self.is_gradient and getattr(explainer, "CAM", None):
             raise ValueError("BatchExplainer covers the gradient and guided-backpropagation explainers, not the CAM variants")
-        self.W = explainer._grad_weights() if self.is_gradient else explainer._lrp_weights()
+        self.eng = self.W = None
         self._dec_ws = {}         # persistent decoder workspaces holding the prepared copies of self.W (ops._decoder_workspace)
+        self._graphs = {}
+        self._sync_weights()
         self.chunk = chunk
         self.use_graph = use_graph
         # decoder GEMMs as bf16x3 on the tensor cores in both chain modes (measured 1e-5 of max off the fp32 CUDA-core
@@ -44,8 +45,18 @@ class BatchExplainer:
         self.is_aoa = hasattr(explainer, "num_head") and hasattr(explainer.model, "decoder_multihead_attention")
         self.is_adaptive = not self.is_aoa and not hasattr(explainer.model, "LanguageLSTM")   # single-LSTM decoder
         self.head_idx = int(head_idx)
-        self._graphs = {}
         self._copy_stream = None
+
+    def _sync_weights(self):
+        """Decoder weights and encoder engine from the explainer, which rebuilds them after the model's parameters were
+        replaced or updated in place.  Then the decoder workspaces (prepared copies of the old weights) and the captured
+        graphs (pointing at the old tensors) are dropped as well."""
+        W = self.ex._grad_weights() if self.is_gradient else self.ex._lrp_weights()
+        eng = self.ex.engine()
+        if W is not self.W or eng is not self.eng:
+            self.W, self.eng = W, eng
+            self._dec_ws = {}
+            self._graphs = {}
 
     def _requests(self, B, T, device, words_per_image=None):
         """(image, word) requests in image-major order; ``words_per_image[b]`` <= T limits image b to its own caption
@@ -116,6 +127,7 @@ class BatchExplainer:
         ``host_out=(heat_host, words_host)`` (pinned tensors) additionally delivers the results to the host, the
         heat-map copy overlapped chunk by chunk with the relevance kernels.
         With ``use_graph`` the returned tensors are the graph's static outputs (overwritten by the next call)."""
+        self._sync_weights()
         B, T = tokens.shape[0], tokens.shape[1] - 1
         dev = self.ex.device
         wpi = None if words_per_image is None else tuple(int(v) for v in words_per_image)

@@ -93,6 +93,12 @@ class GradientFamily:
 
     # ------------------------------------------------------------------ plumbing
     def engine(self):
+        """The tensor-core encoder engine (converted copies of the encoder's weights), rebuilt when an encoder parameter
+        or buffer changes."""
+        key = self._encoder_stamp()
+        if self._engine is not None and self._engine_key != key:
+            self._engine = None
+        self._engine_key = key
         if self._engine is None:
             from lrpx import tc
             import torch.nn as nn
@@ -106,6 +112,15 @@ class GradientFamily:
                 self._engine = tc.TcVggEngine([c.weight for c in convs], [c.bias for c in convs], cfg, self.device,
                                               precision=self.precision, rule=self.RULE)
         return self._engine
+
+    def _cached_grad_weights(self, build):
+        """``build(state_dict)``: the decoder-gradient kernels' weights, rebuilt when a model parameter is replaced or
+        updated in place; the dict stays the same object until then."""
+        key = ops.weight_stamp(self.model.parameters())
+        if getattr(self, "_gw", None) is None or self._gw_key != key:
+            self._gw = build({k: v.detach() for k, v in self.model.state_dict().items()})
+            self._gw_key = key
+        return self._gw
 
     def _check_encoder(self):
         # Bottleneck ResNets: the fp32 CUDA-core path only (LRPtools.lrp_wrapper.encoder_gradient_simt)

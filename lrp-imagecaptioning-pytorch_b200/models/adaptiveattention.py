@@ -193,9 +193,10 @@ class ExplainAdaptiveAttention(ExplainGridTDAttention):
         self.adalstm_bias_i, self.adalstm_bias_h = m.AdaLSTM.lstm_cell.bias_ih, m.AdaLSTM.lstm_cell.bias_hh
 
     def _lrp_weights(self):
-        if self._weights is None:
+        key = ops.weight_stamp(self.model.parameters())           # rebuilt after an update of the model's parameters
+        if self._weights is None or self._weights_key != key:
             sd = {k: v.detach() for k, v in self.model.state_dict().items()}
-            self._weights = _dec.adaptive_weights(sd)
+            self._weights, self._weights_key = _dec.adaptive_weights(sd), key
         return self._weights
 
     def _explainer_weights(self):
@@ -353,9 +354,7 @@ class ExplainAdaptiveGradient(GradientFamily, ExplainAdaptiveAttention):
         self._check_encoder()
 
     def _grad_weights(self):
-        if getattr(self, "_gw", None) is None:
-            self._gw = adaptive_grad_weights({k: v.detach() for k, v in self.model.state_dict().items()})
-        return self._gw
+        return self._cached_grad_weights(adaptive_grad_weights)
 
     def _set_state(self, img, tokens, enc=None):
         ExplainAdaptiveAttention._set_state(self, img, tokens, enc)

@@ -361,8 +361,10 @@ class ExplainAOAAttention(ExplainGridTDAttention):
         self.model.decoder_multihead_attention.eval()
 
     def _lrp_weights(self):
-        if self._weights is None:
+        key = ops.weight_stamp(self.model.parameters())           # rebuilt after an update of the model's parameters
+        if self._weights is None or self._weights_key != key:
             self._weights = _dec.aoa_weights({k: v.detach() for k, v in self.model.state_dict().items()})
+            self._weights_key = key
         return self._weights
 
     def _explainer_weights(self, quirk_double_bias_ih=True):
@@ -589,9 +591,7 @@ class ExplainAOAGradient(GradientFamily, ExplainAOAAttention):
         self._check_encoder()
 
     def _grad_weights(self):
-        if getattr(self, "_gw", None) is None:
-            self._gw = aoa_grad_weights({k: v.detach() for k, v in self.model.state_dict().items()})
-        return self._gw
+        return self._cached_grad_weights(aoa_grad_weights)
 
     def _set_state(self, img, tokens, enc=None):
         ExplainAOAAttention._set_state(self, img, tokens, enc)

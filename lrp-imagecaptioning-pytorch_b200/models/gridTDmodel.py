@@ -571,8 +571,8 @@ class ExplainGridTDAttention(object):
         self.output_weight = m.fc.weight
         self.visualizatioin_save_path = os.path.join(args.save_path, args.dataset + 'explanation')
         os.makedirs(self.visualizatioin_save_path, exist_ok=True)
-        self._engine = None
-        self._weights = None
+        self._engine = self._engine_key = None
+        self._weights = self._weights_key = None
         self._state = None
 
     # ------------------------------------------------------------------ helpers
@@ -590,12 +590,25 @@ class ExplainGridTDAttention(object):
         return x.unsqueeze(0).to(self.device)
 
     def _lrp_weights(self):
-        if self._weights is None:
+        """The decoder relevance kernels' weights (gate rows concatenated, projector reshaped), rebuilt when a model
+        parameter is replaced or updated in place; the dict stays the same object until then."""
+        key = ops.weight_stamp(self.model.parameters())
+        if self._weights is None or self._weights_key != key:
             sd = {k: v.detach() for k, v in self.model.state_dict().items()}
-            self._weights = _dec.gridtd_weights(sd)
+            self._weights, self._weights_key = _dec.gridtd_weights(sd), key
         return self._weights
 
+    def _encoder_stamp(self):
+        enc = getattr(getattr(self.model, "img_encoder", None), "encoder", None)
+        return () if enc is None else ops.weight_stamp(list(enc.parameters()) + list(enc.buffers()))
+
     def engine(self):
+        """The tensor-core encoder engine (it holds converted copies of the encoder's weights): rebuilt when an encoder
+        parameter or buffer changes."""
+        key = self._encoder_stamp()
+        if self._engine is not None and self._engine_key != key:
+            self._engine = None
+        self._engine_key = key
         if self._engine is None and getattr(self, "is_resnet", False):
             from lrpx import tc_resnet
             self._engine = tc_resnet.TcResNetEngine(self.model.img_encoder.encoder, self.device)
@@ -956,9 +969,7 @@ class ExplainGridTDGradient(GradientFamily, ExplainGridTDAttention):
         self._check_encoder()
 
     def _grad_weights(self):
-        if getattr(self, "_gw", None) is None:
-            self._gw = gridtd_grad_weights({k: v.detach() for k, v in self.model.state_dict().items()})
-        return self._gw
+        return self._cached_grad_weights(gridtd_grad_weights)
 
     def get_hidden_parameters(self, img_filepath):
         """reference :1323-1422 (beam size 3, up to 50 words)."""

@@ -432,3 +432,28 @@ def test_decoder_workspace_cache_policy(monkeypatch):
     assert ops._decoder_workspace(cache, "gridtd", (8, 8), 100, "cuda", True)[1:] == (0, None)
     assert ops._decoder_workspace(cache, "gridtd", (1, 2, 3), 0, "cuda", True)[0] is not None            # nbytes 0 -> 4-byte dummy
     assert made[-1] == 4
+
+
+def test_decoder_workspace_cache_keyed_on_weights(monkeypatch):
+    """ops._decoder_workspace with the call's weights (host logic, no GPU): the prepared weight copies in a cached
+    workspace belong to the weights they were made from.  Other weight tensors of the same shapes, or the same tensors
+    after an in-place update (a new version counter, even when the values come back), are another entry."""
+    import torch
+    from lrpx import ops
+    W = {"W_b": torch.zeros(3), "W_a": torch.zeros(2)}
+    W2 = {"W_b": torch.zeros(3), "W_a": torch.zeros(2)}
+    monkeypatch.setattr(torch, "empty", lambda n, device=None, dtype=None: ("ws", n))
+    monkeypatch.setattr(torch.cuda, "is_current_stream_capturing", lambda: False)
+    cache = {}
+    ws, extra, key = ops._decoder_workspace(cache, "gridtd", (1, 2, 3), 100, "cuda", True, W)
+    assert extra == 0 and key is not None
+    cache[key] = ws
+    assert ops._decoder_workspace(cache, "gridtd", (1, 2, 3), 100, "cuda", True, W)[1] == ops.DEC_W3_READY
+    assert ops._decoder_workspace(cache, "gridtd", (1, 2, 3), 100, "cuda", True, dict(reversed(W.items())))[1] == \
+        ops.DEC_W3_READY                                                  # the key does not depend on the dict's order
+    _, e2, k2 = ops._decoder_workspace(cache, "gridtd", (1, 2, 3), 100, "cuda", True, W2)
+    assert e2 == 0 and k2 not in (None, key)
+    W["W_a"].add_(1.0)
+    W["W_a"].sub_(1.0)
+    _, e3, k3 = ops._decoder_workspace(cache, "gridtd", (1, 2, 3), 100, "cuda", True, W)
+    assert e3 == 0 and k3 not in (None, key, k2)
