@@ -4,6 +4,8 @@
 #pragma once
 #include "lrpx_common.cuh"
 
+#include <algorithm>
+
 namespace lrpx {
 
 // ------------------------------------------------------------------------------------------------
@@ -121,8 +123,12 @@ __device__ __forceinline__ void split_bf16(float x, __nv_bfloat16& hi, __nv_bflo
   hi = __float2bfloat16(x);
   lo = __float2bfloat16(x - __bfloat162float(hi));
 }
+// bf16 elements of the split operand of a GEMM with `rows` rows and reduction length K: each row is stored [hi | lo]
+// (2K), the layout put_operand, split3_act_kernel and the attention kernels' SPLIT stores write.  The GEMM reads it as
+// [hi | lo | hi] (a_phys = 2K in gemm_any).  Every workspace slot that receives a split operand is sized by this rule.
+static inline size_t split_elems(size_t rows, size_t K) { return rows * 2 * K; }
 // a producer kernel writes its GEMM operand both as fp32 (CUDA-core GEMM) and, when `a3` is given, directly as the
-// split row [hi | hi | lo] of the tensor-core GEMM (saves the separate split pass over the operand)
+// split row [hi | lo] of the tensor-core GEMM (saves the separate split pass over the operand)
 __device__ __forceinline__ void put_operand(float* u, __nv_bfloat16* a3, size_t row, int K, int k, float x) {
   u[row * K + k] = x;
   if (a3) {
@@ -220,8 +226,12 @@ static int gemm_any(const float* A, const float* W, const __nv_bfloat16* wt3, __
   g.x = e.x0; g.x1 = e.x1; g.bias = e.add_q; g.row_img = e.req_img;
   return lrpx_tc_conv(&g, st);
 }
+// Route of the GEMM with weight W (K x N): the prepared copy W' written into dst (N x 3K) when `tc` is set and the
+// tensor cores take the shape, null when the GEMM stays on the CUDA cores.
 // ready: dst still holds the split copy of W from an earlier call on the same workspace (LRPX_DEC_W3_READY)
-static __nv_bfloat16* prep_weight3(const float* W, __nv_bfloat16* dst, int K, int N, cudaStream_t st, bool ready = false) {
+static const __nv_bfloat16* tc_weight(bool tc, const float* W, __nv_bfloat16* dst, int K, int N, cudaStream_t st,
+                                      bool ready = false) {
+  if (!tc || !tc_shape_ok(N, K)) return nullptr;
   if (!ready) split3_weight_kernel<<<ew_grid((long long)K * N), 256, 0, st>>>(W, dst, K, N);
   return dst;
 }
@@ -238,7 +248,48 @@ static __global__ void words_norm_kernel(float* r_words, const int32_t* req_t, i
     for (int i = threadIdx.x; i <= t; i += 32) r[i] = r[i] / m;
 }
 
-static size_t align_up(size_t x) { return (x + 63) & ~(size_t)63; }
+// block-wide sum of `v` written by thread 0 through `store`
+template <class F>
+__device__ __forceinline__ void block_sum_store(float v, F store) {
+  for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  __shared__ float sm[32];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  if (lane == 0) sm[wid] = v;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float s = 0.f;
+    for (int k = 0; k < (blockDim.x + 31) / 32; ++k) s += sm[k];
+    store(s);
+  }
+}
+// Word relevance of request q, for the args struct of any decoder entry point: r_words (Q x T) and, when given,
+// r_words_raw hold the same values until words_norm_kernel normalises r_words.  Words past t stay zero.
+template <class Args>
+__device__ __forceinline__ void zero_words(const Args& a, int q) {
+  for (int j = threadIdx.x; j < a.T; j += blockDim.x) {
+    a.r_words[(size_t)q * a.T + j] = 0.f;
+    if (a.r_words_raw) a.r_words_raw[(size_t)q * a.T + j] = 0.f;
+  }
+}
+template <class Args>
+__device__ __forceinline__ void store_word(const Args& a, int q, int i, float s) {
+  a.r_words[(size_t)q * a.T + i] = s;
+  if (a.r_words_raw) a.r_words_raw[(size_t)q * a.T + i] = s;
+}
 
+static size_t align_up(size_t x) { return (x + 63) & ~(size_t)63; }
+// Walks a workspace layout slot by slot, each slot starting on an align_up boundary: with a null base it only sizes the
+// workspace (the *_workspace_bytes entry points), with the caller's base it places the slots.
+struct Carver {
+  float* base;
+  size_t off = 0;          // floats
+  float* f32(size_t n) {
+    float* p = base ? base + off : nullptr;
+    off += align_up(n);
+    return p;
+  }
+  __nv_bfloat16* bf16(size_t n) { return reinterpret_cast<__nv_bfloat16*>(f32((n + 1) / 2)); }
+  size_t bytes() const { return off * sizeof(float); }
+};
 
 }  // namespace lrpx

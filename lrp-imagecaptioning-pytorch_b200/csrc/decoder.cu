@@ -54,10 +54,7 @@ __global__ void grid_init_kernel(lrpx_gridtd_args a, GridWs w) {
     w.r_c1[o] = 0.f;
   }
   for (int j = threadIdx.x; j < a.E; j += blockDim.x) w.r_glob[(size_t)q * a.E + j] = 0.f;
-  for (int j = threadIdx.x; j < a.T; j += blockDim.x) {
-    a.r_words[(size_t)q * a.T + j] = 0.f;
-    if (a.r_words_raw) a.r_words_raw[(size_t)q * a.T + j] = 0.f;
-  }
+  zero_words(a, q);
 }
 
 // LanguageLSTM cell rule (:1061-1069) -> u = r_g2 / stab(g2)
@@ -129,18 +126,7 @@ __global__ void grid_post1_kernel(lrpx_gridtd_args a, GridWs w, int i) {
     else wsum += rx;
   }
   // r_h1[i] = rx1[H+2E:] is dead: it is overwritten at step i-1 before being read (:1075 vs :1110)
-  for (int o = 16; o; o >>= 1) wsum += __shfl_xor_sync(0xffffffffu, wsum, o);
-  __shared__ float sm[32];
-  int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  if (lane == 0) sm[wid] = wsum;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    float s = 0.f;
-    for (int k = 0; k < (blockDim.x + 31) / 32; ++k) s += sm[k];
-    float* dst = a.r_words_raw ? a.r_words_raw : a.r_words;
-    dst[(size_t)q * a.T + i] = s;
-    if (a.r_words_raw) a.r_words[(size_t)q * a.T + i] = s;
-  }
+  block_sum_store(wsum, [&](float s) { store_word(a, q, i, s); });
 }
 
 // u_g = r_glob / stab(glob_pre)   (:1116-1119)
@@ -312,38 +298,30 @@ __global__ void __launch_bounds__(512, 2) grid_attn_rows_kernel(lrpx_gridtd_args
   }
 }
 static size_t grid_carve(const lrpx_gridtd_args* a, float* base, GridWs* w) {
-  size_t off = 0;
-  auto take = [&](size_t n) {
-    float* p = base ? base + off : nullptr;
-    off += align_up(n);
-    return p;
-  };
+  Carver c{base};
   size_t Q = a->Q, H = a->H, E = a->E;
   size_t nmax = 3 * H > 2 * H + 2 * E ? 3 * H : 2 * H + 2 * E;
   if ((size_t)a->C > nmax) nmax = a->C;
-  GridWs t;
-  t.r_h2 = take(Q * H); t.r_c2 = take(Q * H); t.r_c1 = take(Q * H); t.r_cth = take(Q * H);
-  t.r_glob = take(Q * E);
-  t.u = take(Q * (H > E ? H : E));
-  t.v = take(Q * nmax);
-  t.uctx = take(Q * a->T * H);
-  t.coefavg = take(Q * a->C);
-  t.wproj = take(Q * a->P * H);
-  t.gA = take((size_t)a->B * a->P * H);
-  t.a3 = t.w3_g2 = t.w3_g1 = t.w3_glob = t.w3_proj = nullptr;
-  t.a3u = nullptr;
+  GridWs t{};
+  t.r_h2 = c.f32(Q * H); t.r_c2 = c.f32(Q * H); t.r_c1 = c.f32(Q * H); t.r_cth = c.f32(Q * H);
+  t.r_glob = c.f32(Q * E);
+  t.u = c.f32(Q * (H > E ? H : E));
+  t.v = c.f32(Q * nmax);
+  t.uctx = c.f32(Q * a->T * H);
+  t.coefavg = c.f32(Q * a->C);
+  t.wproj = c.f32(Q * a->P * H);
+  t.gA = c.f32((size_t)a->B * a->P * H);
   if (a->flags & LRPX_DEC_TC_GEMM) {
-    auto take16 = [&](size_t n) { return reinterpret_cast<__nv_bfloat16*>(take((n + 1) / 2)); };   // n bf16 elements
-    size_t rows_max = Q * a->P;
-    t.a3 = take16(rows_max * 3 * H > Q * 3 * E ? rows_max * 3 * H : Q * 3 * E);
-    t.w3_g2 = take16((size_t)3 * H * 3 * H);
-    t.w3_g1 = take16((size_t)(2 * H + 2 * E) * 3 * H);
-    t.w3_glob = take16((size_t)a->C * 3 * E);
-    t.w3_proj = take16((size_t)a->C * 3 * H);
-    t.a3u = take16(Q * 3 * H);
+    // a3: W_proj (Q*P, H), W_glob (Q, E), W_g2 and W_g1 (Q, H) unless fused;  a3u: W_g2 and W_g1 fused (Q, H)
+    t.a3 = c.bf16(std::max({split_elems(Q * a->P, H), split_elems(Q, E), split_elems(Q, H)}));
+    t.w3_g2 = c.bf16((size_t)3 * H * 3 * H);
+    t.w3_g1 = c.bf16((size_t)(2 * H + 2 * E) * 3 * H);
+    t.w3_glob = c.bf16((size_t)a->C * 3 * E);
+    t.w3_proj = c.bf16((size_t)a->C * 3 * H);
+    t.a3u = c.bf16(split_elems(Q, H));
   }
   if (w) *w = t;
-  return off * sizeof(float);
+  return c.bytes();
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -370,10 +348,7 @@ __global__ void aoa_init_kernel(lrpx_aoa_args a, AoaWs w) {
     w.u[(size_t)q * a.H + j] = rc / stab(cl[j]);              // lin() through decoder_aoa_linear (:1107-1110)
     w.r_glob[(size_t)q * a.H + j] = 0.f;
   }
-  for (int j = threadIdx.x; j < a.T; j += blockDim.x) {
-    a.r_words[(size_t)q * a.T + j] = 0.f;
-    if (a.r_words_raw) a.r_words_raw[(size_t)q * a.T + j] = 0.f;
-  }
+  zero_words(a, q);
 }
 // r_ctx = ctx * v ;  uval = r_ctx / stab(ctx) on the chosen head, 0 elsewhere (lrp_mha :848-860, Q5)
 __global__ void aoa_ctx_kernel(lrpx_aoa_args a, AoaWs w) {
@@ -416,17 +391,7 @@ __global__ void aoa_post_kernel(lrpx_aoa_args a, AoaWs w, int i) {
     else if (k < E + H) w.r_glob[(size_t)q * H + (k - E)] += rx;      // :1133
     else w.r_h[(size_t)q * H + (k - E - H)] = rx;                     // :1129
   }
-  for (int o = 16; o; o >>= 1) wsum += __shfl_xor_sync(0xffffffffu, wsum, o);
-  __shared__ float sm[32];
-  int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  if (lane == 0) sm[wid] = wsum;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    float s = 0.f;
-    for (int k = 0; k < (blockDim.x + 31) / 32; ++k) s += sm[k];
-    a.r_words[(size_t)q * a.T + i] = s;
-    if (a.r_words_raw) a.r_words_raw[(size_t)q * a.T + i] = s;
-  }
+  block_sum_store(wsum, [&](float s) { store_word(a, q, i, s); });
 }
 // wval = r_val / stab(value), r_val = value * alpha[head][p] * uval   (:1112-1113, :1141-1144)
 // addq = r_glob / stab(glob) / P                                     (:1136-1139)
@@ -443,30 +408,24 @@ __global__ void aoa_val_kernel(lrpx_aoa_args a, AoaWs w) {
 }
 
 static size_t aoa_carve(const lrpx_aoa_args* a, float* base, AoaWs* w) {
-  size_t off = 0;
-  auto take = [&](size_t n) {
-    float* p = base ? base + off : nullptr;
-    off += align_up(n);
-    return p;
-  };
+  Carver c{base};
   size_t Q = a->Q, H = a->H;
-  AoaWs t;
-  t.r_h = take(Q * H); t.r_glob = take(Q * H); t.u = take(Q * H);
-  t.v = take(Q * (a->E + 2 * H));
-  t.uval = take(Q * H); t.addq = take(Q * H);
-  t.wval = take(Q * a->P * H);
-  t.w2 = take(Q * a->P * H);
-  t.a3 = t.w3_aoa = t.w3_g = t.w3_v = t.w3_proj = nullptr;
+  AoaWs t{};
+  t.r_h = c.f32(Q * H); t.r_glob = c.f32(Q * H); t.u = c.f32(Q * H);
+  t.v = c.f32(Q * (a->E + 2 * H));
+  t.uval = c.f32(Q * H); t.addq = c.f32(Q * H);
+  t.wval = c.f32(Q * a->P * H);
+  t.w2 = c.f32(Q * a->P * H);
   if (a->flags & LRPX_DEC_TC_GEMM) {
-    auto take16 = [&](size_t n) { return reinterpret_cast<__nv_bfloat16*>(take((n + 1) / 2)); };
-    t.a3 = take16(Q * a->P * 3 * H);
-    t.w3_aoa = take16(H * 3 * H);
-    t.w3_g = take16((size_t)(a->E + 2 * H) * 3 * H);
-    t.w3_v = take16(H * 3 * H);
-    t.w3_proj = take16((size_t)a->C * 3 * H);
+    // a3: W_v and W_proj (Q*P, H), W_aoa and W_g (Q, H)
+    t.a3 = c.bf16(std::max(split_elems(Q * a->P, H), split_elems(Q, H)));
+    t.w3_aoa = c.bf16(H * 3 * H);
+    t.w3_g = c.bf16((size_t)(a->E + 2 * H) * 3 * H);
+    t.w3_v = c.bf16(H * 3 * H);
+    t.w3_proj = c.bf16((size_t)a->C * 3 * H);
   }
   if (w) *w = t;
-  return off * sizeof(float);
+  return c.bytes();
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -501,10 +460,7 @@ __global__ void ada_init_kernel(lrpx_adaptive_args a, AdaWs w) {
     w.uctx[o] = r_ctx / stab(cx);
   }
   for (int j = threadIdx.x; j < a.E; j += blockDim.x) w.r_glob[(size_t)q * a.E + j] = 0.f;
-  for (int j = threadIdx.x; j < a.T; j += blockDim.x) {
-    a.r_words[(size_t)q * a.T + j] = 0.f;
-    if (a.r_words_raw) a.r_words_raw[(size_t)q * a.T + j] = 0.f;
-  }
+  zero_words(a, q);
 }
 
 // cell rule (:726-734) -> u = r_g / stab(tanh g)   (the reference passes tanh(gt) as forward_output, :737)
@@ -541,18 +497,7 @@ __global__ void ada_post_kernel(lrpx_adaptive_args a, AdaWs w, int i) {
     else if (k < 2 * E) { if (i == t) w.r_glob[(size_t)q * E + (k - E)] = x[k] * vq[k]; }   // only the explained step (:740)
     else w.r_h[(size_t)q * H + (k - 2 * E)] = hp[k - 2 * E] * vq[k];
   }
-  for (int o = 16; o; o >>= 1) wsum += __shfl_xor_sync(0xffffffffu, wsum, o);
-  __shared__ float sm[32];
-  int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  if (lane == 0) sm[wid] = wsum;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    float s = 0.f;
-    for (int k = 0; k < (blockDim.x + 31) / 32; ++k) s += sm[k];
-    float* dst = a.r_words_raw ? a.r_words_raw : a.r_words;
-    dst[(size_t)q * a.T + i] = s;
-    if (a.r_words_raw) a.r_words[(size_t)q * a.T + i] = s;
-  }
+  block_sum_store(wsum, [&](float s) { store_word(a, q, i, s); });
 }
 
 // u_g = r_glob / stab(avg @ W_glob^T)   (:743-746, forward_output=False: no bias)
@@ -599,34 +544,27 @@ __global__ void __launch_bounds__(256) ada_attn_kernel(lrpx_adaptive_args a, Ada
 }
 
 static size_t ada_carve(const lrpx_adaptive_args* a, float* base, AdaWs* w) {
-  size_t off = 0;
-  auto take = [&](size_t n) {
-    float* p = base ? base + off : nullptr;
-    off += align_up(n);
-    return p;
-  };
+  Carver c{base};
   size_t Q = a->Q, H = a->H, E = a->E;
   size_t nmax = 2 * E + H > (size_t)a->C ? 2 * E + H : (size_t)a->C;
-  AdaWs t;
-  t.r_h = take(Q * H); t.r_c = take(Q * H);
-  t.r_glob = take(Q * E);
-  t.u = take(Q * (H > E ? H : E));
-  t.v = take(Q * nmax);
-  t.uctx = take(Q * H);
-  t.coefavg = take(Q * a->C);
-  t.wproj = take(Q * a->P * H);
-  t.a3 = t.w3_g = t.w3_glob = t.w3_proj = t.a3u = nullptr;
+  AdaWs t{};
+  t.r_h = c.f32(Q * H); t.r_c = c.f32(Q * H);
+  t.r_glob = c.f32(Q * E);
+  t.u = c.f32(Q * (H > E ? H : E));
+  t.v = c.f32(Q * nmax);
+  t.uctx = c.f32(Q * H);
+  t.coefavg = c.f32(Q * a->C);
+  t.wproj = c.f32(Q * a->P * H);
   if (a->flags & LRPX_DEC_TC_GEMM) {
-    auto take16 = [&](size_t n) { return reinterpret_cast<__nv_bfloat16*>(take((n + 1) / 2)); };   // n bf16 elements
-    size_t rows_max = Q * a->P;
-    t.a3 = take16(rows_max * 3 * H > Q * 3 * E ? rows_max * 3 * H : Q * 3 * E);
-    t.w3_g = take16((size_t)(2 * E + H) * 3 * H);
-    t.w3_glob = take16((size_t)a->C * 3 * E);
-    t.w3_proj = take16((size_t)a->C * 3 * H);
-    t.a3u = take16(Q * 3 * H);
+    // a3: W_proj (Q*P, H), W_glob (Q, E);  a3u: W_g, always fused (Q, H)
+    t.a3 = c.bf16(std::max(split_elems(Q * a->P, H), split_elems(Q, E)));
+    t.w3_g = c.bf16((size_t)(2 * E + H) * 3 * H);
+    t.w3_glob = c.bf16((size_t)a->C * 3 * E);
+    t.w3_proj = c.bf16((size_t)a->C * 3 * H);
+    t.a3u = c.bf16(split_elems(Q, H));
   }
   if (w) *w = t;
-  return off * sizeof(float);
+  return c.bytes();
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -710,12 +648,6 @@ __global__ void fc_lrp_weights_kernel(const float* __restrict__ logits, const fl
 
 using namespace lrpx;
 
-#define RUN(expr)                 \
-  do {                            \
-    int rc__ = (expr);            \
-    if (rc__ != LRPX_OK) return rc__; \
-  } while (0)
-
 extern "C" {
 
 size_t lrpx_gridtd_decoder_workspace_bytes(const lrpx_gridtd_args* a) {
@@ -743,11 +675,10 @@ int lrpx_gridtd_decoder_lrp_f32(const lrpx_gridtd_args* a, void* workspace, size
   // tensor-core GEMMs where the shape allows it (per GEMM), CUDA cores otherwise
   const bool tc = (a->flags & LRPX_DEC_TC_GEMM) != 0;
   const bool w3_ready = (a->flags & LRPX_DEC_W3_READY) != 0;
-  const __nv_bfloat16* w3_g2 = (tc && tc_shape_ok(3 * H, H)) ? prep_weight3(a->W_g2, w.w3_g2, H, 3 * H, st, w3_ready) : nullptr;
-  const __nv_bfloat16* w3_g1 =
-      (tc && tc_shape_ok(2 * H + 2 * E, H)) ? prep_weight3(a->W_g1, w.w3_g1, H, 2 * H + 2 * E, st, w3_ready) : nullptr;
-  const __nv_bfloat16* w3_glob = (tc && tc_shape_ok(a->C, E)) ? prep_weight3(a->W_glob, w.w3_glob, E, a->C, st, w3_ready) : nullptr;
-  const __nv_bfloat16* w3_proj = (tc && tc_shape_ok(a->C, H)) ? prep_weight3(a->W_proj, w.w3_proj, H, a->C, st, w3_ready) : nullptr;
+  const __nv_bfloat16* w3_g2 = tc_weight(tc, a->W_g2, w.w3_g2, H, 3 * H, st, w3_ready);
+  const __nv_bfloat16* w3_g1 = tc_weight(tc, a->W_g1, w.w3_g1, H, 2 * H + 2 * E, st, w3_ready);
+  const __nv_bfloat16* w3_glob = tc_weight(tc, a->W_glob, w.w3_glob, E, a->C, st, w3_ready);
+  const __nv_bfloat16* w3_proj = tc_weight(tc, a->W_proj, w.w3_proj, H, a->C, st, w3_ready);
   // the step kernels write the split operand themselves when both step GEMMs run on the tensor cores
   const bool fused_split = w3_g2 && w3_g1;
   if (!fused_split) w.a3u = nullptr;
@@ -817,10 +748,10 @@ int lrpx_aoa_decoder_lrp_f32(const lrpx_aoa_args* a, void* workspace, size_t wor
   GemmEpi none{};
   const bool tc = (a->flags & LRPX_DEC_TC_GEMM) != 0;
   const bool w3_ready = (a->flags & LRPX_DEC_W3_READY) != 0;
-  const __nv_bfloat16* w3_aoa = (tc && tc_shape_ok(H, H)) ? prep_weight3(a->W_aoa, w.w3_aoa, H, H, st, w3_ready) : nullptr;
-  const __nv_bfloat16* w3_g = (tc && tc_shape_ok(E + 2 * H, H)) ? prep_weight3(a->W_g, w.w3_g, H, E + 2 * H, st, w3_ready) : nullptr;
-  const __nv_bfloat16* w3_v = (tc && tc_shape_ok(H, H)) ? prep_weight3(a->W_v, w.w3_v, H, H, st, w3_ready) : nullptr;
-  const __nv_bfloat16* w3_proj = (tc && tc_shape_ok(a->C, H)) ? prep_weight3(a->W_proj, w.w3_proj, H, a->C, st, w3_ready) : nullptr;
+  const __nv_bfloat16* w3_aoa = tc_weight(tc, a->W_aoa, w.w3_aoa, H, H, st, w3_ready);
+  const __nv_bfloat16* w3_g = tc_weight(tc, a->W_g, w.w3_g, H, E + 2 * H, st, w3_ready);
+  const __nv_bfloat16* w3_v = tc_weight(tc, a->W_v, w.w3_v, H, H, st, w3_ready);
+  const __nv_bfloat16* w3_proj = tc_weight(tc, a->W_proj, w.w3_proj, H, a->C, st, w3_ready);
   aoa_init_kernel<<<Q, nt, 0, st>>>(*a, w);
   RUN(gemm_any<GE_STORE>(w.u, a->W_aoa, w3_aoa, w.a3, w.v, Q, H, H, none, st));
   aoa_ctx_kernel<<<Q, nt, 0, st>>>(*a, w);
@@ -862,9 +793,9 @@ int lrpx_adaptive_decoder_lrp_f32(const lrpx_adaptive_args* a, void* workspace, 
   GemmEpi none{};
   const bool tc = (a->flags & LRPX_DEC_TC_GEMM) != 0;
   const bool w3_ready = (a->flags & LRPX_DEC_W3_READY) != 0;
-  const __nv_bfloat16* w3_g = (tc && tc_shape_ok(2 * E + H, H)) ? prep_weight3(a->W_g, w.w3_g, H, 2 * E + H, st, w3_ready) : nullptr;
-  const __nv_bfloat16* w3_glob = (tc && tc_shape_ok(a->C, E)) ? prep_weight3(a->W_glob, w.w3_glob, E, a->C, st, w3_ready) : nullptr;
-  const __nv_bfloat16* w3_proj = (tc && tc_shape_ok(a->C, H)) ? prep_weight3(a->W_proj, w.w3_proj, H, a->C, st, w3_ready) : nullptr;
+  const __nv_bfloat16* w3_g = tc_weight(tc, a->W_g, w.w3_g, H, 2 * E + H, st, w3_ready);
+  const __nv_bfloat16* w3_glob = tc_weight(tc, a->W_glob, w.w3_glob, E, a->C, st, w3_ready);
+  const __nv_bfloat16* w3_proj = tc_weight(tc, a->W_proj, w.w3_proj, H, a->C, st, w3_ready);
   if (!w3_g) w.a3u = nullptr;
   ada_init_kernel<<<Q, nt, 0, st>>>(*a, w);
   for (int i = T - 1; i >= 0; --i) {

@@ -17,15 +17,7 @@
 #include "lrpx_common.cuh"
 #include "dec_gemm.cuh"
 
-#include <algorithm>
-
 namespace lrpx {
-
-#define RUN(x)                         \
-  do {                                 \
-    int rc__ = (x);                    \
-    if (rc__ != LRPX_OK) return rc__;  \
-  } while (0)
 
 // LSTM cell backward for one unit (gridTDmodel.py:1463-1472): dh = gradient of h_{i+1}, dc = gradient already carried
 // by c_{i+1}.  Returns the four gate pre-activation gradients (order i, f, g, o) and the carry into c_i.
@@ -56,20 +48,6 @@ __device__ __forceinline__ void put_gates(float* u, __nv_bfloat16* a3, size_t q,
 __device__ __forceinline__ void zero_gates(float* u, __nv_bfloat16* a3, size_t q, int H, int j) {
   for (int k = 0; k < 4; ++k) put_operand(u, a3, q, 4 * H, k * H + j, 0.f);
 }
-// block-wide sum of `v` written by thread 0 through `store`
-template <class F>
-__device__ __forceinline__ void block_sum_store(float v, F store) {
-  for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  __shared__ float sm[32];
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  if (lane == 0) sm[wid] = v;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    float s = 0.f;
-    for (int k = 0; k < (blockDim.x + 31) / 32; ++k) s += sm[k];
-    store(s);
-  }
-}
 
 // ------------------------------------------------------------------------------------------------
 // gridTD
@@ -89,10 +67,7 @@ __global__ void ggrad_init_kernel(lrpx_gridtd_grad_args a, GGradWs w) {
     w.d_c1[o] = 0.f;
   }
   for (int j = threadIdx.x; j < a.E; j += blockDim.x) w.d_glob[(size_t)q * a.E + j] = 0.f;
-  for (int j = threadIdx.x; j < a.T; j += blockDim.x) {
-    a.r_words[(size_t)q * a.T + j] = 0.f;
-    if (a.r_words_raw) a.r_words_raw[(size_t)q * a.T + j] = 0.f;
-  }
+  zero_words(a, q);
 }
 // LanguageLSTM cell backward (:1463-1473) -> u = [d_i | d_f | d_g | d_o]
 __global__ void ggrad_cell2_kernel(lrpx_gridtd_grad_args a, GGradWs w, int i) {
@@ -144,10 +119,7 @@ __global__ void ggrad_post1_kernel(lrpx_gridtd_grad_args a, GGradWs w, int i) {
     else if (k < H + E) w.d_glob[(size_t)q * E + (k - H)] += d;
     else wsum += d;
   }
-  block_sum_store(wsum, [&](float s) {
-    a.r_words[(size_t)q * a.T + i] = s;                                        // :1503
-    if (a.r_words_raw) a.r_words_raw[(size_t)q * a.T + i] = s;
-  });
+  block_sum_store(wsum, [&](float s) { store_word(a, q, i, s); });            // :1503
 }
 // coefavg = (d_glob @ W_glob) / P    (:1499, :1501)
 __global__ void ggrad_avg_kernel(lrpx_gridtd_grad_args a, GGradWs w) {
@@ -233,37 +205,29 @@ __global__ void ggrad_attn_slow_kernel(const float* __restrict__ alpha, const fl
 }
 
 static size_t ggrad_carve(const lrpx_gridtd_grad_args* a, float* base, GGradWs* w) {
-  size_t off = 0;
-  auto take = [&](size_t n) {
-    float* p = base ? base + off : nullptr;
-    off += align_up(n);
-    return p;
-  };
+  Carver c{base};
   const size_t Q = a->Q, H = a->H, E = a->E, C = a->C;
   size_t nmax = 3 * H > H + 2 * E ? 3 * H : H + 2 * E;
   if (C > nmax) nmax = C;
   GGradWs t{};
-  t.d_h2 = take(Q * H); t.d_c2 = take(Q * H); t.d_c1 = take(Q * H);
-  t.d_glob = take(Q * E);
-  t.u = take(Q * 4 * H);
-  t.v = take(Q * nmax);
-  t.uctx = take(Q * a->T * H);
-  t.coefavg = take(Q * C);
-  t.dproj = take(Q * a->P * H);
+  t.d_h2 = c.f32(Q * H); t.d_c2 = c.f32(Q * H); t.d_c1 = c.f32(Q * H);
+  t.d_glob = c.f32(Q * E);
+  t.u = c.f32(Q * 4 * H);
+  t.v = c.f32(Q * nmax);
+  t.uctx = c.f32(Q * a->T * H);
+  t.coefavg = c.f32(Q * C);
+  t.dproj = c.f32(Q * a->P * H);
   if (a->flags & LRPX_DEC_TC_GEMM) {
-    auto take16 = [&](size_t n) { return reinterpret_cast<__nv_bfloat16*>(take((n + 1) / 2)); };
-    // a3 takes the split operand of every GEMM but the fused step GEMMs: the projector (Q*P x H), the global
-    // projection (Q x E) and, when the step kernels do not split (fused_split off), the step GEMMs (Q x 4H)
-    const size_t kmax = std::max({(size_t)a->P * H, E, 4 * H});
-    t.a3 = take16(Q * 2 * kmax);
-    t.a3u = take16(Q * 2 * 4 * H);
-    t.w3_2 = take16(3 * H * 3 * 4 * H);
-    t.w3_1 = take16((H + 2 * E) * 3 * 4 * H);
-    t.w3_glob = take16(C * 3 * E);
-    t.w3_proj = take16(C * 3 * H);
+    // a3: W_proj (Q*P, H), W_glob (Q, E), W2 and W1 (Q, 4H) unless fused;  a3u: W2 and W1 fused (Q, 4H)
+    t.a3 = c.bf16(std::max({split_elems(Q * a->P, H), split_elems(Q, E), split_elems(Q, 4 * H)}));
+    t.a3u = c.bf16(split_elems(Q, 4 * H));
+    t.w3_2 = c.bf16(3 * H * 3 * 4 * H);
+    t.w3_1 = c.bf16((H + 2 * E) * 3 * 4 * H);
+    t.w3_glob = c.bf16(C * 3 * E);
+    t.w3_proj = c.bf16(C * 3 * H);
   }
   if (w) *w = t;
-  return off * sizeof(float);
+  return c.bytes();
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -291,10 +255,7 @@ __global__ void agrad_init_kernel(lrpx_aoa_grad_args a, AGradWs w) {
     w.uA[o] = d0 * sg;
     w.uB[o] = d0 * a.caoa_lin[bt + j] * (1.f - sg) * sg;
   }
-  for (int j = threadIdx.x; j < a.T; j += blockDim.x) {
-    a.r_words[(size_t)q * a.T + j] = 0.f;
-    if (a.r_words_raw) a.r_words_raw[(size_t)q * a.T + j] = 0.f;
-  }
+  zero_words(a, q);
 }
 // d_h[t+1] += d_B @ W_gate  (:1470);  d_value[p] = d_context (.) alpha[head][p] on the chosen head (gradient_mha :1415-1433)
 __global__ void agrad_ctx_kernel(lrpx_aoa_grad_args a, AGradWs w, const float* __restrict__ v_ctx,
@@ -334,39 +295,30 @@ __global__ void agrad_post_kernel(lrpx_aoa_grad_args a, AGradWs w, int i) {
     else if (k < E + H) { if (i == 0) w.d_glob[(size_t)q * H + (k - E)] = d / (float)a.P; }   // assigned, step 0 survives
     else w.d_h[(size_t)q * H + (k - E - H)] = d;
   }
-  block_sum_store(wsum, [&](float s) {
-    a.r_words[(size_t)q * a.T + i] = s;
-    if (a.r_words_raw) a.r_words_raw[(size_t)q * a.T + i] = s;
-  });
+  block_sum_store(wsum, [&](float s) { store_word(a, q, i, s); });
 }
 
 static size_t agrad_carve(const lrpx_aoa_grad_args* a, float* base, AGradWs* w) {
-  size_t off = 0;
-  auto take = [&](size_t n) {
-    float* p = base ? base + off : nullptr;
-    off += align_up(n);
-    return p;
-  };
+  Carver c{base};
   const size_t Q = a->Q, H = a->H, E = a->E;
   AGradWs t{};
-  t.d_h = take(Q * H); t.d_c = take(Q * H); t.d_glob = take(Q * H);
-  t.uA = take(Q * H); t.uB = take(Q * H);
-  t.u = take(Q * 4 * H);
-  t.v = take(Q * (E + 2 * H));
-  t.dval = take(Q * a->P * H);
-  t.dproj = take(Q * a->P * H);
+  t.d_h = c.f32(Q * H); t.d_c = c.f32(Q * H); t.d_glob = c.f32(Q * H);
+  t.uA = c.f32(Q * H); t.uB = c.f32(Q * H);
+  t.u = c.f32(Q * 4 * H);
+  t.v = c.f32(Q * (E + 2 * H));
+  t.dval = c.f32(Q * a->P * H);
+  t.dproj = c.f32(Q * a->P * H);
   if (a->flags & LRPX_DEC_TC_GEMM) {
-    auto take16 = [&](size_t n) { return reinterpret_cast<__nv_bfloat16*>(take((n + 1) / 2)); };
-    const size_t big = Q * a->P * 2 * H, small = Q * 2 * 4 * H;
-    t.a3 = take16(big > small ? big : small);
-    t.w3_aoa = take16(H * 3 * H);
-    t.w3_gate = take16(H * 3 * H);
-    t.w3_g = take16((E + 2 * H) * 3 * 4 * H);
-    t.w3_v = take16(H * 3 * H);
-    t.w3_proj = take16((size_t)a->C * 3 * H);
+    // a3: W_v and W_proj (Q*P, H), W_g (Q, 4H), W_aoa and W_gate (Q, H)
+    t.a3 = c.bf16(std::max({split_elems(Q * a->P, H), split_elems(Q, 4 * H), split_elems(Q, H)}));
+    t.w3_aoa = c.bf16(H * 3 * H);
+    t.w3_gate = c.bf16(H * 3 * H);
+    t.w3_g = c.bf16((E + 2 * H) * 3 * 4 * H);
+    t.w3_v = c.bf16(H * 3 * H);
+    t.w3_proj = c.bf16((size_t)a->C * 3 * H);
   }
   if (w) *w = t;
-  return off * sizeof(float);
+  return c.bytes();
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -395,10 +347,7 @@ __global__ void dgrad_init_kernel(lrpx_adaptive_grad_args a, DGradWs w) {
     w.d_h[o] = d0;                                                             // :992
   }
   for (int j = threadIdx.x; j < a.E; j += blockDim.x) w.d_glob[(size_t)q * a.E + j] = 0.f;
-  for (int j = threadIdx.x; j < a.T; j += blockDim.x) {
-    a.r_words[(size_t)q * a.T + j] = 0.f;
-    if (a.r_words_raw) a.r_words_raw[(size_t)q * a.T + j] = 0.f;
-  }
+  zero_words(a, q);
 }
 __global__ void dgrad_cell_kernel(lrpx_adaptive_grad_args a, DGradWs w, int i) {
   const int q = blockIdx.x, H = a.H;
@@ -425,10 +374,7 @@ __global__ void dgrad_post_kernel(lrpx_adaptive_grad_args a, DGradWs w, int i) {
     else if (k < 2 * E) w.d_glob[(size_t)q * E + (k - E)] += d;
     else w.d_h[(size_t)q * H + (k - 2 * E)] = d;
   }
-  block_sum_store(wsum, [&](float s) {
-    a.r_words[(size_t)q * a.T + i] = s;
-    if (a.r_words_raw) a.r_words_raw[(size_t)q * a.T + i] = s;
-  });
+  block_sum_store(wsum, [&](float s) { store_word(a, q, i, s); });
 }
 // d_feat[q][p][c] = (d_glob @ W_glob)[c] / P + alpha_t[p] * (d_context @ W_proj)[c]     (:1011-1015)
 __global__ void dgrad_out_kernel(lrpx_adaptive_grad_args a, const float* __restrict__ avg /* (Q,C) */,
@@ -442,30 +388,23 @@ __global__ void dgrad_out_kernel(lrpx_adaptive_grad_args a, const float* __restr
 }
 
 static size_t dgrad_carve(const lrpx_adaptive_grad_args* a, float* base, DGradWs* w) {
-  size_t off = 0;
-  auto take = [&](size_t n) {
-    float* p = base ? base + off : nullptr;
-    off += align_up(n);
-    return p;
-  };
+  Carver c{base};
   const size_t Q = a->Q, H = a->H, E = a->E, C = a->C;
   size_t nmax = 2 * E + H > C ? 2 * E + H : C;
   DGradWs t{};
-  t.d_h = take(Q * H); t.d_c = take(Q * H); t.d_glob = take(Q * E); t.dctx = take(Q * H);
-  t.u = take(Q * 4 * H);
-  t.v = take(Q * nmax);
-  t.y = take(Q * C);
+  t.d_h = c.f32(Q * H); t.d_c = c.f32(Q * H); t.d_glob = c.f32(Q * E); t.dctx = c.f32(Q * H);
+  t.u = c.f32(Q * 4 * H);
+  t.v = c.f32(Q * nmax);
+  t.y = c.f32(Q * C);
   if (a->flags & LRPX_DEC_TC_GEMM) {
-    auto take16 = [&](size_t n) { return reinterpret_cast<__nv_bfloat16*>(take((n + 1) / 2)); };
-    // a3 takes the split operand of every GEMM: the step GEMM (Q x 4H), the global projection (Q x E), the projector
-    // (Q x H)
-    t.a3 = take16(Q * 2 * std::max({4 * H, E, H}));
-    t.w3_g = take16((2 * E + H) * 3 * 4 * H);
-    t.w3_glob = take16(C * 3 * E);
-    t.w3_proj = take16(C * 3 * H);
+    // a3: W_g (Q, 4H), W_glob (Q, E), W_proj (Q, H)
+    t.a3 = c.bf16(std::max({split_elems(Q, 4 * H), split_elems(Q, E), split_elems(Q, H)}));
+    t.w3_g = c.bf16((2 * E + H) * 3 * 4 * H);
+    t.w3_glob = c.bf16(C * 3 * E);
+    t.w3_proj = c.bf16(C * 3 * H);
   }
   if (w) *w = t;
-  return off * sizeof(float);
+  return c.bytes();
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -562,11 +501,10 @@ int lrpx_gridtd_decoder_grad_f32(const lrpx_gridtd_grad_args* a, void* workspace
   const int nt = H >= 256 ? 256 : 128;
   GemmEpi none{};
   const bool tc = (a->flags & LRPX_DEC_TC_GEMM) != 0;
-  const __nv_bfloat16* w3_2 = (tc && tc_shape_ok(3 * H, 4 * H)) ? prep_weight3(a->W2, w.w3_2, 4 * H, 3 * H, st) : nullptr;
-  const __nv_bfloat16* w3_1 =
-      (tc && tc_shape_ok(H + 2 * E, 4 * H)) ? prep_weight3(a->W1, w.w3_1, 4 * H, H + 2 * E, st) : nullptr;
-  const __nv_bfloat16* w3_glob = (tc && tc_shape_ok(C, E)) ? prep_weight3(a->W_glob, w.w3_glob, E, C, st) : nullptr;
-  const __nv_bfloat16* w3_proj = (tc && tc_shape_ok(C, H)) ? prep_weight3(a->W_proj, w.w3_proj, H, C, st) : nullptr;
+  const __nv_bfloat16* w3_2 = tc_weight(tc, a->W2, w.w3_2, 4 * H, 3 * H, st);
+  const __nv_bfloat16* w3_1 = tc_weight(tc, a->W1, w.w3_1, 4 * H, H + 2 * E, st);
+  const __nv_bfloat16* w3_glob = tc_weight(tc, a->W_glob, w.w3_glob, E, C, st);
+  const __nv_bfloat16* w3_proj = tc_weight(tc, a->W_proj, w.w3_proj, H, C, st);
   const bool fused_split = w3_2 && w3_1;      // the step kernels write the split operand themselves
   if (!fused_split) w.a3u = nullptr;
   __nv_bfloat16* a3_step = fused_split ? w.a3u : w.a3;
@@ -628,12 +566,11 @@ int lrpx_aoa_decoder_grad_f32(const lrpx_aoa_grad_args* a, void* workspace, size
   const int nt = H >= 256 ? 256 : 128;
   GemmEpi none{};
   const bool tc = (a->flags & LRPX_DEC_TC_GEMM) != 0;
-  const bool hh = tc && tc_shape_ok(H, H);
-  const __nv_bfloat16* w3_aoa = hh ? prep_weight3(a->W_aoa, w.w3_aoa, H, H, st) : nullptr;
-  const __nv_bfloat16* w3_gate = hh ? prep_weight3(a->W_gate, w.w3_gate, H, H, st) : nullptr;
-  const __nv_bfloat16* w3_g = (tc && tc_shape_ok(E + 2 * H, 4 * H)) ? prep_weight3(a->W_g, w.w3_g, 4 * H, E + 2 * H, st) : nullptr;
-  const __nv_bfloat16* w3_v = hh ? prep_weight3(a->W_v, w.w3_v, H, H, st) : nullptr;
-  const __nv_bfloat16* w3_proj = (tc && tc_shape_ok(C, H)) ? prep_weight3(a->W_proj, w.w3_proj, H, C, st) : nullptr;
+  const __nv_bfloat16* w3_aoa = tc_weight(tc, a->W_aoa, w.w3_aoa, H, H, st);
+  const __nv_bfloat16* w3_gate = tc_weight(tc, a->W_gate, w.w3_gate, H, H, st);
+  const __nv_bfloat16* w3_g = tc_weight(tc, a->W_g, w.w3_g, 4 * H, E + 2 * H, st);
+  const __nv_bfloat16* w3_v = tc_weight(tc, a->W_v, w.w3_v, H, H, st);
+  const __nv_bfloat16* w3_proj = tc_weight(tc, a->W_proj, w.w3_proj, H, C, st);
   agrad_init_kernel<<<Q, nt, 0, st>>>(*a, w);
   float* v_ctx = w.v;                       // (Q,H)
   float* v_gate = w.v + (size_t)Q * H;      // (Q,H)   (v holds Q*(E+2H) floats)
@@ -679,9 +616,9 @@ int lrpx_adaptive_decoder_grad_f32(const lrpx_adaptive_grad_args* a, void* works
   const int nt = H >= 256 ? 256 : 128;
   GemmEpi none{};
   const bool tc = (a->flags & LRPX_DEC_TC_GEMM) != 0;
-  const __nv_bfloat16* w3_g = (tc && tc_shape_ok(2 * E + H, 4 * H)) ? prep_weight3(a->W_g, w.w3_g, 4 * H, 2 * E + H, st) : nullptr;
-  const __nv_bfloat16* w3_glob = (tc && tc_shape_ok(C, E)) ? prep_weight3(a->W_glob, w.w3_glob, E, C, st) : nullptr;
-  const __nv_bfloat16* w3_proj = (tc && tc_shape_ok(C, H)) ? prep_weight3(a->W_proj, w.w3_proj, H, C, st) : nullptr;
+  const __nv_bfloat16* w3_g = tc_weight(tc, a->W_g, w.w3_g, 4 * H, 2 * E + H, st);
+  const __nv_bfloat16* w3_glob = tc_weight(tc, a->W_glob, w.w3_glob, E, C, st);
+  const __nv_bfloat16* w3_proj = tc_weight(tc, a->W_proj, w.w3_proj, H, C, st);
   dgrad_init_kernel<<<Q, nt, 0, st>>>(*a, w);
   for (int i = T - 1; i >= 0; --i) {
     dgrad_cell_kernel<<<Q, nt, 0, st>>>(*a, w, i);

@@ -29,6 +29,13 @@ void set_error(const char* fmt, ...);
     }                                                                              \
   } while (0)
 
+// returns the status of a call that reports one (LRPX_OK or an error code) when it is not LRPX_OK
+#define RUN(expr)                      \
+  do {                                 \
+    int rc__ = (expr);                 \
+    if (rc__ != LRPX_OK) return rc__;  \
+  } while (0)
+
 // LRPtools/utils.py:16-18
 __device__ __forceinline__ float safe_div(float num, float den) {
   return num / (den + (den == 0.f ? LRPX_Z_EPSILON : 0.f));

@@ -380,100 +380,85 @@ def _decoder_workspace(ws_cache, kind, dims, nbytes, dev, tc_gemm, weights=None)
     return ws, 0, key
 
 
+def _decoder_call(run, size, args_cls, dims, flags, state, state_keys, weights, weight_keys, reqs, want_raw, out,
+                  ws_cache=None, ws_kind=None):
+    """Shared body of the six batched decoder entry points.  ``dims``: the dimension fields of ``args_cls`` in the order
+    B, T, H, E, P, C, V, Q[, num_head]; ``reqs``: req_img, req_t, req_word[, req_head].  Checks the requests, fills the
+    args struct with the float32 ``state_keys`` / ``weight_keys`` tensors, the int32 requests and the outputs (``out``
+    (Q,P,C), r_words (Q,T)[, r_words_raw]), sizes the workspace with the lib function ``size``, calls ``run``.
+    ``ws_kind`` names the decoder in the ``ws_cache`` key (_decoder_workspace).  Returns out, r_words[, r_words_raw]."""
+    dev = state["feat"].device
+    Q, T = dims["Q"], dims["T"]
+    _check_requests(dims["B"], T, dims["V"], *reqs.values(), num_head=dims.get("num_head", 0))
+    f = {k: _f32(state[k], k) for k in state_keys}
+    f.update({k: _f32(weights[k], k) for k in weight_keys})
+    f.update({k: v.to(device=dev, dtype=torch.int32).contiguous() for k, v in reqs.items()})
+    res = torch.empty(Q, dims["P"], dims["C"], device=dev, dtype=torch.float32)
+    r_words = torch.zeros(Q, T, device=dev, dtype=torch.float32)
+    r_raw = torch.zeros(Q, T, device=dev, dtype=torch.float32) if want_raw else None
+    f.update({out: res, "r_words": r_words, "r_words_raw": r_raw})
+    keep = []
+    a = _fill_args(args_cls(**dims, flags=flags), f, keep)
+    nbytes = getattr(lib(), size)(C.byref(a))
+    ws, extra, store = _decoder_workspace(ws_cache, ws_kind, tuple(dims.values()), nbytes, dev,
+                                          bool(flags & DEC_TC_GEMM), weights)
+    a.flags |= extra
+    check(getattr(lib(), run)(C.byref(a), _ptr(ws), nbytes, _stream()), run)
+    if store is not None:
+        ws_cache[store] = ws
+    return (res, r_words, r_raw) if want_raw else (res, r_words)
+
+
 def gridtd_decoder_lrp(state: dict, weights: dict, req_img, req_t, req_word, want_raw=False, tc_gemm=False, ws_cache=None):
     """state: tensors of lrpx_gridtd_args (stacked over B images), weights: W_g1,W_g2,W_fc,W_glob,W_proj.
     tc_gemm: run the GEMMs as error-compensated bf16x3 on the tensor cores (LRPX_DEC_TC_GEMM) instead of fp32
     CUDA cores.  Returns r_feat (Q,P,C), r_words (Q,T)[, r_words_raw]."""
-    dev = state["feat"].device
     B, P, Cc = state["feat"].shape
     T, H = state["g1"].shape[1], state["g1"].shape[2]
     E = state["glob_pre"].shape[1]
     V = state["pred"].shape[2]
     Q = int(req_img.numel())
-    _check_requests(B, T, V, req_img, req_t, req_word)
-    keep = []
-    a = _lib.GridTDArgs(B=B, T=T, H=H, E=E, P=P, C=Cc, V=V, Q=Q, flags=DEC_TC_GEMM if tc_gemm else 0)
-    f = {k: _f32(state[k], k) for k in ["feat", "avg", "A_pre", "A", "glob_pre", "x1", "x2", "h1", "c1", "h2", "c2",
-                                        "g1", "i1", "f1", "g2", "i2", "f2", "st", "ctx", "ctx_hat", "alpha", "beta",
-                                        "pred"]}
-    f.update({k: _f32(weights[k], k) for k in ["W_g1", "W_g2", "W_fc", "W_glob", "W_proj"]})
-    f["req_img"] = req_img.to(device=dev, dtype=torch.int32).contiguous()
-    f["req_t"] = req_t.to(device=dev, dtype=torch.int32).contiguous()
-    f["req_word"] = req_word.to(device=dev, dtype=torch.int32).contiguous()
-    r_feat = torch.empty(Q, P, Cc, device=dev, dtype=torch.float32)
-    r_words = torch.zeros(Q, T, device=dev, dtype=torch.float32)
-    r_raw = torch.zeros(Q, T, device=dev, dtype=torch.float32) if want_raw else None
-    f.update(r_feat=r_feat, r_words=r_words, r_words_raw=r_raw)
-    _fill_args(a, f, keep)
-    nbytes = lib().lrpx_gridtd_decoder_workspace_bytes(C.byref(a))
-    ws, extra, store = _decoder_workspace(ws_cache, "gridtd", (B, T, H, E, P, Cc, V, Q), nbytes, dev, tc_gemm, weights)
-    a.flags |= extra
-    check(lib().lrpx_gridtd_decoder_lrp_f32(C.byref(a), _ptr(ws), nbytes, _stream()), "lrpx_gridtd_decoder_lrp_f32")
-    if store is not None:
-        ws_cache[store] = ws
-    return (r_feat, r_words, r_raw) if want_raw else (r_feat, r_words)
+    return _decoder_call(
+        "lrpx_gridtd_decoder_lrp_f32", "lrpx_gridtd_decoder_workspace_bytes", _lib.GridTDArgs,
+        dict(B=B, T=T, H=H, E=E, P=P, C=Cc, V=V, Q=Q), DEC_TC_GEMM if tc_gemm else 0,
+        state, ["feat", "avg", "A_pre", "A", "glob_pre", "x1", "x2", "h1", "c1", "h2", "c2", "g1", "i1", "f1", "g2", "i2",
+                "f2", "st", "ctx", "ctx_hat", "alpha", "beta", "pred"],
+        weights, ["W_g1", "W_g2", "W_fc", "W_glob", "W_proj"],
+        dict(req_img=req_img, req_t=req_t, req_word=req_word), want_raw, "r_feat", ws_cache, "gridtd")
 
 
 def aoa_decoder_lrp(state: dict, weights: dict, num_head, req_img, req_t, req_word, req_head, want_raw=False,
                     tc_gemm=False, ws_cache=None):
-    dev = state["feat"].device
     B, P, Cc = state["feat"].shape
     T, H = state["g"].shape[1], state["g"].shape[2]
     E = state["x"].shape[2] - H
     V = state["pred"].shape[2]
     Q = int(req_img.numel())
-    _check_requests(B, T, V, req_img, req_t, req_word, req_head, num_head)
-    keep = []
-    a = _lib.AoaArgs(B=B, T=T, H=H, E=E, P=P, C=Cc, V=V, Q=Q, num_head=num_head, flags=DEC_TC_GEMM if tc_gemm else 0)
-    f = {k: _f32(state[k], k) for k in ["feat", "A_pre", "A", "glob", "value", "x", "h", "c", "g", "i", "ctx", "caoa",
-                                        "caoa_lin", "alpha", "pred"]}
-    f.update({k: _f32(weights[k], k) for k in ["W_g", "W_fc", "W_aoa", "W_v", "W_proj"]})
-    for k, v in (("req_img", req_img), ("req_t", req_t), ("req_word", req_word), ("req_head", req_head)):
-        f[k] = v.to(device=dev, dtype=torch.int32).contiguous()
-    r_feat = torch.empty(Q, P, Cc, device=dev, dtype=torch.float32)
-    r_words = torch.zeros(Q, T, device=dev, dtype=torch.float32)
-    r_raw = torch.zeros(Q, T, device=dev, dtype=torch.float32) if want_raw else None
-    f.update(r_feat=r_feat, r_words=r_words, r_words_raw=r_raw)
-    _fill_args(a, f, keep)
-    nbytes = lib().lrpx_aoa_decoder_workspace_bytes(C.byref(a))
-    ws, extra, store = _decoder_workspace(ws_cache, "aoa", (B, T, H, E, P, Cc, V, Q, num_head), nbytes, dev, tc_gemm, weights)
-    a.flags |= extra
-    check(lib().lrpx_aoa_decoder_lrp_f32(C.byref(a), _ptr(ws), nbytes, _stream()), "lrpx_aoa_decoder_lrp_f32")
-    if store is not None:
-        ws_cache[store] = ws
-    return (r_feat, r_words, r_raw) if want_raw else (r_feat, r_words)
+    return _decoder_call(
+        "lrpx_aoa_decoder_lrp_f32", "lrpx_aoa_decoder_workspace_bytes", _lib.AoaArgs,
+        dict(B=B, T=T, H=H, E=E, P=P, C=Cc, V=V, Q=Q, num_head=num_head), DEC_TC_GEMM if tc_gemm else 0,
+        state, ["feat", "A_pre", "A", "glob", "value", "x", "h", "c", "g", "i", "ctx", "caoa", "caoa_lin", "alpha",
+                "pred"],
+        weights, ["W_g", "W_fc", "W_aoa", "W_v", "W_proj"],
+        dict(req_img=req_img, req_t=req_t, req_word=req_word, req_head=req_head), want_raw, "r_feat", ws_cache, "aoa")
 
 
 def adaptive_decoder_lrp(state: dict, weights: dict, req_img, req_t, req_word, want_raw=False, tc_gemm=False, ws_cache=None):
     """ExplainAdaptiveAttention.explain_caption_wordt (adaptiveattention.py:679-771) batched over requests.
     state: tensors of lrpx_adaptive_args (stacked over B images), weights: W_g, W_fc, W_glob, W_proj.
     Returns r_feat (Q,P,C), r_words (Q,T)[, r_words_raw]."""
-    dev = state["feat"].device
     B, P, Cc = state["feat"].shape
     T, H = state["g"].shape[1], state["g"].shape[2]
     E = state["z_glob"].shape[1]
     V = state["pred"].shape[2]
     Q = int(req_img.numel())
-    _check_requests(B, T, V, req_img, req_t, req_word)
-    keep = []
-    a = _lib.AdaptiveArgs(B=B, T=T, H=H, E=E, P=P, C=Cc, V=V, Q=Q, flags=DEC_TC_GEMM if tc_gemm else 0)
-    f = {k: _f32(state[k], k) for k in ["feat", "avg", "z_proj", "A", "z_glob", "x", "h", "c", "g", "i", "f", "st",
-                                        "ctx", "ctx_hat", "alpha", "beta", "pred"]}
-    f.update({k: _f32(weights[k], k) for k in ["W_g", "W_fc", "W_glob", "W_proj"]})
-    for k, v in (("req_img", req_img), ("req_t", req_t), ("req_word", req_word)):
-        f[k] = v.to(device=dev, dtype=torch.int32).contiguous()
-    r_feat = torch.empty(Q, P, Cc, device=dev, dtype=torch.float32)
-    r_words = torch.zeros(Q, T, device=dev, dtype=torch.float32)
-    r_raw = torch.zeros(Q, T, device=dev, dtype=torch.float32) if want_raw else None
-    f.update(r_feat=r_feat, r_words=r_words, r_words_raw=r_raw)
-    _fill_args(a, f, keep)
-    nbytes = lib().lrpx_adaptive_decoder_workspace_bytes(C.byref(a))
-    ws, extra, store = _decoder_workspace(ws_cache, "adaptive", (B, T, H, E, P, Cc, V, Q), nbytes, dev, tc_gemm, weights)
-    a.flags |= extra
-    check(lib().lrpx_adaptive_decoder_lrp_f32(C.byref(a), _ptr(ws), nbytes, _stream()), "lrpx_adaptive_decoder_lrp_f32")
-    if store is not None:
-        ws_cache[store] = ws
-    return (r_feat, r_words, r_raw) if want_raw else (r_feat, r_words)
+    return _decoder_call(
+        "lrpx_adaptive_decoder_lrp_f32", "lrpx_adaptive_decoder_workspace_bytes", _lib.AdaptiveArgs,
+        dict(B=B, T=T, H=H, E=E, P=P, C=Cc, V=V, Q=Q), DEC_TC_GEMM if tc_gemm else 0,
+        state, ["feat", "avg", "z_proj", "A", "z_glob", "x", "h", "c", "g", "i", "f", "st", "ctx", "ctx_hat", "alpha",
+                "beta", "pred"],
+        weights, ["W_g", "W_fc", "W_glob", "W_proj"],
+        dict(req_img=req_img, req_t=req_t, req_word=req_word), want_raw, "r_feat", ws_cache, "adaptive")
 
 
 # ------------------------------------------------------------------------------------------ gradient family (f4)
@@ -484,30 +469,17 @@ def gridtd_decoder_grad(state: dict, weights: dict, req_img, req_t, req_word, gu
     """ExplainGridTDGradient.explain_caption_wordt (gridTDmodel.py:1424-1508; ``guided``: :1588-1675) batched over
     requests.  state: the explainer forward's tensors incl. the output / sentinel gates (o1, o2, sg); weights: W1 (4H,
     H+2E), W2 (4H, 3H), W_fc, W_glob, W_proj.  Returns d_feat (Q,P,C), r_words (Q,T)[, r_words_raw]."""
-    dev = state["feat"].device
     B, P, Cc = state["feat"].shape
     T, H = state["g1"].shape[1], state["g1"].shape[2]
     E = weights["W_glob"].shape[0]
     V = weights["W_fc"].shape[0]
     Q = int(req_img.numel())
-    _check_requests(B, T, V, req_img, req_t, req_word)
-    keep = []
-    a = _lib.GridTDGradArgs(B=B, T=T, H=H, E=E, P=P, C=Cc, V=V, Q=Q,
-                            flags=(DEC_TC_GEMM if tc_gemm else 0) | (DEC_GUIDED if guided else 0))
-    f = {k: _f32(state[k], k) for k in ["feat", "c1", "c2", "g1", "i1", "f1", "o1", "g2", "i2", "f2", "o2", "sg", "alpha",
-                                        "beta"]}
-    f.update({k: _f32(weights[k], k) for k in ["W1", "W2", "W_fc", "W_glob", "W_proj"]})
-    for k, v in (("req_img", req_img), ("req_t", req_t), ("req_word", req_word)):
-        f[k] = v.to(device=dev, dtype=torch.int32).contiguous()
-    d_feat = torch.empty(Q, P, Cc, device=dev, dtype=torch.float32)
-    r_words = torch.zeros(Q, T, device=dev, dtype=torch.float32)
-    r_raw = torch.zeros(Q, T, device=dev, dtype=torch.float32) if want_raw else None
-    f.update(d_feat=d_feat, r_words=r_words, r_words_raw=r_raw)
-    _fill_args(a, f, keep)
-    nbytes = lib().lrpx_gridtd_decoder_grad_workspace_bytes(C.byref(a))
-    ws = torch.empty(max(nbytes, 4), device=dev, dtype=torch.uint8)
-    check(lib().lrpx_gridtd_decoder_grad_f32(C.byref(a), _ptr(ws), nbytes, _stream()), "lrpx_gridtd_decoder_grad_f32")
-    return (d_feat, r_words, r_raw) if want_raw else (d_feat, r_words)
+    return _decoder_call(
+        "lrpx_gridtd_decoder_grad_f32", "lrpx_gridtd_decoder_grad_workspace_bytes", _lib.GridTDGradArgs,
+        dict(B=B, T=T, H=H, E=E, P=P, C=Cc, V=V, Q=Q), (DEC_TC_GEMM if tc_gemm else 0) | (DEC_GUIDED if guided else 0),
+        state, ["feat", "c1", "c2", "g1", "i1", "f1", "o1", "g2", "i2", "f2", "o2", "sg", "alpha", "beta"],
+        weights, ["W1", "W2", "W_fc", "W_glob", "W_proj"],
+        dict(req_img=req_img, req_t=req_t, req_word=req_word), want_raw, "d_feat")
 
 
 def aoa_decoder_grad(state: dict, weights: dict, num_head, req_img, req_t, req_word, req_head, want_raw=False,
@@ -515,56 +487,34 @@ def aoa_decoder_grad(state: dict, weights: dict, num_head, req_img, req_t, req_w
     """ExplainAOAGradient.explain_caption_wordt (aoamodel.py:1435-1499) batched over requests.  state: the explainer
     forward's tensors incl. the output gate ``o`` and the gate pre-activation ``caoa_gate``; weights: W_g (4H, E+2H),
     W_fc, W_aoa, W_gate, W_v, W_proj."""
-    dev = state["feat"].device
     B, P, Cc = state["feat"].shape
     T, H = state["g"].shape[1], state["g"].shape[2]
     E = weights["W_g"].shape[1] - 2 * H
     V = weights["W_fc"].shape[0]
     Q = int(req_img.numel())
-    _check_requests(B, T, V, req_img, req_t, req_word, req_head, num_head)
-    keep = []
-    a = _lib.AoaGradArgs(B=B, T=T, H=H, E=E, P=P, C=Cc, V=V, Q=Q, num_head=num_head, flags=DEC_TC_GEMM if tc_gemm else 0)
-    f = {k: _f32(state[k], k) for k in ["c", "g", "i", "f", "o", "caoa_gate", "caoa_lin", "alpha"]}
-    f.update({k: _f32(weights[k], k) for k in ["W_g", "W_fc", "W_aoa", "W_gate", "W_v", "W_proj"]})
-    for k, v in (("req_img", req_img), ("req_t", req_t), ("req_word", req_word), ("req_head", req_head)):
-        f[k] = v.to(device=dev, dtype=torch.int32).contiguous()
-    d_feat = torch.empty(Q, P, Cc, device=dev, dtype=torch.float32)
-    r_words = torch.zeros(Q, T, device=dev, dtype=torch.float32)
-    r_raw = torch.zeros(Q, T, device=dev, dtype=torch.float32) if want_raw else None
-    f.update(d_feat=d_feat, r_words=r_words, r_words_raw=r_raw)
-    _fill_args(a, f, keep)
-    nbytes = lib().lrpx_aoa_decoder_grad_workspace_bytes(C.byref(a))
-    ws = torch.empty(max(nbytes, 4), device=dev, dtype=torch.uint8)
-    check(lib().lrpx_aoa_decoder_grad_f32(C.byref(a), _ptr(ws), nbytes, _stream()), "lrpx_aoa_decoder_grad_f32")
-    return (d_feat, r_words, r_raw) if want_raw else (d_feat, r_words)
+    return _decoder_call(
+        "lrpx_aoa_decoder_grad_f32", "lrpx_aoa_decoder_grad_workspace_bytes", _lib.AoaGradArgs,
+        dict(B=B, T=T, H=H, E=E, P=P, C=Cc, V=V, Q=Q, num_head=num_head), DEC_TC_GEMM if tc_gemm else 0,
+        state, ["c", "g", "i", "f", "o", "caoa_gate", "caoa_lin", "alpha"],
+        weights, ["W_g", "W_fc", "W_aoa", "W_gate", "W_v", "W_proj"],
+        dict(req_img=req_img, req_t=req_t, req_word=req_word, req_head=req_head), want_raw, "d_feat")
 
 
 def adaptive_decoder_grad(state: dict, weights: dict, req_img, req_t, req_word, want_raw=False, tc_gemm=False):
     """ExplainAdaptiveGradient.explain_caption_wordt (adaptiveattention.py:965-1021) batched over requests.  state: the
     explainer forward's tensors incl. the output gate ``o`` and the sentinel gate ``sg``; weights: W_g (4H, 2E+H), W_fc,
     W_glob, W_proj."""
-    dev = state["feat"].device
     B, P, Cc = state["feat"].shape
     T, H = state["g"].shape[1], state["g"].shape[2]
     E = weights["W_glob"].shape[0]
     V = weights["W_fc"].shape[0]
     Q = int(req_img.numel())
-    _check_requests(B, T, V, req_img, req_t, req_word)
-    keep = []
-    a = _lib.AdaptiveGradArgs(B=B, T=T, H=H, E=E, P=P, C=Cc, V=V, Q=Q, flags=DEC_TC_GEMM if tc_gemm else 0)
-    f = {k: _f32(state[k], k) for k in ["c", "g", "i", "f", "o", "sg", "alpha", "beta"]}
-    f.update({k: _f32(weights[k], k) for k in ["W_g", "W_fc", "W_glob", "W_proj"]})
-    for k, v in (("req_img", req_img), ("req_t", req_t), ("req_word", req_word)):
-        f[k] = v.to(device=dev, dtype=torch.int32).contiguous()
-    d_feat = torch.empty(Q, P, Cc, device=dev, dtype=torch.float32)
-    r_words = torch.zeros(Q, T, device=dev, dtype=torch.float32)
-    r_raw = torch.zeros(Q, T, device=dev, dtype=torch.float32) if want_raw else None
-    f.update(d_feat=d_feat, r_words=r_words, r_words_raw=r_raw)
-    _fill_args(a, f, keep)
-    nbytes = lib().lrpx_adaptive_decoder_grad_workspace_bytes(C.byref(a))
-    ws = torch.empty(max(nbytes, 4), device=dev, dtype=torch.uint8)
-    check(lib().lrpx_adaptive_decoder_grad_f32(C.byref(a), _ptr(ws), nbytes, _stream()), "lrpx_adaptive_decoder_grad_f32")
-    return (d_feat, r_words, r_raw) if want_raw else (d_feat, r_words)
+    return _decoder_call(
+        "lrpx_adaptive_decoder_grad_f32", "lrpx_adaptive_decoder_grad_workspace_bytes", _lib.AdaptiveGradArgs,
+        dict(B=B, T=T, H=H, E=E, P=P, C=Cc, V=V, Q=Q), DEC_TC_GEMM if tc_gemm else 0,
+        state, ["c", "g", "i", "f", "o", "sg", "alpha", "beta"],
+        weights, ["W_g", "W_fc", "W_glob", "W_proj"],
+        dict(req_img=req_img, req_t=req_t, req_word=req_word), want_raw, "d_feat")
 
 
 def grad_cam(feat, grads, req_img=None):

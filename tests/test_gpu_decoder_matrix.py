@@ -5,7 +5,8 @@ Each GEMM of a decoder picks its own route: the error-compensated bf16x3 tensor-
 ``tc_shape_ok(N, K)`` holds, the fp32 CUDA-core SGEMM otherwise.  The route also decides which workspace slot receives
 the split operand (``a3``, or ``a3u`` when the step kernels write the split themselves).  SHAPES runs every GEMM of
 every decoder on both routes and the fused split both on and off; ``test_route_table_covers_both_routes`` (no GPU)
-keeps that list honest.  Further cases: odd hidden widths and pixel counts, the long-caption fallback of the gridTD
+keeps that list honest, and ``test_workspace_holds_weight_copies_and_split_operands`` (no GPU) checks the workspace
+sizes against the same GEMM table.  Further cases: odd hidden widths and pixel counts, the long-caption fallback of the gridTD
 relevance attention, workspace sizing with E > 4H, request counts beyond a grid's y limit (65 535), a second device.
 
 Bars: scale-relative atol 1e-5 on the CUDA-core route, 1e-4 on the tensor-core route (bf16x3 keeps ~2^-16 relative per
@@ -26,19 +27,23 @@ DEV = "cuda"
 
 # ------------------------------------------------------------------------------------------------ route table (CPU)
 def tc_shape_ok(N, K):
-    """csrc/dec_gemm.cuh:188 — the shapes the tensor-core GEMM takes (N output columns, K reduction length)."""
+    """``tc_shape_ok`` of csrc/dec_gemm.cuh — the shapes the tensor-core GEMM takes (N output columns, K reduction
+    length)."""
     return K % 64 == 0 and N % 32 == 0 and (N <= 256 or N % 256 == 0)
 
 
-def gemm_table(kind, H, E, C):
-    """(weight, N, K) of every GEMM the entry point runs (csrc/decoder.cu, csrc/decoder_grad.cu)."""
+def gemm_table(kind, H, E, C, Q=1, P=1):
+    """(weight, N, K, rows) of every GEMM the entry point runs for Q requests of P pixels (csrc/decoder.cu,
+    csrc/decoder_grad.cu)."""
+    QP = Q * P
     return {
-        "gridtd_lrp": [("W_g2", 3 * H, H), ("W_g1", 2 * H + 2 * E, H), ("W_glob", C, E), ("W_proj", C, H)],
-        "aoa_lrp": [("W_aoa", H, H), ("W_g", E + 2 * H, H), ("W_v", H, H), ("W_proj", C, H)],
-        "adaptive_lrp": [("W_g", 2 * E + H, H), ("W_glob", C, E), ("W_proj", C, H)],
-        "gridtd_grad": [("W2", 3 * H, 4 * H), ("W1", H + 2 * E, 4 * H), ("W_glob", C, E), ("W_proj", C, H)],
-        "aoa_grad": [("W_aoa", H, H), ("W_gate", H, H), ("W_g", E + 2 * H, 4 * H), ("W_v", H, H), ("W_proj", C, H)],
-        "adaptive_grad": [("W_g", 2 * E + H, 4 * H), ("W_glob", C, E), ("W_proj", C, H)],
+        "gridtd_lrp": [("W_g2", 3 * H, H, Q), ("W_g1", 2 * H + 2 * E, H, Q), ("W_glob", C, E, Q), ("W_proj", C, H, QP)],
+        "aoa_lrp": [("W_aoa", H, H, Q), ("W_g", E + 2 * H, H, Q), ("W_v", H, H, QP), ("W_proj", C, H, QP)],
+        "adaptive_lrp": [("W_g", 2 * E + H, H, Q), ("W_glob", C, E, Q), ("W_proj", C, H, QP)],
+        "gridtd_grad": [("W2", 3 * H, 4 * H, Q), ("W1", H + 2 * E, 4 * H, Q), ("W_glob", C, E, Q), ("W_proj", C, H, QP)],
+        "aoa_grad": [("W_aoa", H, H, Q), ("W_gate", H, H, Q), ("W_g", E + 2 * H, 4 * H, Q), ("W_v", H, H, QP),
+                     ("W_proj", C, H, QP)],
+        "adaptive_grad": [("W_g", 2 * E + H, 4 * H, Q), ("W_glob", C, E, Q), ("W_proj", C, H, Q)],
     }[kind]
 
 
@@ -60,7 +65,7 @@ def test_route_table_covers_both_routes():
         seen = {}
         fused_states = set()
         for H, E, C in SHAPES:
-            routes = {name: tc_shape_ok(N, K) for name, N, K in gemm_table(kind, H, E, C)}
+            routes = {name: tc_shape_ok(N, K) for name, N, K, _ in gemm_table(kind, H, E, C)}
             for name, tc in routes.items():
                 seen.setdefault(name, set()).add(tc)
             if kind in FUSED:
@@ -74,11 +79,37 @@ def test_route_table_covers_both_routes():
 def test_route_table_edge_cases():
     """The shapes the workspace and wide-grid tests rely on take the routes their docstrings name."""
     # adaptive gradient at (32, 192, 512): only W_glob on the tensor cores, and it splits Q x E with E > 4H
-    routes = {n: tc_shape_ok(N, K) for n, N, K in gemm_table("adaptive_grad", 32, 192, 512)}
+    routes = {n: tc_shape_ok(N, K) for n, N, K, _ in gemm_table("adaptive_grad", 32, 192, 512)}
     assert routes == {"W_g": False, "W_glob": True, "W_proj": False}
     # (64, 64, 64): every GEMM of every decoder on the tensor cores
     for kind in dict.fromkeys(map(_gemm_kind, KINDS)):
-        assert all(tc_shape_ok(N, K) for _, N, K in gemm_table(kind, 64, 64, 64)), kind
+        assert all(tc_shape_ok(N, K) for _, N, K, _ in gemm_table(kind, 64, 64, 64)), kind
+
+
+def test_workspace_holds_weight_copies_and_split_operands():
+    """With tc_gemm the workspace grows by at least the prepared copy of every weight (N x 3K bf16, stored
+    [hi | hi | lo]) plus the largest split operand (rows x 2K bf16, stored [hi | lo]) of the decoder's GEMMs.  A slot
+    sized by a smaller formula lets that split overwrite the slot next to it.  Host calls: no GPU needed."""
+    import ctypes
+    from lrpx import _lib
+    lib = _lib.lib()
+    entry = {"gridtd_lrp": (_lib.GridTDArgs, lib.lrpx_gridtd_decoder_workspace_bytes),
+             "aoa_lrp": (_lib.AoaArgs, lib.lrpx_aoa_decoder_workspace_bytes),
+             "adaptive_lrp": (_lib.AdaptiveArgs, lib.lrpx_adaptive_decoder_workspace_bytes),
+             "gridtd_grad": (_lib.GridTDGradArgs, lib.lrpx_gridtd_decoder_grad_workspace_bytes),
+             "aoa_grad": (_lib.AoaGradArgs, lib.lrpx_aoa_decoder_grad_workspace_bytes),
+             "adaptive_grad": (_lib.AdaptiveGradArgs, lib.lrpx_adaptive_decoder_grad_workspace_bytes)}
+    Q, P = 16, 7
+    for kind in dict.fromkeys(map(_gemm_kind, KINDS)):
+        args_cls, ws_bytes = entry[kind]
+        for H, E, C in SHAPES + [(32, 192, 512), (36, 64, 64), (30, 64, 64)]:
+            dims = dict(B=3, T=5, H=H, E=E, P=P, C=C, V=40, Q=Q)
+            if kind.startswith("aoa"):
+                dims["num_head"] = heads_for(H)
+            size = lambda flags: ws_bytes(ctypes.byref(args_cls(**dims, flags=flags)))
+            table = gemm_table(kind, H, E, C, Q, P)
+            need = sum(2 * N * 3 * K for _, N, K, _ in table) + 2 * max(rows * 2 * K for _, _, K, rows in table)
+            assert size(1) - size(0) >= need, f"{kind} (H, E, C) = {(H, E, C)}"
 
 
 def heads_for(H):
