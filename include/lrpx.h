@@ -660,9 +660,10 @@ typedef struct {
   const float* bn_w;    /* FWDX: folded BatchNorm y = z*bn_w[n] + bn_b[n] (eval mode) and its rule
                          * R = |z w| / (|z w| + |b|) R_out (lrp_modules.py:204-215) as a factor of gain0           */
   const float* bn_b;
-  const void* idn;      /* FWDX: identity branch (bf16 PF, cout channels): out = relu(y + idn), Add rule ratios
-                         * rho1 = y / stab'(y+idn) (factor of gain0), rho2 = idn / stab'(y+idn); out3 = rho2 * hd   */
-  const void* hd;       /* FWDX: bf16 PF factor of the identity-branch gain (the downsample conv's ratio / z+) or NULL */
+  const void* idn;      /* FWDX: identity branch (bf16 PF, cout channels; hi|lo rows of 2*cout when split): out = relu(y + idn),
+                         * Add rule ratios rho1 = y / stab'(y+idn) (factor of gain0), rho2 = idn / stab'(y+idn); out3 = rho2 * hd */
+  const void* hd;       /* FWDX: PF factor of the identity-branch gain (the downsample conv's ratio / z+; bf16, fp32 when
+                         * split) or NULL */
   void* out4;           /* FWDX: act * gain0                                                       */
   void* out5;           /* FWDX: act * out3                                                        */
   int add_pitch;
@@ -761,6 +762,15 @@ int lrpx_tc_stem_col2im_bf16(const void* P, int ldp, const float* x, const int32
                              int w, int mode, void* stream);
 /* lrpx_tc_pf_to_dense_f32 for hi|lo rows of 2*c channels (value = hi + lo) */
 int lrpx_tc_pf_split_to_dense_f32(const void* src, float* dst, int n, int h, int w, int c, int layout, void* stream);
+/* ---- the residual-network stem in the fp32-accurate forward (split = 0: exactly the bf16 functions above) */
+/* lrpx_tc_im2col7s2_split_bf16 with hi|lo rows (split = 1): 640 bf16 [hi of the 320 | lo of the 320], hi + lo ~ the fp32
+ * tap; hi is the bf16 function's row.  The A operand of lrpx_tc_conv(ksize 1, cin 960, a_phys 640, split 1, FWDX) with
+ * weight rows [hi | hi | lo] of [w | w | 0] and [w+ | w- | 0] (models/resnet.py:143-149, lrp_modules.py:81-84). */
+int lrpx_tc_im2col7s2_split_x(const float* x, void* dst, int n, int h, int w, int split, void* stream);
+/* lrpx_tc_maxpool3s2_bf16 on hi|lo rows (split = 1, 2*c bf16 per row): the winner is the largest hi + lo, first maximum in
+ * PyTorch scan order, idx = 255 where the maximum is 0; pooled keeps the winner's hi|lo row (resnet.py:150,
+ * lrp_modules.py:186-191).  lrpx_tc_subsample2_bf16 with c = 2*c serves hi|lo rows as they are. */
+int lrpx_tc_maxpool3s2_x(const void* act, void* pooled, uint8_t* idx, int n, int h, int w, int c, int split, void* stream);
 
 #ifdef __cplusplus
 }

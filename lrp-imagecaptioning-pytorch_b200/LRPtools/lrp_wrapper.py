@@ -225,23 +225,26 @@ def _is_bottleneck_resnet(model):
 
 
 class _TcResNetPlan:
-    """Tensor-core route of ``compute_lrp(precision='bf16')`` for Bottleneck ResNets (alpha=1, beta=0 preset)."""
+    """Tensor-core route of ``compute_lrp(precision='bf16' | 'mixed')`` for Bottleneck ResNets (alpha=1, beta=0 preset):
+    ONE engine per precision, rebuilt when a parameter or buffer changes (data pointer / in-place version)."""
 
     def __init__(self, model):
         self.model = model
         self.convs = [m for m in model.modules() if isinstance(m, nn.Conv2d)]
-        self._eng = None
+        self._eng = {}
 
     def engine(self, precision, lrp_params):
         from lrpx import tc_resnet
-        if precision != "bf16" or float(lrp_params.get("alpha", 1.)) != 1. or float(lrp_params.get("beta", 0.)) != 0. \
-                or not lrp_params.get("ignore_bias", True):
+        if precision not in ("bf16", "mixed") or float(lrp_params.get("alpha", 1.)) != 1. \
+                or float(lrp_params.get("beta", 0.)) != 0. or not lrp_params.get("ignore_bias", True):
             return None
         ps = [p for p in self.model.parameters()] + [b for b in self.model.buffers()]
         stamp = tuple((t.data_ptr(), t._version) for t in ps)
-        if self._eng is None or self._eng[0] != stamp:
-            self._eng = (stamp, tc_resnet.TcResNetEngine(self.model, ps[0].device))
-        return self._eng[1]
+        hit = self._eng.get(precision)
+        if hit is None or hit[0] != stamp:
+            cls = tc_resnet.TcResNetMixed if precision == "mixed" else tc_resnet.TcResNetEngine
+            hit = self._eng[precision] = (stamp, cls(self.model, ps[0].device))
+        return hit[1]
 
 
 class _TcPlan:
@@ -298,7 +301,8 @@ def add_lrp(model):
 #            chain with error-compensated bf16x3 operands and fp32 gains / inter-layer storage; every other
 #            topology runs the fp32 CUDA-core rule kernels.
 #   'bf16' — the tcgen05 chain with bf16 operands and storage (Spearman >= 0.99 / rel-L2 <= 5e-2 vs the reference).
-#   'mixed' — fp32-accurate forward (activations, max-pool winners, gains), bf16 chain: lrpx.tc.TcVggMixed.
+#   'mixed' — fp32-accurate forward (activations, max-pool winners, gains), bf16 chain: lrpx.tc.TcVggMixed, and for
+#            Bottleneck ResNets lrpx.tc_resnet.TcResNetMixed (alpha 1 / beta 0 / ignore_bias preset only).
 #   'simt' — the fp32 CUDA-core rule kernels whatever the topology (the rule-by-rule walker).
 DEFAULT_PRECISION = os.environ.get("LRPX_PRECISION", "fp32")
 
@@ -330,14 +334,16 @@ def compute_lrp(model, sample, target=None, return_output=False, rectify_logits=
                        and params.get("ignore_bias", True))
         preset = params.get("alpha", 1.) == 1. and params.get("beta", 0.) == 0. and params.get("ignore_bias", True)
         if precision == "mixed":
-            use_tc = use_tc and preset and not isinstance(tcp, _TcResNetPlan) and tcp.convs[0].out_channels % 64 == 0
+            use_tc = use_tc and preset and (isinstance(tcp, _TcResNetPlan) or tcp.convs[0].out_channels % 64 == 0)
         if isinstance(tcp, _TcResNetPlan):
-            use_tc = use_tc and not general and not model.training   # ResNets: the bf16 chain only
+            # ResNets: the bf16 chain only, on the bf16 ('bf16') or the fp32-accurate ('mixed') forward
+            use_tc = use_tc and (not general or precision == "mixed") and not model.training
         elif general and tcp.convs[0].out_channels % 64:
             use_tc = False                    # the general kernels need a 64-channel first layer: CUDA-core walker
     if precision in ("bf16", "mixed") and not use_tc:
         raise NotImplementedError(f"compute_lrp(precision={precision!r}): the tensor-core chain covers VGG-style encoders "
-                                  "(conv3x3/ReLU/max-pool 2x2) under the alpha-beta rule only ('mixed': alpha 1 / beta 0)")
+                                  "(conv3x3/ReLU/max-pool 2x2) under the alpha-beta rule and Bottleneck ResNets under "
+                                  "alpha 1 / beta 0 ('mixed': alpha 1 / beta 0 on both)")
     with torch.no_grad():
         x = sample.detach()
         if use_tc:

@@ -105,8 +105,8 @@ struct TcParams {
   const void* gain4; // MULX: gainB of group 1
   const float* bn_w; // FWDX: folded BatchNorm scale / shift per output channel (nullptr: plain bias)
   const float* bn_b;
-  const void* idn;   // FWDX: residual identity branch (bf16 PF, cout channels): Add rule ratios
-  const void* hd;    // FWDX: per-element factor of the identity-branch gain (bf16 PF) or nullptr
+  const void* idn;   // FWDX: residual identity branch (bf16 PF, cout channels; hi|lo rows when split): Add rule ratios
+  const void* hd;    // FWDX: per-element factor of the identity-branch gain (bf16 PF, fp32 when split) or nullptr
   void* out4;        // FWDX: act * gain0
   void* out5;        // FWDX: act * (identity-branch gain)
   int fwd_flags;     // FWDX: bit 0 = no ReLU, bit 1 = store only the even pixels into a half-resolution PF tensor
@@ -899,6 +899,9 @@ __device__ __forceinline__ void epi_fwdx_simple(const TcParams& p, const RowInfo
   }
 }
 
+// SPLIT_ADD: the residual operands of the fp32-accurate (split) forward, instantiated on its own (TC_EPI_FWDX_SPLIT_ADD)
+// so that the bf16 form keeps its registers and spills
+template <bool SPLIT_ADD>
 __device__ __forceinline__ void epi_fwdx(const TcParams& p, const RowInfo& r, uint32_t taddr, int n_tile, int c,
                                          uint32_t release_bar) {
   const bool sp = p.split != 0;
@@ -945,8 +948,19 @@ __device__ __forceinline__ void epi_fwdx(const TcParams& p, const RowInfo& r, ui
 #pragma unroll
     for (int k = 0; k < 16; ++k) { idv[k] = 0.f; hdv[k] = 1.f; }
     const size_t go = orow * cout + ch;
-    if (p.idn && r.valid) load_bf16x16(p.idn, go, idv);
-    if (p.hd && r.valid) load_bf16x16(p.hd, go, hdv);
+    if (SPLIT_ADD) {
+      // idn is a hi|lo row of 2*cout (its value hi + lo; hdv holds lo for the moment), hd an fp32 gain (store_gain16, split)
+      if (p.idn && r.valid) {
+        load_bf16x16(p.idn, orow * (2 * cout) + ch, idv);
+        load_bf16x16(p.idn, orow * (2 * cout) + cout + ch, hdv);
+#pragma unroll
+        for (int k = 0; k < 16; ++k) { idv[k] += hdv[k]; hdv[k] = 1.f; }
+      }
+      if (p.hd && r.valid) load_gain16(p.hd, go, true, hdv);
+    } else {
+      if (p.idn && r.valid) load_bf16x16(p.idn, go, idv);
+      if (p.hd && r.valid) load_bf16x16(p.hd, go, hdv);
+    }
     float act[16], g0[16], g1[16], ag0[16], ag1[16];
 #pragma unroll
     for (int k = 0; k < 16; ++k) {
@@ -1067,13 +1081,15 @@ __device__ __forceinline__ void epi_mul_fold(const TcParams& p, const RowInfo& r
 constexpr int TC_EPI_FWDX_SIMPLE = 12;
 constexpr int TC_EPI_MUL_FOLD = 15;         // MUL with the three filter COLUMNS folded into N (64-channel layers, epi_mul_fold)
 constexpr int TC_EPI_MULX_S = 13, TC_EPI_MULX_UNPOOL_S = 14;      // MULX / MULX_UNPOOL with one gain group, no addend (epi_mulx)
+constexpr int TC_EPI_FWDX_SPLIT_ADD = 16;   // FWDX with split rows and a residual operand (idn / hd): epi_fwdx<true>
 
 // number of 32-column units per (lane quarter, M half) of a tile
 __device__ __forceinline__ int epi_units_per_half(const TcParams& p, int epi) {
   if (epi == LRPX_TC_EPI_INPUT || epi == LRPX_TC_EPI_INPUT3) return 1;
   if (epi == TC_EPI_MUL_FOLD) return 4;                   // four units of 16 output channels (`c` counts 32 per unit: c >> 1)
   if (epi == TC_EPI_FWDX_SIMPLE) return p.half >> 4;      // 16-column units (run_epilogue_tile: c = u << 4)
-  const int ncols = (epi == LRPX_TC_EPI_FWD_GAIN || epi == LRPX_TC_EPI_FWDX || epi == TC_EPI_FWDX_SIMPLE) ? p.half : p.bn;
+  const int ncols = (epi == LRPX_TC_EPI_FWD_GAIN || epi == LRPX_TC_EPI_FWDX || epi == TC_EPI_FWDX_SIMPLE ||
+                     epi == TC_EPI_FWDX_SPLIT_ADD) ? p.half : p.bn;
   return ncols >> 5;
 }
 
@@ -1108,7 +1124,9 @@ __device__ __forceinline__ void epi_unit(const TcParams& p, const RowInfo& r0, u
   } else if (EPI == TC_EPI_FWDX_SIMPLE) {
     epi_fwdx_simple(p, r, taddr, n_tile, c, release_bar);
   } else if (EPI == LRPX_TC_EPI_FWDX) {
-    epi_fwdx(p, r, taddr, n_tile, c, release_bar);
+    epi_fwdx<false>(p, r, taddr, n_tile, c, release_bar);
+  } else if (EPI == TC_EPI_FWDX_SPLIT_ADD) {
+    epi_fwdx<true>(p, r, taddr, n_tile, c, release_bar);
   } else if (EPI == LRPX_TC_EPI_INPUT) {
     uint32_t v[16];
     TMEM_LD_X16(taddr, v);
@@ -2371,6 +2389,7 @@ extern "C" int lrpx_tc_conv(const lrpx_tc_conv_args* a, void* stream) {
           return launch_tc_slab<LRPX_TC_EPI_MULX_UNPOOL>(ma0, ma1, mb, mbh, mo, p, grid, st);
         case LRPX_TC_EPI_FWDX:
           if (p.fwd_simple) return launch_tc_slab<TC_EPI_FWDX_SIMPLE>(ma0, ma1, mb, mbh, mo, p, grid, st);
+          if (p.split && (p.idn || p.hd)) return launch_tc_slab<TC_EPI_FWDX_SPLIT_ADD>(ma0, ma1, mb, mbh, mo, p, grid, st);
           return launch_tc_slab<LRPX_TC_EPI_FWDX>(ma0, ma1, mb, mbh, mo, p, grid, st);
         default: return launch_tc_slab<LRPX_TC_EPI_STORE_F32>(ma0, ma1, mb, mbh, mo, p, grid, st);
       }
@@ -2407,6 +2426,7 @@ extern "C" int lrpx_tc_conv(const lrpx_tc_conv_args* a, void* stream) {
       return launch_tc<LRPX_TC_EPI_MULX_UNPOOL>(ma, mb, p, grid, st);
     case LRPX_TC_EPI_FWDX:
       if (p.fwd_simple) return launch_tc<TC_EPI_FWDX_SIMPLE>(ma, mb, p, grid, st);
+      if (p.split && (p.idn || p.hd)) return launch_tc<TC_EPI_FWDX_SPLIT_ADD>(ma, mb, p, grid, st);
       return launch_tc<LRPX_TC_EPI_FWDX>(ma, mb, p, grid, st);
     default: return launch_tc<LRPX_TC_EPI_STORE_F32>(ma, mb, p, grid, st);
   }

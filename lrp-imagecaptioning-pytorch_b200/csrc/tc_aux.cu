@@ -606,6 +606,41 @@ __global__ void im2col7s2_split_kernel(const float* __restrict__ x, uint4* __res
   }
 }
 
+// the same im2col with hi|lo rows: 640 bf16 [hi of the 320 | lo of the 320], hi + lo ~ the fp32 tap (the A operand of the
+// error-compensated stem, a_phys = 640 under K = 960).  hi is what im2col7s2_split_kernel writes.
+__global__ void im2col7s2_split_x_kernel(const float* __restrict__ x, uint4* __restrict__ dst, int n, int h, int w) {
+  const int ho = h / 2, wo = w / 2, wp1 = wo + 1, blk = (ho + 1) * wp1;
+  const long long total = (long long)n * blk * 40;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const int cg = (int)(i % 40);
+    const long long prow = i / 40;
+    const int img = (int)(prow / blk), rem = (int)(prow % blk);
+    const int a = rem / wp1, b = rem % wp1;
+    uint32_t hi[4] = {0u, 0u, 0u, 0u}, lo[4] = {0u, 0u, 0u, 0u};
+    if (a > 0 && b > 0) {
+      const float* xi = x + (size_t)img * 3 * h * w;
+      float v[8];
+#pragma unroll
+      for (int k = 0; k < 8; ++k) {
+        const int e = cg * 8 + k;
+        float f = 0.f;
+        if (e < 294) {
+          const int t = e < 147 ? e : e - 147;
+          const int ci = t / 49, ky = (t % 49) / 7, kx = t % 7;
+          const int yy = 2 * (a - 1) - 3 + ky, xs = 2 * (b - 1) - 3 + kx;
+          const float xv = (yy >= 0 && yy < h && xs >= 0 && xs < w) ? __ldg(xi + ((size_t)ci * h + yy) * w + xs) : 0.f;
+          f = e < 147 ? fmaxf(xv, 0.f) : fminf(xv, 0.f);
+        }
+        v[k] = f;
+      }
+#pragma unroll
+      for (int k = 0; k < 4; ++k) split2(v[2 * k], v[2 * k + 1], hi[k], lo[k]);
+    }
+    dst[prow * 80 + cg] = make_uint4(hi[0], hi[1], hi[2], hi[3]);
+    dst[prow * 80 + 40 + cg] = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+  }
+}
+
 // 3x3 / stride 2 / pad 1 max-pool on PF bf16 (post-ReLU input), 8 channels per thread.  Window of output (y,x): input rows
 // 2y-1..2y+1, columns 2x-1..2x+1, padding skipped (PyTorch pads with -inf); scan order (ky,kx) row-major, strict '>' so
 // the first maximum wins (max_pool2d_with_indices).  idx = ky*3+kx of the winner, 255 when the maximum is 0: such a
@@ -652,6 +687,59 @@ __global__ void maxpool3s2_pf_kernel(const uint4* __restrict__ act, uint4* __res
       for (int e = 0; e < 8; ++e) ov[e >> 1] |= bb[e] << (16 * (e & 1));
     }
     pooled[i] = make_uint4(ov[0], ov[1], ov[2], ov[3]);
+    idx[i] = make_uint2(bi[0] | (bi[1] << 8) | (bi[2] << 16) | (bi[3] << 24), bi[4] | (bi[5] << 8) | (bi[6] << 16) | (bi[7] << 24));
+  }
+}
+
+// the same pool on hi|lo rows (2*c bf16 per row): the winner is the largest hi + lo (exact in fp32), same scan order and
+// 255 rule; pooled keeps the winner's hi and lo.
+__global__ void maxpool3s2_x_kernel(const uint4* __restrict__ act, uint4* __restrict__ pooled, uint2* __restrict__ idx,
+                                    int n, int h, int w, int c8) {
+  const int oh = h / 2, ow = w / 2, wp1 = w + 1, owp1 = ow + 1;
+  const long long blk_f = (long long)(h + 1) * wp1, blk_p = (long long)(oh + 1) * owp1;
+  const long long total = (long long)n * blk_p * c8;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const long long prow = i / c8;
+    const int cc = (int)(i - prow * c8);
+    const long long img = prow / blk_p;
+    const int rem = (int)(prow - img * blk_p);
+    const int a = rem / owp1, b = rem - a * owp1;
+    uint32_t ohi[4] = {0u, 0u, 0u, 0u}, olo[4] = {0u, 0u, 0u, 0u};
+    uint32_t bi[8];
+#pragma unroll
+    for (int e = 0; e < 8; ++e) bi[e] = 255u;
+    if (a > 0 && b > 0) {
+      float best[8];
+      uint32_t bh[8], bl[8];
+#pragma unroll
+      for (int e = 0; e < 8; ++e) { best[e] = 0.f; bh[e] = 0u; bl[e] = 0u; }
+#pragma unroll
+      for (int ky = 0; ky < 3; ++ky) {
+        const int fa = 2 * (a - 1) + ky;
+        if (fa < 1) continue;
+#pragma unroll
+        for (int kx = 0; kx < 3; ++kx) {
+          const int fb = 2 * (b - 1) + kx;
+          if (fb < 1) continue;
+          const long long fr = (img * blk_f + (long long)fa * wp1 + fb) * 2 * c8;
+          const uint4 vh = act[fr + cc], vl = act[fr + c8 + cc];
+          const uint32_t hw[4] = {vh.x, vh.y, vh.z, vh.w}, lw[4] = {vl.x, vl.y, vl.z, vl.w};
+#pragma unroll
+          for (int e = 0; e < 8; ++e) {
+            const uint32_t hb = (hw[e >> 1] >> (16 * (e & 1))) & 0xFFFFu, lb = (lw[e >> 1] >> (16 * (e & 1))) & 0xFFFFu;
+            const float f = __uint_as_float(hb << 16) + __uint_as_float(lb << 16);
+            if (f > best[e]) { best[e] = f; bh[e] = hb; bl[e] = lb; bi[e] = (uint32_t)(ky * 3 + kx); }
+          }
+        }
+      }
+#pragma unroll
+      for (int e = 0; e < 8; ++e) {
+        ohi[e >> 1] |= bh[e] << (16 * (e & 1));
+        olo[e >> 1] |= bl[e] << (16 * (e & 1));
+      }
+    }
+    pooled[prow * 2 * c8 + cc] = make_uint4(ohi[0], ohi[1], ohi[2], ohi[3]);
+    pooled[prow * 2 * c8 + c8 + cc] = make_uint4(olo[0], olo[1], olo[2], olo[3]);
     idx[i] = make_uint2(bi[0] | (bi[1] << 8) | (bi[2] << 16) | (bi[3] << 24), bi[4] | (bi[5] << 8) | (bi[6] << 16) | (bi[7] << 24));
   }
 }
@@ -836,6 +924,24 @@ int lrpx_tc_subsample2_bf16(const void* src, void* dst, int n, int h, int w, int
   LRPX_CHECK_ARG(src && dst && n > 0 && h > 0 && w > 0 && h % 2 == 0 && w % 2 == 0 && c % 8 == 0, "bad argument");
   long long total = (long long)n * (h / 2 + 1) * (w / 2 + 1) * (c / 8);
   subsample2_pf_kernel<<<grid_for(total), 256, 0, as_stream(stream)>>>((const uint4*)src, (uint4*)dst, n, h, w, c / 8);
+  LRPX_CHECK_LAUNCH();
+  return LRPX_OK;
+}
+
+int lrpx_tc_im2col7s2_split_x(const float* x, void* dst, int n, int h, int w, int split, void* stream) {
+  if (!split) return lrpx_tc_im2col7s2_split_bf16(x, dst, n, h, w, stream);
+  LRPX_CHECK_ARG(x && dst && n > 0 && h > 0 && w > 0 && h % 2 == 0 && w % 2 == 0, "bad argument (h, w even)");
+  long long total = (long long)n * (h / 2 + 1) * (w / 2 + 1) * 40;
+  im2col7s2_split_x_kernel<<<grid_for(total), 256, 0, as_stream(stream)>>>(x, (uint4*)dst, n, h, w);
+  LRPX_CHECK_LAUNCH();
+  return LRPX_OK;
+}
+
+int lrpx_tc_maxpool3s2_x(const void* act, void* pooled, uint8_t* idx, int n, int h, int w, int c, int split, void* stream) {
+  if (!split) return lrpx_tc_maxpool3s2_bf16(act, pooled, idx, n, h, w, c, stream);
+  LRPX_CHECK_ARG(act && pooled && idx && n > 0 && h > 0 && w > 0 && h % 2 == 0 && w % 2 == 0 && c % 8 == 0, "bad argument");
+  long long total = (long long)n * (h / 2 + 1) * (w / 2 + 1) * (c / 8);
+  maxpool3s2_x_kernel<<<grid_for(total), 256, 0, as_stream(stream)>>>((const uint4*)act, (uint4*)pooled, (uint2*)idx, n, h, w, c / 8);
   LRPX_CHECK_LAUNCH();
   return LRPX_OK;
 }

@@ -204,6 +204,8 @@ SYMBOLS = {
     "lrpx_tc_subsample2_bf16": (_i, [_P, _P, _i, _i, _i, _i, _P]),
     "lrpx_tc_stem_col2im_f32": (_i, [_P, _i, _P, _P, _P, _i, _i, _i, _i, _P]),
     "lrpx_tc_stem_col2im_bf16": (_i, [_P, _i, _P, _P, _P, _i, _i, _i, _i, _P]),
+    "lrpx_tc_im2col7s2_split_x": (_i, [_P, _P, _i, _i, _i, _i, _P]),
+    "lrpx_tc_maxpool3s2_x": (_i, [_P, _P, _P, _i, _i, _i, _i, _i, _P]),
 }
 
 _lib = None

@@ -18,14 +18,14 @@ from . import _graph, ops
 class BatchExplainer:
     def __init__(self, explainer, chunk=128, use_graph=False, tc_gemm=None, head_idx=0, deliver="full"):
         """explainer: models.gridTDmodel.ExplainGridTDAttention, models.aoamodel.ExplainAOAAttention or
-        models.adaptiveattention.ExplainAdaptiveAttention on a VGG encoder with precision 'fp32' (fp32-accurate chain)
-        or 'bf16'; ``head_idx``: the attention head an AoA explanation follows (aoamodel.py:1165,
+        models.adaptiveattention.ExplainAdaptiveAttention on a VGG encoder with precision 'fp32' (fp32-accurate chain),
+        'bf16' or 'mixed', or on a Bottleneck-ResNet encoder with precision 'bf16' or 'mixed'; ``head_idx``: the attention head an AoA explanation follows (aoamodel.py:1165,
         ``explain_caption(img, head_idx)``); ``deliver``: format of the heat-maps (TcVggEngine.heat_shape): 'full' =
         fp32 (Q,3,H,W) like the reference, 'channel_mean' = fp32 (Q,H,W), 'fp16'; ``tc_gemm``: decoder GEMMs as bf16x3
         on tensor cores (default: with precision 'bf16') or on fp32 CUDA cores."""
         if not getattr(explainer, "uses_tc", False):
-            raise ValueError("BatchExplainer drives the tensor-core chain: it needs a VGG-style encoder and "
-                             "precision='fp32' (fp32-accurate mode) or 'bf16'")
+            raise ValueError("BatchExplainer drives the tensor-core chain: it needs a VGG-style encoder with "
+                             "precision 'fp32', 'bf16' or 'mixed', or a Bottleneck ResNet with 'bf16' or 'mixed'")
         self.ex = explainer
         # gradient-family explainers (models/_gradient.py): same pipeline, the decoder-gradient kernels and the chain's
         # 'gradient' / 'guided' rule instead of the relevance ones

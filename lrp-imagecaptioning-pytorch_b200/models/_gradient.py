@@ -125,8 +125,8 @@ class GradientFamily:
     def _check_encoder(self):
         # Bottleneck ResNets: the fp32 CUDA-core path only (LRPtools.lrp_wrapper.encoder_gradient_simt)
         if getattr(self, "is_resnet", False) and self.precision in ("bf16", "mixed"):
-            raise NotImplementedError("ResNet encoders: the gradient-family explainers run on the fp32 CUDA-core kernels "
-                                      "(precision 'fp32' or 'simt')")
+            raise NotImplementedError(f"precision={self.precision!r}: on a ResNet encoder the gradient-family explainers "
+                                      "support precision 'fp32' and 'simt' (the fp32 CUDA-core kernels)")
 
     def explainer_forward(self, feat, tokens, quirk_double_bias_ih=False, want_gates=True):
         # the gradient explainers' LSTM forwards add bias_ih + bias_hh (gridTDmodel.py:1265): no Q3 here

@@ -509,11 +509,12 @@ class ExplainGridTDAttention(object):
       'fp32' — the reference's fp32 bar.  VGG encoders: the tcgen05 chain in its fp32-accurate mode (error-compensated
                bf16x3 operands, fp32 gains, hi|lo inter-layer storage); other encoders: the fp32 CUDA-core rule kernels
                through LRPtools.  Decoder GEMMs on fp32 CUDA cores.
-      'bf16' — VGG encoders only: the tcgen05 chain with bf16 operands / storage (Spearman >= 0.99, rel-L2 <= 5e-2 vs
-               the reference), decoder GEMMs as bf16x3 on tensor cores.  The throughput mode of bench.py.
-      'mixed' — VGG encoders: the encoder FORWARD in the fp32-accurate mode (once per image), the relevance chain in
-               bf16 (lrpx.tc.TcVggMixed): accurate features for the decoder and accurate max-pool winners at ~0.85 of
-               the bf16 mode's throughput.
+      'bf16' — VGG and Bottleneck-ResNet encoders: the tcgen05 chain with bf16 operands / storage (Spearman >= 0.99,
+               rel-L2 <= 5e-2 vs the reference), decoder GEMMs as bf16x3 on tensor cores.  The throughput mode of
+               bench.py.
+      'mixed' — VGG and Bottleneck-ResNet encoders: the encoder FORWARD in the fp32-accurate mode (once per image),
+               the relevance chain in bf16 (lrpx.tc.TcVggMixed, lrpx.tc_resnet.TcResNetMixed): accurate features for
+               the decoder, accurate max-pool winners and, on a ResNet, Add-rule ratios formed from accurate sums.
       'simt' — the fp32 CUDA-core rule kernels through LRPtools whatever the encoder."""
     EPS = LRPutil.EPSILON
     EX_TYPE = 'lrp'
@@ -552,15 +553,17 @@ class ExplainGridTDAttention(object):
         tcp = lrp_wrapper._tc_cfg(self.model.img_encoder.encoder) if is_vgg else None
         # the general kernels (fp32-accurate mode) need a first conv with a multiple of 64 output channels
         tc_ok = tcp is not None and (self.precision == 'bf16' or tcp[0][0].out_channels % 64 == 0)
-        # Bottleneck ResNets run the bf16 chain of lrpx.tc_resnet (their fp32 bar is the CUDA-core rule path)
+        # Bottleneck ResNets run the bf16 chain of lrpx.tc_resnet on a bf16 or fp32-accurate forward (their fp32 bar
+        # is the CUDA-core rule path)
         self.is_resnet = self.has_encoder and lrp_wrapper._is_bottleneck_resnet(self.model.img_encoder.encoder)
-        if self.is_resnet and self.precision == 'bf16':
+        if self.is_resnet and self.precision in ('bf16', 'mixed'):
             tc_ok = True
         if self.precision == 'bf16' and not tc_ok and self.has_encoder:
             raise NotImplementedError("the tensor-core chain supports VGG-style encoders; use precision='fp32'")
         # the encoder runs on the tcgen05 engine (one forward per image shared by all its words)
-        if self.precision == 'mixed' and not (tc_ok and not self.is_resnet):
-            raise NotImplementedError("precision='mixed' needs a VGG-style encoder with a 64-channel first layer")
+        if self.precision == 'mixed' and not tc_ok:
+            raise NotImplementedError("precision='mixed' needs a VGG-style encoder with a 64-channel first layer or a "
+                                      "Bottleneck ResNet")
         self.uses_tc = tc_ok and self.precision in ('fp32', 'bf16', 'mixed')
         self.mean = [0.485, 0.456, 0.406]
         self.std = [0.229, 0.224, 0.225]
@@ -611,7 +614,8 @@ class ExplainGridTDAttention(object):
         self._engine_key = key
         if self._engine is None and getattr(self, "is_resnet", False):
             from lrpx import tc_resnet
-            self._engine = tc_resnet.TcResNetEngine(self.model.img_encoder.encoder, self.device)
+            cls = tc_resnet.TcResNetMixed if self.precision == 'mixed' else tc_resnet.TcResNetEngine
+            self._engine = cls(self.model.img_encoder.encoder, self.device)
         if self._engine is None:
             from lrpx import tc
             enc = self.model.img_encoder.encoder
