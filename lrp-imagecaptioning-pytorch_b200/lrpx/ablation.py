@@ -37,13 +37,6 @@ class AblationExperiments:
         """relevance (H, W) -> mask (H, W), the reference's signature (one map)."""
         return ops.block_image(relevance.reshape(1, 1, *relevance.shape), self.num_delete_patches, self.patch_size)[0]
 
-    def _searcher(self):
-        from . import beam
-        ex = self.ex
-        if getattr(ex, "_beam", None) is None:
-            ex._beam = getattr(beam, ex._BEAM)(ex.model)
-        return ex._beam
-
     def _teacher_forced_scores(self, feat, prefixes, words):
         """softmax score of ``words[i]`` as the next word after ``prefixes[i]`` (token lists starting with <start>) for
         the images with features ``feat`` (n,P,C): evaluation.py:139-142 (teacherforce_forward + softmax of the last row)."""
@@ -72,7 +65,7 @@ class AblationExperiments:
                                         want_mask=False)
             orig = torch.softmax(pred[req_img.long(), req_t.long()], dim=-1).gather(
                 1, torch.tensor(words, device=dev).view(-1, 1))[:, 0]
-            searcher = self._searcher()
+            searcher = ex._searcher()
             caps, feats = [], []
             for q0 in range(0, Q, self.chunk):
                 est = eng.forward(masked[q0:q0 + self.chunk])

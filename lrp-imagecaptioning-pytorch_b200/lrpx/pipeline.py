@@ -8,11 +8,28 @@ word decoder relevance + encoder relevance) is done here for B images x T words 
   all B*T requests  ->  encoder relevance chain (tcgen05)  ->  heat-maps (B*T,3,H,W) + r_words (B*T,T)
 
 Optionally the whole pass is captured once into a CUDA graph (fixed B and caption length) and replayed, which
-removes the launch latency of the ~2.7k small kernels of the decoder phases.
+removes the launch latency of the ~2.7k small kernels of the decoder phases.  ``explain_images`` first captions the
+images with the device beam search on the features of the same encoder pass.
 """
+from dataclasses import dataclass
+
 import torch
 
 from . import _graph, ops
+
+
+@dataclass
+class ImageExplanation:
+    """``BatchExplainer.explain_images`` for B images: Q = sum(words_per_image) requests over captions of at most T
+    words."""
+    captions: list            # B token lists without <start>: explain_caption's beam_caption_encode[1:]
+    tokens: torch.Tensor      # (B, T+1) long: <start>, the caption, 0-padding
+    words_per_image: tuple    # the B caption lengths
+    req_img: torch.Tensor     # (Q,) int32: request q explains word req_t[q] + 1 of image req_img[q], image-major
+    req_t: torch.Tensor       # (Q,) int32
+    heat: torch.Tensor        # the Q heat-maps in the ``deliver`` format
+    r_words: torch.Tensor     # (Q, T) relevance of the preceding words
+    pred: torch.Tensor        # (B, T, V) logits of the explainer forward (AblationExperiments.image_ablation's pred)
 
 
 class BatchExplainer:
@@ -74,7 +91,11 @@ class BatchExplainer:
 
     def _run(self, imgs, tokens, req_img, req_t, heat, host=None):
         est = self.eng.forward(imgs)
-        feat = self.eng.features(est, "pixel")
+        return self._explain_encoded(est, self.eng.features(est, "pixel"), tokens, req_img, req_t, heat, host)[0]
+
+    def _explain_encoded(self, est, feat, tokens, req_img, req_t, heat, host=None):
+        """Everything after the encoder forward: explainer forward on ``feat`` (the pixel-major features of the encoder
+        state ``est``), decoder kernels, relevance chain into ``heat``.  -> (r_words, the explainer forward's logits)."""
         st = self.ex.explainer_forward(feat, tokens)
         req_word = tokens[req_img.long(), req_t.long() + 1].to(torch.int32)       # the word each request explains
         if self.is_gradient and self.is_aoa:
@@ -97,7 +118,7 @@ class BatchExplainer:
                                                      ws_cache=self._dec_ws)
         if host is None:
             self.eng.relevance(est, r_feat, req_img, chunk=self.chunk, out=heat, deliver=self.deliver)
-            return r_words
+            return r_words, st["pred"]
         # results go to pinned host buffers: the copy of chunk i runs on a side stream under the kernels of chunk i+1
         host_heat, host_words = host
         main = torch.cuda.current_stream()
@@ -117,7 +138,7 @@ class BatchExplainer:
             host_words.copy_(r_words, non_blocking=True)
         self.eng.relevance(est, r_feat, req_img, chunk=self.chunk, out=heat, on_chunk=on_chunk, deliver=self.deliver)
         main.wait_stream(side)
-        return r_words
+        return r_words, st["pred"]
 
     def explain(self, imgs, tokens, out=None, host_out=None, words_per_image=None):
         """imgs (B,3,H,W) fp32 (CUDA, or pinned host memory), tokens (B,T+1) long with column 0 = <start>.
@@ -132,11 +153,7 @@ class BatchExplainer:
         dev = self.ex.device
         wpi = None if words_per_image is None else tuple(int(v) for v in words_per_image)
         Q = B * T if wpi is None else sum(wpi)
-        # heat-map buffer in the delivery format (the engine's image size is known after its first forward; before
-        # that it is the size of these images)
-        H, W = int(imgs.shape[2]), int(imgs.shape[3])
-        shp = (Q, H, W) if self.deliver == "channel_mean" else (Q, 3, H, W)
-        dt = torch.float16 if self.deliver == "fp16" else torch.float32
+        shp, dt = self._heat_shape(imgs, Q)
         if Q == 0:                                               # nothing to explain
             return (torch.empty((0,) + shp[1:], device=dev, dtype=dt), torch.empty(0, T, device=dev))
         if not self.use_graph:
@@ -170,6 +187,56 @@ class BatchExplainer:
         s_toks.copy_(tokens, non_blocking=True)
         graph.replay()
         return heat, r_words
+
+    def explain_images(self, imgs, beam_size=None, max_cap_length=None, out=None, host_out=None):
+        """Captions B images with the explainer's device beam search and explains every word of every caption: what
+        ``explain_caption`` does for one image, for a batch.  The encoder runs once: the search reads the features of
+        that pass and the explanation reuses its state, so the captions are the ones the per-image API explains (a
+        search through ``model.beam_search_device`` encodes the images a second time, with the library forward).
+
+        imgs (B,3,H,W) fp32 (CUDA, or pinned host memory).  ``beam_size`` / ``max_cap_length`` default to the
+        explainer's ``CAPTION_SEARCH``, the search of its ``get_hidden_parameters``.  The requests are the (image, word)
+        pairs of the captions in image-major order, as ``explain(..., words_per_image=...)`` orders them; an image whose
+        caption is empty (<end> first) has none.  ``out`` (heat-maps) and ``host_out=(heat_host, words_host)`` (pinned;
+        filled as ``explain`` fills them) need room for the result, which goes to their first Q rows and to the first T
+        columns of ``words_host``: B * max_cap_length rows and max_cap_length columns always suffice.
+        Runs eagerly even with ``use_graph``: the search replays its own CUDA graphs, and a graph of the explanation
+        would be captured anew for every pattern of caption lengths.  -> ImageExplanation."""
+        self._sync_weights()
+        ex, dev = self.ex, self.ex.device
+        beam_size = ex.CAPTION_SEARCH[0] if beam_size is None else beam_size
+        max_cap_length = ex.CAPTION_SEARCH[1] if max_cap_length is None else max_cap_length
+        imgs = imgs.to(dev, non_blocking=True)
+        B = imgs.shape[0]
+        est = self.eng.forward(imgs)
+        feat = self.eng.features(est, "pixel")
+        with torch.no_grad():
+            proj, glob = ex._search_inputs(feat)
+        captions = ex._searcher().search(proj, glob, ex.word_map, beam_size=beam_size, max_cap_length=max_cap_length)
+        wpi = tuple(len(c) for c in captions)
+        T, Q = max(wpi), sum(wpi)
+        start = ex.word_map['<start>']
+        tokens = torch.tensor([[start] + c + [0] * (T - len(c)) for c in captions], dtype=torch.long, device=dev)
+        req_img, req_t = self._requests(B, T, dev, wpi)
+        shp, dt = self._heat_shape(imgs, Q)
+        if Q == 0:                                               # nothing to explain: explain's empty results
+            heat, r_words = torch.empty(shp, device=dev, dtype=dt), torch.empty(0, T, device=dev)
+            pred = torch.empty(B, T, ex.model.fc.out_features, device=dev)
+        else:
+            bufs = ([] if out is None else [out]) + ([] if host_out is None else list(host_out))
+            if any(b.shape[0] < Q for b in bufs) or (host_out is not None and host_out[1].shape[1] < T):
+                raise ValueError(f"out / host_out hold fewer than the {Q} requests of {T} words found")
+            heat = torch.empty(shp, device=dev, dtype=dt) if out is None else out[:Q]
+            host = None if host_out is None else (host_out[0][:Q], host_out[1][:Q, :T])
+            r_words, pred = self._explain_encoded(est, feat, tokens, req_img, req_t, heat, host)
+        return ImageExplanation(captions, tokens, wpi, req_img, req_t, heat, r_words, pred)
+
+    def _heat_shape(self, imgs, Q):
+        """(shape, dtype) of Q heat-maps in the delivery format (the engine's image size is known after its first
+        forward; before that it is the size of these images)"""
+        H, W = int(imgs.shape[2]), int(imgs.shape[3])
+        shp = (Q, H, W) if self.deliver == "channel_mean" else (Q, 3, H, W)
+        return shp, (torch.float16 if self.deliver == "fp16" else torch.float32)
 
     def _stage_host_images(self, imgs, s_imgs):
         """Host images reach the graph's static input through one of two device staging buffers: the host->device copy

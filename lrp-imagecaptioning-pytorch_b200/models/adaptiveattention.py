@@ -285,21 +285,16 @@ class ExplainAdaptiveAttention(ExplainGridTDAttention):
         return self.explainer_forward(feat, toks)["pred"][0]
 
     # ------------------------------------------------------------------ reference entry points
-    def get_hidden_parameters(self, img_filepath):
-        """reference :626-677 (beam size 3, at most 20 words)."""
-        self._caption_state(img_filepath, beam_size=3)
+    CAPTION_SEARCH = (3, 20)              # get_hidden_parameters, reference :626-677
 
     def forward_greedy(self, img_filepath):
         """reference :567-624: the same saved state for the beam-size-1 caption."""
-        self._caption_state(img_filepath, beam_size=1)
+        self.img = self.preprocess_img(img_filepath)
+        enc = self._find_caption(img_filepath, beam_size=1, max_cap_length=20)
+        self._set_state(self.img, self.beam_caption_encode, enc)
 
     _BEAM = "AdaptiveBeamSearch"
     _REMOVE_BAD_ENDINGS = False           # this model's beam search keeps the sentence as it is (:444-446)
-
-    def _caption_state(self, img_filepath, beam_size):
-        self.img = self.preprocess_img(img_filepath)
-        enc = self._find_caption(img_filepath, beam_size=beam_size, max_cap_length=20)
-        self._set_state(self.img, self.beam_caption_encode, enc)
 
     def _set_state(self, img, tokens, enc=None):
         if self._empty_caption(tokens):

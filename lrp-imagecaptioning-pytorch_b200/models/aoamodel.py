@@ -442,6 +442,7 @@ class ExplainAOAAttention(ExplainGridTDAttention):
         return st
 
     _BEAM = "AoaBeamSearch"
+    CAPTION_SEARCH = (3, 20)
 
     def _search_inputs(self, feat):
         m = self.model
@@ -449,11 +450,6 @@ class ExplainAOAAttention(ExplainGridTDAttention):
         Wp = m.img_projector.weight.reshape(m.hidden_dim, -1)
         proj = torch.addmm(m.img_projector.bias, feat.reshape(B * P, C), Wp.t()).clamp(min=0).view(B, P, -1)   # (B,P,H)
         return proj, proj.mean(1)
-
-    def get_hidden_parameters(self, img_filepath):
-        self.img = self.preprocess_img(img_filepath)
-        enc = self._find_caption(img_filepath, beam_size=3, max_cap_length=20)
-        self._set_state(self.img, self.beam_caption_encode, enc)
 
     def forward_greedy(self, img_filepath):
         """reference :883-950: the saved state for the beam-size-1 caption."""

@@ -810,6 +810,16 @@ class ExplainGridTDAttention(object):
     DEVICE_BEAM_SEARCH = True
     _BEAM = "GridTDBeamSearch"            # class in lrpx.beam
     _REMOVE_BAD_ENDINGS = True
+    # (beam_size, max_cap_length) of the caption search of get_hidden_parameters (reference :933-1012), also the
+    # defaults of lrpx.pipeline.BatchExplainer.explain_images
+    CAPTION_SEARCH = (2, 50)
+
+    def _searcher(self):
+        """The device caption search over this explainer's model (lrpx.beam.<_BEAM>), built once."""
+        if getattr(self, "_beam", None) is None:
+            from lrpx import beam
+            self._beam = getattr(beam, self._BEAM)(self.model)
+        return self._beam
 
     def _search_inputs(self, feat):
         """(B,P,C) encoder features -> what the model's ``_encode`` hands to its beam search."""
@@ -826,13 +836,11 @@ class ExplainGridTDAttention(object):
         enc = None
         if (self.DEVICE_BEAM_SEARCH and self.uses_tc and self.has_encoder and self.img.is_cuda
                 and 'beam_search' not in m.__dict__):
-            from lrpx import beam
-            if getattr(self, "_beam", None) is None:
-                self._beam = getattr(beam, self._BEAM)(m)
             enc = self.encode_images(self.img)
             with torch.no_grad():
                 proj, glob = self._search_inputs(enc[0])
-            idx = self._beam.search(proj, glob, self.word_map, beam_size=beam_size, max_cap_length=max_cap_length)[0]
+            idx = self._searcher().search(proj, glob, self.word_map, beam_size=beam_size,
+                                          max_cap_length=max_cap_length)[0]
             if getattr(self, "_rev_word_map", None) is None:          # built once: ~1 ms for a 10 000-word vocabulary
                 self._rev_word_map = {v: k for k, v in self.word_map.items()}
             rev = self._rev_word_map
@@ -848,7 +856,8 @@ class ExplainGridTDAttention(object):
 
     def get_hidden_parameters(self, img_filepath):
         self.img = self.preprocess_img(img_filepath)
-        enc = self._find_caption(img_filepath, beam_size=2, max_cap_length=50)
+        beam_size, max_cap_length = self.CAPTION_SEARCH
+        enc = self._find_caption(img_filepath, beam_size=beam_size, max_cap_length=max_cap_length)
         self._set_state(self.img, self.beam_caption_encode, enc)
 
     def forward_greedy(self, img_filepath):
@@ -967,6 +976,7 @@ class ExplainGridTDGradient(GradientFamily, ExplainGridTDAttention):
     weights and gates held constant, as the reference's hand-written backward does) and the per-word sums of the
     embedding gradients.  ``model=`` / ``precision=`` are keywords the reference does not have."""
     EX_TYPE = 'gradient'
+    CAPTION_SEARCH = (3, 50)              # get_hidden_parameters, reference :1323-1422
 
     def __init__(self, args, word_map, model=None, precision=None):
         ExplainGridTDAttention.__init__(self, args, word_map, model=model, precision=precision)
@@ -974,12 +984,6 @@ class ExplainGridTDGradient(GradientFamily, ExplainGridTDAttention):
 
     def _grad_weights(self):
         return self._cached_grad_weights(gridtd_grad_weights)
-
-    def get_hidden_parameters(self, img_filepath):
-        """reference :1323-1422 (beam size 3, up to 50 words)."""
-        self.img = self.preprocess_img(img_filepath)
-        enc = self._find_caption(img_filepath, beam_size=3, max_cap_length=50)
-        self._set_state(self.img, self.beam_caption_encode, enc)
 
     def _set_state(self, img, tokens, enc=None):
         ExplainGridTDAttention._set_state(self, img, tokens, enc)
