@@ -10,6 +10,7 @@ Supported topologies: a Sequential of leaves (the VGG encoder slice) and the Bot
 models/resnet.py.  Anything else raises ``NotImplementedError`` in ``add_lrp``.
 """
 import os
+from collections import defaultdict
 
 import torch
 import torch.nn as nn
@@ -231,7 +232,7 @@ class _TcResNetPlan:
     def __init__(self, model):
         self.model = model
         self.convs = [m for m in model.modules() if isinstance(m, nn.Conv2d)]
-        self._eng = {}
+        self._eng = defaultdict(ops.WeightCache)
 
     def engine(self, precision, lrp_params):
         from lrpx import tc_resnet
@@ -239,12 +240,8 @@ class _TcResNetPlan:
                 or float(lrp_params.get("beta", 0.)) != 0. or not lrp_params.get("ignore_bias", True):
             return None
         ps = [p for p in self.model.parameters()] + [b for b in self.model.buffers()]
-        stamp = tuple((t.data_ptr(), t._version) for t in ps)
-        hit = self._eng.get(precision)
-        if hit is None or hit[0] != stamp:
-            cls = tc_resnet.TcResNetMixed if precision == "mixed" else tc_resnet.TcResNetEngine
-            hit = self._eng[precision] = (stamp, cls(self.model, ps[0].device))
-        return hit[1]
+        cls = tc_resnet.TcResNetMixed if precision == "mixed" else tc_resnet.TcResNetEngine
+        return self._eng[precision].get(ps, lambda: cls(self.model, ps[0].device))
 
 
 class _TcPlan:
@@ -253,7 +250,7 @@ class _TcPlan:
 
     def __init__(self, convs, cfg):
         self.convs, self.cfg = convs, cfg
-        self._eng = {}
+        self._eng = defaultdict(ops.WeightCache)
 
     def engine(self, precision, lrp_params):
         from lrpx import tc
@@ -261,17 +258,13 @@ class _TcPlan:
         ignore_bias = bool(lrp_params.get("ignore_bias", True))
         ws = [c.weight for c in self.convs]
         bs = [c.bias for c in self.convs]
-        stamp = tuple((t.data_ptr(), t._version) for t in ws + [b for b in bs if b is not None])
-        key = (precision, alpha, beta, ignore_bias)
-        hit = self._eng.get(key)
-        if hit is None or hit[0] != stamp:
+
+        def build():
             if precision == "mixed":          # fp32-accurate forward, bf16 chain (alpha 1 / beta 0 preset only)
-                eng = tc.TcVggMixed(ws, bs, self.cfg, ws[0].device)
-            else:
-                eng = tc.TcVggEngine(ws, bs, self.cfg, ws[0].device, precision=precision, alpha=alpha, beta=beta,
-                                     ignore_bias=ignore_bias)
-            hit = self._eng[key] = (stamp, eng)
-        return hit[1]
+                return tc.TcVggMixed(ws, bs, self.cfg, ws[0].device)
+            return tc.TcVggEngine(ws, bs, self.cfg, ws[0].device, precision=precision, alpha=alpha, beta=beta,
+                                  ignore_bias=ignore_bias)
+        return self._eng[precision, alpha, beta, ignore_bias].get(ws + [b for b in bs if b is not None], build)
 
 
 def _build_plan(model):

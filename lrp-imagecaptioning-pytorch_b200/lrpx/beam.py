@@ -27,7 +27,7 @@ class _DeviceBeamSearch:
     def __init__(self, model, use_graph=True):
         self.model = model
         self.use_graph = use_graph
-        self._w_key = None
+        self._w = ops.WeightCache()
         self._plans = {}
 
     # subclasses: _weight_sources() -> tensors whose change invalidates the cache; _build_weights() -> dict;
@@ -37,14 +37,12 @@ class _DeviceBeamSearch:
         # the captured graphs hold raw pointers: every tensor a step reads belongs to the key, so that a model moved or
         # re-loaded after the first search gets fresh plans
         m = self.model
-        key = tuple((t.data_ptr(), t._version) for t in self._weight_sources()) + \
-            tuple(t.data_ptr() for t in (m.embedding.weight, m.fc.weight, m.fc.bias))      # read in place: pointer only
-        if self._w_key != key:
-            with torch.no_grad():
-                self._w = self._build_weights()
-            self._w_key = key
+
+        def build():
             self._plans = {}
-        return self._w
+            return self._build_weights()
+        return self._w.get(self._weight_sources(), build,
+                           tuple(t.data_ptr() for t in (m.embedding.weight, m.fc.weight, m.fc.bias)))   # read in place: pointer only
 
     def _plan(self, B, k, L, P, start_id, end_id):
         key = (B, k, L, P, start_id, end_id)

@@ -243,7 +243,7 @@ class LinearX3:
 
     def __init__(self, weight, bias=None):
         self.src = (weight, bias)
-        self.key = None
+        self._split = WeightCache()
         n, k = weight.shape
         if k % 64 or n % 4:
             raise _lib.LrpxError("LinearX3: in_features must be a multiple of 64 and out_features a multiple of 4")
@@ -256,18 +256,15 @@ class LinearX3:
 
     def _prep(self):
         w, b = self.src
-        key = (w.data_ptr(), w._version, None if b is None else (b.data_ptr(), b._version))
-        if key != self.key:
-            with torch.no_grad():
-                wf = w.detach().float()
-                if self.n_pad != self.n:
-                    wf = torch.cat((wf, wf.new_zeros(self.n_pad - self.n, self.k)), 0)
-                hi = wf.to(torch.bfloat16)
-                lo = (wf - hi.float()).to(torch.bfloat16)
-                self.w3 = torch.cat((hi, hi, lo), 1).contiguous()
-                self.b = None if b is None else b.detach().float().contiguous()
-            self.key = key
-        return self.w3, self.b
+
+        def split():
+            wf = w.detach().float()
+            if self.n_pad != self.n:
+                wf = torch.cat((wf, wf.new_zeros(self.n_pad - self.n, self.k)), 0)
+            hi = wf.to(torch.bfloat16)
+            lo = (wf - hi.float()).to(torch.bfloat16)
+            return torch.cat((hi, hi, lo), 1).contiguous(), None if b is None else b.detach().float().contiguous()
+        return self._split.get([t for t in self.src if t is not None], split)
 
     def __call__(self, x, out=None):
         """x (m, k) fp32 CUDA (rows may be strided: pitch = x.stride(0)) -> (m, n) fp32"""
@@ -356,6 +353,24 @@ def weight_stamp(tensors):
     """(data pointer, in-place version counter) of each tensor: changes when a tensor is replaced or updated in place
     (``load_state_dict``, an optimizer step, ``p.add_()``).  Caches of prepared weight copies are keyed on it."""
     return tuple((t.data_ptr(), t._version) for t in tensors)
+
+
+class WeightCache:
+    """One value built from some source tensors (prepared weight copies, an engine holding converted weights).
+    ``get(sources, build, extra_key)`` runs ``build()`` under no_grad the first time and whenever ``extra_key +
+    weight_stamp(sources)`` changes; while the key holds it returns the same object: callers compare it by ``is``, and
+    captured CUDA graphs point into it."""
+
+    def __init__(self):
+        self.key = self.value = None
+
+    def get(self, sources, build, extra_key=()):
+        key = tuple(extra_key) + weight_stamp(sources)
+        if key != self.key:
+            with torch.no_grad():
+                self.value = build()
+            self.key = key
+        return self.value
 
 
 def _decoder_workspace(ws_cache, kind, dims, nbytes, dev, tc_gemm, weights=None):

@@ -15,7 +15,7 @@ from dataclasses import dataclass
 
 import torch
 
-from . import _graph, ops
+from . import _graph
 
 
 @dataclass
@@ -46,8 +46,8 @@ class BatchExplainer:
         self.ex = explainer
         # gradient-family explainers (models/_gradient.py): same pipeline, the decoder-gradient kernels and the chain's
         # 'gradient' / 'guided' rule instead of the relevance ones
-        self.is_gradient = hasattr(explainer, "_grad_weights")
-        if self.is_gradient and getattr(explainer, "CAM", None):
+        self.is_gradient = explainer.GRADIENT
+        if self.is_gradient and explainer.CAM:
             raise ValueError("BatchExplainer covers the gradient and guided-backpropagation explainers, not the CAM variants")
         self.eng = self.W = None
         self._dec_ws = {}         # persistent decoder workspaces holding the prepared copies of self.W (ops._decoder_workspace)
@@ -59,8 +59,6 @@ class BatchExplainer:
         # GEMMs, below the chain's own 2e-4 in the fp32-accurate mode); tc_gemm=False forces the CUDA-core GEMMs
         self.tc_gemm = True if tc_gemm is None else bool(tc_gemm)
         self.deliver = deliver
-        self.is_aoa = hasattr(explainer, "num_head") and hasattr(explainer.model, "decoder_multihead_attention")
-        self.is_adaptive = not self.is_aoa and not hasattr(explainer.model, "LanguageLSTM")   # single-LSTM decoder
         self.head_idx = int(head_idx)
         self._copy_stream = None
 
@@ -98,24 +96,8 @@ class BatchExplainer:
         state ``est``), decoder kernels, relevance chain into ``heat``.  -> (r_words, the explainer forward's logits)."""
         st = self.ex.explainer_forward(feat, tokens)
         req_word = tokens[req_img.long(), req_t.long() + 1].to(torch.int32)       # the word each request explains
-        if self.is_gradient and self.is_aoa:
-            r_feat, r_words = ops.aoa_decoder_grad(st, self.W, self.ex.num_head, req_img, req_t, req_word,
-                                                   torch.full_like(req_t, self.head_idx), tc_gemm=self.tc_gemm)
-        elif self.is_gradient and self.is_adaptive:
-            r_feat, r_words = ops.adaptive_decoder_grad(st, self.W, req_img, req_t, req_word, tc_gemm=self.tc_gemm)
-        elif self.is_gradient:
-            r_feat, r_words = ops.gridtd_decoder_grad(st, self.W, req_img, req_t, req_word,
-                                                      guided=self.ex.GUIDED_DECODER, tc_gemm=self.tc_gemm)
-        elif self.is_aoa:
-            r_feat, r_words = ops.aoa_decoder_lrp(st, self.W, self.ex.num_head, req_img, req_t, req_word,
-                                                  torch.full_like(req_t, self.head_idx), tc_gemm=self.tc_gemm,
-                                                  ws_cache=self._dec_ws)
-        elif self.is_adaptive:
-            r_feat, r_words = ops.adaptive_decoder_lrp(st, self.W, req_img, req_t, req_word, tc_gemm=self.tc_gemm,
-                                                       ws_cache=self._dec_ws)
-        else:
-            r_feat, r_words = ops.gridtd_decoder_lrp(st, self.W, req_img, req_t, req_word, tc_gemm=self.tc_gemm,
-                                                     ws_cache=self._dec_ws)
+        # on the explainer's cached decoder weights: the self.W of the last _sync_weights
+        r_feat, r_words = self.ex._decode(st, req_img, req_t, req_word, self.tc_gemm, self.head_idx, self._dec_ws)
         if host is None:
             self.eng.relevance(est, r_feat, req_img, chunk=self.chunk, out=heat, deliver=self.deliver)
             return r_words, st["pred"]

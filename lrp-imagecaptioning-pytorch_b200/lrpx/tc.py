@@ -677,6 +677,3 @@ class TcVggMixed:
 
     def __getattr__(self, name):          # relevance, relevance_head / _tail, heat_shape, convs, flop counters: the chain's
         return getattr(self.chain, name)
-
-
-TcVggGradientHybrid = TcVggMixed          # the name the gradient-family explainers use

@@ -90,37 +90,12 @@ class GradientFamily:
     GUIDED_DECODER = False       # gridTD guided variants: d_img_feature[image_features <= 0] = 0 (gridTDmodel.py:1674)
     CAM = None                   # None | 'cam' (Grad-CAM map instead of the image gradient) | 'guided' (guided x CAM)
     ACCUMULATE_LIKE_REFERENCE = False     # the gradient explain_cnn works on a fresh copy of the image every time
+    GRADIENT = True
 
-    # ------------------------------------------------------------------ plumbing
-    def engine(self):
-        """The tensor-core encoder engine (converted copies of the encoder's weights), rebuilt when an encoder parameter
-        or buffer changes."""
-        key = self._encoder_stamp()
-        if self._engine is not None and self._engine_key != key:
-            self._engine = None
-        self._engine_key = key
-        if self._engine is None:
-            from lrpx import tc
-            import torch.nn as nn
-            enc = self.model.img_encoder.encoder
-            convs = [m for m in enc if isinstance(m, nn.Conv2d)]
-            cfg = [m.out_channels if isinstance(m, nn.Conv2d) else "M" for m in enc if isinstance(m, (nn.Conv2d, nn.MaxPool2d))]
-            if self.precision in ("bf16", "mixed"):       # bf16 chain on the masks of the fp32-accurate forward (see the class)
-                self._engine = tc.TcVggGradientHybrid([c.weight for c in convs], [c.bias for c in convs], cfg, self.device,
-                                                      rule=self.RULE)
-            else:
-                self._engine = tc.TcVggEngine([c.weight for c in convs], [c.bias for c in convs], cfg, self.device,
-                                              precision=self.precision, rule=self.RULE)
-        return self._engine
-
-    def _cached_grad_weights(self, build):
-        """``build(state_dict)``: the decoder-gradient kernels' weights, rebuilt when a model parameter is replaced or
-        updated in place; the dict stays the same object until then."""
-        key = ops.weight_stamp(self.model.parameters())
-        if getattr(self, "_gw", None) is None or self._gw_key != key:
-            self._gw = build({k: v.detach() for k, v in self.model.state_dict().items()})
-            self._gw_key = key
-        return self._gw
+    def _grad_weights(self):
+        """The decoder-gradient kernels' weights (``_GRAD_WEIGHTS(state_dict)``), rebuilt when a model parameter is
+        replaced or updated in place; the dict stays the same object until then."""
+        return self._caches["grad"].get(self.model.parameters(), lambda: self._GRAD_WEIGHTS(self._state_dict()))
 
     def _check_encoder(self):
         # Bottleneck ResNets: the fp32 CUDA-core path only (LRPtools.lrp_wrapper.encoder_gradient_simt)
@@ -184,9 +159,5 @@ class GradientFamily:
         rows = torch.zeros(d_img_feature.shape[0], dtype=torch.int32, device=self.device)
         return self._finish(self._pix(d_img_feature), rows)
 
-    def _explain_all(self, d_feat, r_words):
-        T = self.caption_length
-        out = self._finish(d_feat, torch.zeros(T, dtype=torch.int32, device=self.device))
-        relevance_imgs = [out[t:t + 1] for t in range(T)]
-        relevance_preceeding_words = [r_words[t, :t + 1] for t in range(T)]
-        return relevance_imgs, relevance_preceeding_words
+    def _explain_image(self, d_feat):
+        return self._finish(d_feat, torch.zeros(d_feat.shape[0], dtype=torch.int32, device=self.device))

@@ -192,28 +192,21 @@ class ExplainAdaptiveAttention(ExplainGridTDAttention):
         self.adalstm_weight_i, self.adalstm_weight_h = m.AdaLSTM.lstm_cell.weight_ih, m.AdaLSTM.lstm_cell.weight_hh
         self.adalstm_bias_i, self.adalstm_bias_h = m.AdaLSTM.lstm_cell.bias_ih, m.AdaLSTM.lstm_cell.bias_hh
 
-    def _lrp_weights(self):
-        key = ops.weight_stamp(self.model.parameters())           # rebuilt after an update of the model's parameters
-        if self._weights is None or self._weights_key != key:
-            sd = {k: v.detach() for k, v in self.model.state_dict().items()}
-            self._weights, self._weights_key = _dec.adaptive_weights(sd), key
-        return self._weights
+    _LRP_WEIGHTS = staticmethod(_dec.adaptive_weights)
 
     def _explainer_weights(self):
         """[W_hh ; h_gate] (recurrent, in the step kernel's layout), [W_ih ; x_gate] (input side), summed biases;
         cached until a parameter changes."""
         m = self.model
         cell, xg, hg = m.AdaLSTM.lstm_cell, m.AdaLSTM.x_gate, m.AdaLSTM.h_gate
-        src = [cell.weight_ih, cell.weight_hh, cell.bias_ih, cell.bias_hh, xg.weight, xg.bias, hg.weight, hg.bias]
-        key = tuple((t.data_ptr(), t._version) for t in src)
-        if getattr(self, "_expl_w_key", None) != key:
-            with torch.no_grad():
-                W_rec = torch.cat((cell.weight_hh, hg.weight), 0).t().contiguous()          # (H, 5H)
-                W_in = torch.cat((cell.weight_ih, xg.weight), 0).t().contiguous()           # (2E, 5H)
-                b = torch.cat((cell.bias_ih + cell.bias_hh, xg.bias + hg.bias)).contiguous()
-                self._expl_w = (ops.lstm_prep_weights(W_rec, 5), W_in, b)
-            self._expl_w_key = key
-        return self._expl_w
+
+        def build():
+            W_rec = torch.cat((cell.weight_hh, hg.weight), 0).t().contiguous()          # (H, 5H)
+            W_in = torch.cat((cell.weight_ih, xg.weight), 0).t().contiguous()           # (2E, 5H)
+            b = torch.cat((cell.bias_ih + cell.bias_hh, xg.bias + hg.bias)).contiguous()
+            return ops.lstm_prep_weights(W_rec, 5), W_in, b
+        return self._caches["expl_w"].get([cell.weight_ih, cell.weight_hh, cell.bias_ih, cell.bias_hh, xg.weight, xg.bias,
+                                           hg.weight, hg.bias], build)
 
     def explainer_forward(self, feat, tokens, quirk_double_bias_ih=None, want_gates=False):
         """(``quirk_double_bias_ih`` is accepted for the shared gradient-family plumbing and has no effect: this model's
@@ -245,17 +238,13 @@ class ExplainAdaptiveAttention(ExplainGridTDAttention):
             glob = (z_glob + m.global_img_feature_proj.bias).clamp(min=0)
             img_proj = self._lx("wv", att.W_v_proj.weight, att.W_v_proj.bias)(A.view(B * P, H)).view(B, P, K)   # (B,P,K)
             Wrec_p, W_in, b = self._explainer_weights()
-
-            def _att_layer():                        # [h | s] @ blockdiag(W_g^T, W_s^T) + [0 | b_s] as one Linear
-                Wa = torch.zeros(2 * K, 2 * H, device=dev)
-                Wa[:K, :H] = att.W_g_proj.weight
-                Wa[K:, H:] = att.W_s_proj.weight
-                return Wa, torch.cat((torch.zeros(K, device=dev), att.W_s_proj.bias))
-            att_lin = self._lx("att", [att.W_g_proj.weight, att.W_s_proj.weight], att.W_s_proj.bias, _att_layer)
+            att_lin = self._attention_layer()
             w_h = att.w_h.weight.reshape(-1).contiguous()
             emb = m.embedding(tokens[:, :T])                                                     # (B,T,E)
             x = torch.cat((emb, glob.unsqueeze(1).expand(B, T, E)), -1).contiguous()             # (B,T,2E)  :649
-            pre = self._lx("pre", W_in, b, lambda: (W_in.t().contiguous(), b))(x.transpose(0, 1).reshape(T * B, 2 * E)).view(T, B, 5 * H)
+            cell, xg, hg = m.AdaLSTM.lstm_cell, m.AdaLSTM.x_gate, m.AdaLSTM.h_gate
+            pre = self._lx("pre", [cell.weight_ih, xg.weight], [cell.bias_ih, cell.bias_hh, xg.bias, hg.bias],
+                           lambda: (W_in.t().contiguous(), b))(x.transpose(0, 1).reshape(T * B, 2 * E)).view(T, B, 5 * H)
             h, c = torch.zeros(B, T + 1, H, device=dev), torch.zeros(B, T + 1, H, device=dev)
             g, i, f, st, ctx, ctx_hat = (new(B, T, H) for _ in range(6))
             alpha, beta = new(B, T, P), new(B, T)
@@ -279,49 +268,23 @@ class ExplainAdaptiveAttention(ExplainGridTDAttention):
             out.update(o=og, sg=sg)
         return out
 
-    def teacherforce_forward(self, img, beam_caption_encode):
-        feat, _, _ = self.encode_images(img)
-        toks = torch.tensor([list(beam_caption_encode) + [0]], dtype=torch.long, device=self.device)
-        return self.explainer_forward(feat, toks)["pred"][0]
-
     # ------------------------------------------------------------------ reference entry points
     CAPTION_SEARCH = (3, 20)              # get_hidden_parameters, reference :626-677
-
-    def forward_greedy(self, img_filepath):
-        """reference :567-624: the same saved state for the beam-size-1 caption."""
-        self.img = self.preprocess_img(img_filepath)
-        enc = self._find_caption(img_filepath, beam_size=1, max_cap_length=20)
-        self._set_state(self.img, self.beam_caption_encode, enc)
 
     _BEAM = "AdaptiveBeamSearch"
     _REMOVE_BAD_ENDINGS = False           # this model's beam search keeps the sentence as it is (:444-446)
 
-    def _set_state(self, img, tokens, enc=None):
-        if self._empty_caption(tokens):
-            return
-        feat, (fh, fw), est = enc if enc is not None else self.encode_images(img)
-        toks = torch.tensor([tokens], dtype=torch.long, device=self.device)
-        st = self.explainer_forward(feat, toks)
-        self._state, self._enc_state, self._feat_hw = st, est, (fh, fw)
-        self.caption_length = len(tokens) - 1
-        self.num_pixels = feat.shape[1]
-        # attributes the reference exposes (:634-646)
+    def _expose_state(self, st):
+        """attributes the reference exposes (:634-646)"""
         self.predictions, self.alphas, self.betas = st["pred"][0], st["alpha"][0], st["beta"][0]
         self.xt, self.ht, self.ct = st["x"][0], st["h"][0], st["c"][0]
         self.gt, self.it_act, self.ft_act = st["g"][0], st["i"][0], st["f"][0]
         self.st, self.context, self.context_hat = st["st"][0], st["ctx"][0], st["ctx_hat"][0]
-        C = feat.shape[2]
-        self.image_features = feat[0].t().reshape(1, C, fh, fw)
         self.avg_feature = st["avg"][0]
 
-    def _decoder_lrp(self, ts):
-        toks = self.beam_caption_encode
-        dev = self.device
-        req_t = torch.tensor(ts, dtype=torch.int32, device=dev)
-        req_word = torch.tensor([toks[t + 1] for t in ts], dtype=torch.int32, device=dev)
-        req_img = torch.zeros(len(ts), dtype=torch.int32, device=dev)
-        return ops.adaptive_decoder_lrp(self._state, self._lrp_weights(), req_img, req_t, req_word,
-                                        tc_gemm=(self.precision in ('bf16', 'mixed')))
+    def _decode(self, st, req_img, req_t, req_word, tc_gemm, head_idx=0, ws_cache=None):
+        return ops.adaptive_decoder_lrp(st, self._lrp_weights(), req_img, req_t, req_word, tc_gemm=tc_gemm,
+                                        ws_cache=ws_cache)
 
 
 # ================================================================================================ gradient family (f4)
@@ -348,37 +311,14 @@ class ExplainAdaptiveGradient(GradientFamily, ExplainAdaptiveAttention):
         ExplainAdaptiveAttention.__init__(self, args, word_map, model=model, precision=precision)
         self._check_encoder()
 
-    def _grad_weights(self):
-        return self._cached_grad_weights(adaptive_grad_weights)
+    _GRAD_WEIGHTS = staticmethod(adaptive_grad_weights)
 
-    def _set_state(self, img, tokens, enc=None):
-        ExplainAdaptiveAttention._set_state(self, img, tokens, enc)
-        if self._state is not None:
-            self.ot_act, self.sen_gate = self._state["o"][0], self._state["sg"][0]
+    def _expose_state(self, st):
+        ExplainAdaptiveAttention._expose_state(self, st)
+        self.ot_act, self.sen_gate = st["o"][0], st["sg"][0]
 
-    def _decoder_grad(self, ts):
-        toks = self.beam_caption_encode
-        i32 = lambda v: torch.tensor(v, dtype=torch.int32, device=self.device)
-        return ops.adaptive_decoder_grad(self._state, self._grad_weights(), i32([0] * len(ts)), i32(list(ts)),
-                                         i32([toks[t + 1] for t in ts]), tc_gemm=(self.precision in ('bf16', 'mixed')))
-
-    def explain_caption_wordt(self, t):
-        """reference :965-1021 (guided: :1100-1163, same values) -> (d_img_feature (1,C,h,w), r_words (t+1,))."""
-        assert t < self.caption_length
-        d_feat, r_words = self._decoder_grad([t])
-        fh, fw = self._feat_hw
-        return d_feat[0].t().reshape(1, -1, fh, fw), r_words[0, :t + 1]
-
-    def explain_caption(self, img_filepath, t_list=None):
-        """reference :1038-1052."""
-        self.img_filepath = img_filepath
-        self.get_hidden_parameters(img_filepath)
-        if self.caption_length == 0:
-            return [], []
-        d_feat, r_words = self._decoder_grad(list(range(self.caption_length)))
-        relevance_imgs, relevance_preceeding_words = self._explain_all(d_feat, r_words)
-        self.save_linguistic_explanation(relevance_preceeding_words)
-        return relevance_imgs, relevance_preceeding_words
+    def _decode(self, st, req_img, req_t, req_word, tc_gemm, head_idx=0, ws_cache=None):
+        return ops.adaptive_decoder_grad(st, self._grad_weights(), req_img, req_t, req_word, tc_gemm=tc_gemm)
 
 
 class ExplainiAdaptiveGuidedGradient(ExplainAdaptiveGradient):

@@ -15,7 +15,6 @@ import math
 import torch
 import torch.nn as nn
 
-from LRPtools import lrp_wrapper
 from LRPtools import utils as LRPutil
 from lrpx import ops
 from lrpx import decoder as _dec
@@ -360,26 +359,18 @@ class ExplainAOAAttention(ExplainGridTDAttention):
                           lambda: AOAModel(args.embed_dim, args.hidden_dim, args.num_head, len(word_map), args.encoder))
         self.model.decoder_multihead_attention.eval()
 
-    def _lrp_weights(self):
-        key = ops.weight_stamp(self.model.parameters())           # rebuilt after an update of the model's parameters
-        if self._weights is None or self._weights_key != key:
-            self._weights = _dec.aoa_weights({k: v.detach() for k, v in self.model.state_dict().items()})
-            self._weights_key = key
-        return self._weights
+    _LRP_WEIGHTS = staticmethod(_dec.aoa_weights)
 
     def _explainer_weights(self, quirk_double_bias_ih=True):
         """Recurrent weights in the step kernel's layout, input-side weights and summed biases; cached until a
         parameter changes."""
         L = self.model.LanguageLSTM
-        src = [L.weight_ih, L.weight_hh, L.bias_ih, L.bias_hh]
-        key = (quirk_double_bias_ih,) + tuple((t.data_ptr(), t._version) for t in src)
-        if getattr(self, "_expl_w_key", None) != key:
-            with torch.no_grad():
-                lb2 = L.bias_ih if quirk_double_bias_ih else L.bias_hh                    # Q3 (:873)
-                self._expl_w = (ops.lstm_prep_weights(L.weight_hh.t().contiguous(), 4), L.weight_ih.t().contiguous(),
-                                (L.bias_ih + lb2).contiguous())
-            self._expl_w_key = key
-        return self._expl_w
+        lb2 = L.bias_ih if quirk_double_bias_ih else L.bias_hh                    # Q3 (:873)
+        return self._caches["expl_w"].get(
+            [L.weight_ih, L.weight_hh, L.bias_ih, L.bias_hh],
+            lambda: (ops.lstm_prep_weights(L.weight_hh.t().contiguous(), 4), L.weight_ih.t().contiguous(),
+                     (L.bias_ih + lb2).contiguous()),
+            (quirk_double_bias_ih,))
 
     def explainer_forward(self, feat, tokens, quirk_double_bias_ih=True, want_gates=False):
         """The explainer's teacher-forced forward (reference :999-1062) batched over images; returns the saved
@@ -415,7 +406,9 @@ class ExplainAOAAttention(ExplainGridTDAttention):
             mha = m.decoder_multihead_attention
             Wp_hh, W_in, b = self._explainer_weights(quirk_double_bias_ih)
             x = torch.cat((m.embedding(tokens[:, :T]), glob.unsqueeze(1).expand(B, T, H)), -1).contiguous()   # (B,T,E+H)
-            pre = self._lx("pre", W_in, b, lambda: (W_in.t().contiguous(), b))(x.transpose(0, 1).reshape(T * B, E + H)).view(T, B, 4 * H)
+            L = m.LanguageLSTM
+            pre = self._lx(("pre", quirk_double_bias_ih), L.weight_ih, [L.bias_ih, L.bias_hh],
+                           lambda: (W_in.t().contiguous(), b))(x.transpose(0, 1).reshape(T * B, E + H)).view(T, B, 4 * H)
             h, c = torch.zeros(B, T + 1, H, device=dev), torch.zeros(B, T + 1, H, device=dev)
             g, i, f = (torch.empty(B, T, H, device=dev) for _ in range(3))
             o = torch.empty(B, T, H, device=dev) if want_gates else None
@@ -451,36 +444,17 @@ class ExplainAOAAttention(ExplainGridTDAttention):
         proj = torch.addmm(m.img_projector.bias, feat.reshape(B * P, C), Wp.t()).clamp(min=0).view(B, P, -1)   # (B,P,H)
         return proj, proj.mean(1)
 
-    def forward_greedy(self, img_filepath):
-        """reference :883-950: the saved state for the beam-size-1 caption."""
-        self.img = self.preprocess_img(img_filepath)
-        enc = self._find_caption(img_filepath, beam_size=1, max_cap_length=20)
-        self._set_state(self.img, self.beam_caption_encode, enc)
-
-    def _set_state(self, img, tokens, enc=None):
-        if self._empty_caption(tokens):
-            return
-        feat, (fh, fw), est = enc if enc is not None else self.encode_images(img)
-        toks = torch.tensor([tokens], dtype=torch.long, device=self.device)
-        st = self.explainer_forward(feat, toks)
-        self._state, self._enc_state, self._feat_hw = st, est, (fh, fw)
-        self.caption_length = len(tokens) - 1
-        self.num_pixels = feat.shape[1]
+    def _expose_state(self, st):
         self.predictions, self.alphas = st["pred"][0], st["alpha"][0]
         self.xt, self.ht, self.ct = st["x"][0], st["h"][0], st["c"][0]
         self.gt, self.it_act, self.ft_act = st["g"][0], st["i"][0], st["f"][0]
         self.context, self.context_aoa = st["ctx"][0], st["caoa"][0]
         self.context_aoa_linear, self.context_aoa_gate = st["caoa_lin"][0], st["caoa_gate"][0]
         self.key, self.value = st["key"], st["value"]
-        self.image_features = feat[0].t().reshape(1, feat.shape[2], fh, fw)
 
-    def _decoder_lrp(self, ts, head_idx):
-        toks = self.beam_caption_encode
-        dev = self.device
-        i32 = lambda v: torch.tensor(v, dtype=torch.int32, device=dev)
-        return ops.aoa_decoder_lrp(self._state, self._lrp_weights(), self.num_head, i32([0] * len(ts)), i32(list(ts)),
-                                   i32([toks[t + 1] for t in ts]), i32([head_idx] * len(ts)),
-                                   tc_gemm=(self.precision in ('bf16', 'mixed')))
+    def _decode(self, st, req_img, req_t, req_word, tc_gemm, head_idx=0, ws_cache=None):
+        return ops.aoa_decoder_lrp(st, self._lrp_weights(), self.num_head, req_img, req_t, req_word,
+                                   torch.full_like(req_t, int(head_idx)), tc_gemm=tc_gemm, ws_cache=ws_cache)
 
     def lrp_mha(self, alpha, value, r_context, context, head_idx):
         """reference :812-862 (same argument order): relevance of the values of ONE head (others get 0, Q5).
@@ -489,34 +463,12 @@ class ExplainAOAAttention(ExplainGridTDAttention):
         return ops.lrp_mha(alpha, value, r_context, context, self.num_head, head_idx)
 
     def explain_caption_wordt(self, t, head_idx):
-        """reference :1064-1156 -> (r_img_feature (1,C,h,w), r_words (t+1,))."""
-        assert t < self.caption_length
-        r_feat, r_words = self._decoder_lrp([t], head_idx)
-        fh, fw = self._feat_hw
-        return r_feat[0].t().reshape(1, -1, fh, fw), r_words[0, :t + 1]
+        """reference :1064-1156 (gradient: :1435-1499) -> (r_img_feature (1,C,h,w), r_words (t+1,))."""
+        return self._explain_word(t, head_idx)
 
     def explain_caption(self, img_filepath, head_idx, t_list=None):
-        """reference :1165-1181."""
-        self.img_filepath = img_filepath
-        self.get_hidden_parameters(img_filepath)
-        T = self.caption_length
-        if T == 0:
-            return [], []
-        r_feat, r_words = self._decoder_lrp(list(range(T)), head_idx)
-        if self.uses_tc:
-            heat = self.engine().relevance(self._enc_state, r_feat, torch.zeros(T, dtype=torch.int32, device=self.device))
-        else:
-            enc = self.model.img_encoder.encoder
-            lrp_wrapper.add_lrp(enc)
-            fh, fw = self._feat_hw
-            heat = torch.cat([lrp_wrapper.compute_lrp(enc, self.img.detach().clone(), precision='simt',
-                                                      target=r_feat[t].t().reshape(1, -1, fh, fw)) for t in range(T)])
-        if self.ACCUMULATE_LIKE_REFERENCE:
-            heat = torch.cumsum(heat, 0)
-        relevance_imgs = [heat[t:t + 1] for t in range(T)]
-        relevance_preceeding_words = [r_words[t, :t + 1] for t in range(T)]
-        self.save_linguistic_explanation(relevance_preceeding_words)
-        return relevance_imgs, relevance_preceeding_words
+        """reference :1165-1181 (gradient: :1517-1534)."""
+        return self._explain_caption(img_filepath, head_idx, t_list)
 
     def explain_region_features(self, images_features, head_idx, beam_size=3, t_list=None):
         """BASELINE config 3: the AoA decoder on bottom-up region features (1, 36, 2048) with ``AOAModelBU`` —
@@ -538,7 +490,7 @@ class ExplainAOAAttention(ExplainGridTDAttention):
         self.num_pixels = feats.shape[1]
         self.predictions, self.alphas = st["pred"][0], st["alpha"][0]
         ts = list(range(self.caption_length)) if t_list is None else list(t_list)
-        r_feat, r_words = self._decoder_lrp(ts, head_idx)
+        r_feat, r_words = self._decode_words(ts, head_idx)
         return [r_feat[k:k + 1] for k in range(len(ts))], [r_words[k, :t + 1] for k, t in enumerate(ts)]
 
     def explain_region_features_batch(self, images_features, head_idx, beam_size=3, tokens=None):
@@ -561,16 +513,16 @@ class ExplainAOAAttention(ExplainGridTDAttention):
         req_img = i32([b for b in range(B) for _ in caps[b]])
         req_t = i32([t for b in range(B) for t in range(len(caps[b]))])
         req_word = i32([w for c in caps for w in c])
-        r_feat, r_words = ops.aoa_decoder_lrp(st, self._lrp_weights(), self.num_head, req_img, req_t, req_word,
-                                              torch.full_like(req_t, int(head_idx)), tc_gemm=(self.precision in ('bf16', 'mixed')))
+        r_feat, r_words = self._decode(st, req_img, req_t, req_word, self.tc_gemm, head_idx)
         return r_feat, r_words, req_img, req_t, caps
 
-    def explain_caption_words(self, img_filepath):
-        """reference :1183-1194: linguistic relevance only (head 0)."""
+    def explain_caption_words(self, img_filepath, head_idx=0):
+        """reference :1183-1194 (gradient: :1536-1548, whose call omits head_idx and cannot run): linguistic relevance
+        only, of head 0 unless ``head_idx`` says otherwise."""
         self.img_filepath = img_filepath
         self.get_hidden_parameters(img_filepath)
         T = self.caption_length
-        _, r_words = self._decoder_lrp(list(range(T)), 0)
+        _, r_words = self._decode_words(range(T), head_idx)
         return [r_words[t, :t + 1] for t in range(T)]
 
 
@@ -586,13 +538,11 @@ class ExplainAOAGradient(GradientFamily, ExplainAOAAttention):
         ExplainAOAAttention.__init__(self, args, word_map, model=model, precision=precision)
         self._check_encoder()
 
-    def _grad_weights(self):
-        return self._cached_grad_weights(aoa_grad_weights)
+    _GRAD_WEIGHTS = staticmethod(aoa_grad_weights)
 
-    def _set_state(self, img, tokens, enc=None):
-        ExplainAOAAttention._set_state(self, img, tokens, enc)
-        if self._state is not None:
-            self.ot_act = self._state["o"][0]
+    def _expose_state(self, st):
+        ExplainAOAAttention._expose_state(self, st)
+        self.ot_act = st["o"][0]
 
     def gradient_mha(self, d_context, alpha, head_idx):
         """reference :1415-1433: d_value[p, head block] = d_context[head block] * alpha[head, p], zero on the other
@@ -605,37 +555,9 @@ class ExplainAOAGradient(GradientFamily, ExplainAOAAttention):
         d_value[:, sl] = alpha[head_idx].unsqueeze(1) * d_context.reshape(-1)[sl].unsqueeze(0)
         return d_value
 
-    def _decoder_grad(self, ts, head_idx):
-        toks = self.beam_caption_encode
-        i32 = lambda v: torch.tensor(v, dtype=torch.int32, device=self.device)
-        return ops.aoa_decoder_grad(self._state, self._grad_weights(), self.num_head, i32([0] * len(ts)), i32(list(ts)),
-                                    i32([toks[t + 1] for t in ts]), i32([head_idx] * len(ts)),
-                                    tc_gemm=(self.precision in ('bf16', 'mixed')))
-
-    def explain_caption_wordt(self, t, head_idx):
-        """reference :1435-1499 -> (d_img_feature (1,C,h,w), r_words (t+1,))."""
-        assert t < self.caption_length
-        d_feat, r_words = self._decoder_grad([t], head_idx)
-        fh, fw = self._feat_hw
-        return d_feat[0].t().reshape(1, -1, fh, fw), r_words[0, :t + 1]
-
-    def explain_caption(self, img_filepath, head_idx, t_list=None):
-        """reference :1517-1534."""
-        self.img_filepath = img_filepath
-        self.get_hidden_parameters(img_filepath)
-        if self.caption_length == 0:
-            return [], []
-        d_feat, r_words = self._decoder_grad(list(range(self.caption_length)), head_idx)
-        relevance_imgs, relevance_preceeding_words = self._explain_all(d_feat, r_words)
-        self.save_linguistic_explanation(relevance_preceeding_words)
-        return relevance_imgs, relevance_preceeding_words
-
-    def explain_caption_words(self, img_filepath, head_idx=0):
-        """reference :1536-1548 (whose call omits head_idx and cannot run): linguistic part only."""
-        self.img_filepath = img_filepath
-        self.get_hidden_parameters(img_filepath)
-        _, r_words = self._decoder_grad(list(range(self.caption_length)), head_idx)
-        return [r_words[t, :t + 1] for t in range(self.caption_length)]
+    def _decode(self, st, req_img, req_t, req_word, tc_gemm, head_idx=0, ws_cache=None):
+        return ops.aoa_decoder_grad(st, self._grad_weights(), self.num_head, req_img, req_t, req_word,
+                                    torch.full_like(req_t, int(head_idx)), tc_gemm=tc_gemm)
 
 
 class ExplainAOAGuidedGradient(ExplainAOAGradient):

@@ -17,6 +17,7 @@ batched kernel call per caption (``lrpx_gridtd_decoder_lrp_f32``), the per-sampl
 The forward passes that produce the saved state are plain torch tensor ops on the device (library GEMMs).
 """
 import os
+from collections import defaultdict
 
 import torch
 import torch.nn as nn
@@ -178,22 +179,24 @@ class GridTDModel(nn.Module):
         enc = self.img_encoder.encoder
         if prec and images.is_cuda and isinstance(enc, nn.Sequential) and not any(p.requires_grad for p in enc.parameters()):
             from lrpx import tc
-            from LRPtools import lrp_wrapper
-            stamp = tuple((p.data_ptr(), p._version) for p in enc.parameters())
-            if self._tc_encoder is None or self._tc_encoder[0] != stamp:
+
+            def build():
                 cfgd = lrp_wrapper._tc_cfg(enc)
                 if cfgd is None:
                     raise NotImplementedError("use_tc_encoder: the encoder is not a VGG-style conv3x3/ReLU/max-pool stack")
                 convs, cfg = cfgd
                 if prec == "fp32" and convs[0].out_channels % 64:
-                    prec = self._tc_encoder_precision = None          # shapes the general kernels do not take: library forward
-                    return self.img_encoder(images)
+                    return None                   # shapes the general kernels do not take: library forward
                 # rule='epsilon' keeps ONE accumulator per output channel in the forward (no z+ needed here)
-                eng = tc.TcVggEngine([c.weight for c in convs], [c.bias for c in convs], cfg, images.device,
-                                     precision="fp32", rule="epsilon") if prec == "fp32" else \
+                return tc.TcVggEngine([c.weight for c in convs], [c.bias for c in convs], cfg, images.device,
+                                      precision="fp32", rule="epsilon") if prec == "fp32" else \
                     tc.TcVggEngine([c.weight for c in convs], [c.bias for c in convs], cfg, images.device)
-                self._tc_encoder = (stamp, eng)
-            eng = self._tc_encoder[1]
+            if self._tc_encoder is None:
+                self._tc_encoder = ops.WeightCache()
+            eng = self._tc_encoder.get(enc.parameters(), build)
+            if eng is None:
+                self._tc_encoder_precision = self._tc_encoder = None
+                return self.img_encoder(images)
             with torch.no_grad():
                 feats = eng.features(eng.forward(images), "nchw")
             return feats, feats.mean((2, 3)).squeeze()
@@ -521,6 +524,9 @@ class ExplainGridTDAttention(object):
     # the reference never zeroes sample.grad, so relevance_imgs[t] of explain_caption is the running sum over
     # the words explained so far (Q1); set False for per-word heat-maps
     ACCUMULATE_LIKE_REFERENCE = True
+    SAVE_LINGUISTIC = True                # explain_caption writes the yaml of the word relevances
+    GRADIENT = False                      # the gradient family (models/_gradient.py) sets True
+    RULE = "alpha_beta"                   # rule of the encoder's tensor-core chain (lrpx.tc.TcVggEngine.RULES)
 
     def __init__(self, args, word_map, model=None, precision=None):
         self._common_init(args, word_map, model, precision,
@@ -574,8 +580,9 @@ class ExplainGridTDAttention(object):
         self.output_weight = m.fc.weight
         self.visualizatioin_save_path = os.path.join(args.save_path, args.dataset + 'explanation')
         os.makedirs(self.visualizatioin_save_path, exist_ok=True)
-        self._engine = self._engine_key = None
-        self._weights = self._weights_key = None
+        # decoder GEMMs of this explainer's own calls: bf16x3 on the tensor cores in the bf16 / mixed modes
+        self.tc_gemm = self.precision in ('bf16', 'mixed')
+        self._caches = defaultdict(ops.WeightCache)       # prepared weight copies and the encoder engine, by name
         self._state = None
 
     # ------------------------------------------------------------------ helpers
@@ -592,46 +599,35 @@ class ExplainGridTDAttention(object):
         x = (x - torch.tensor(self.mean).view(3, 1, 1)) / torch.tensor(self.std).view(3, 1, 1)
         return x.unsqueeze(0).to(self.device)
 
+    def _state_dict(self):
+        return {k: v.detach() for k, v in self.model.state_dict().items()}
+
+    _LRP_WEIGHTS = staticmethod(_dec.gridtd_weights)        # state_dict -> the decoder relevance kernels' weights
+
     def _lrp_weights(self):
         """The decoder relevance kernels' weights (gate rows concatenated, projector reshaped), rebuilt when a model
         parameter is replaced or updated in place; the dict stays the same object until then."""
-        key = ops.weight_stamp(self.model.parameters())
-        if self._weights is None or self._weights_key != key:
-            sd = {k: v.detach() for k, v in self.model.state_dict().items()}
-            self._weights, self._weights_key = _dec.gridtd_weights(sd), key
-        return self._weights
-
-    def _encoder_stamp(self):
-        enc = getattr(getattr(self.model, "img_encoder", None), "encoder", None)
-        return () if enc is None else ops.weight_stamp(list(enc.parameters()) + list(enc.buffers()))
+        return self._caches["lrp"].get(self.model.parameters(), lambda: self._LRP_WEIGHTS(self._state_dict()))
 
     def engine(self):
         """The tensor-core encoder engine (it holds converted copies of the encoder's weights): rebuilt when an encoder
-        parameter or buffer changes."""
-        key = self._encoder_stamp()
-        if self._engine is not None and self._engine_key != key:
-            self._engine = None
-        self._engine_key = key
-        if self._engine is None and getattr(self, "is_resnet", False):
-            from lrpx import tc_resnet
-            cls = tc_resnet.TcResNetMixed if self.precision == 'mixed' else tc_resnet.TcResNetEngine
-            self._engine = cls(self.model.img_encoder.encoder, self.device)
-        if self._engine is None:
+        parameter or buffer changes.  Bottleneck ResNets: lrpx.tc_resnet; VGG-style encoders: lrpx.tc in this class's
+        RULE, with the forward in the fp32-accurate mode for precision 'mixed' and for a gradient rule in 'bf16' (a
+        gradient's ReLU masks flip with the forward's rounding, DESIGN.md)."""
+        enc = self.model.img_encoder.encoder
+
+        def build():
+            if self.is_resnet:
+                from lrpx import tc_resnet
+                cls = tc_resnet.TcResNetMixed if self.precision == 'mixed' else tc_resnet.TcResNetEngine
+                return cls(enc, self.device)
             from lrpx import tc
-            enc = self.model.img_encoder.encoder
-            convs = [m for m in enc if isinstance(m, nn.Conv2d)]
-            cfg = []
-            for m in enc:
-                if isinstance(m, nn.Conv2d):
-                    cfg.append(m.out_channels)
-                elif isinstance(m, nn.MaxPool2d):
-                    cfg.append("M")
-            if self.precision == 'mixed':
-                self._engine = tc.TcVggMixed([c.weight for c in convs], [c.bias for c in convs], cfg, self.device)
-            else:
-                self._engine = tc.TcVggEngine([c.weight for c in convs], [c.bias for c in convs], cfg, self.device,
-                                              precision=self.precision)
-        return self._engine
+            convs, cfg = lrp_wrapper._tc_cfg(enc)
+            ws, bs = [c.weight for c in convs], [c.bias for c in convs]
+            if self.precision == 'mixed' or (self.precision == 'bf16' and self.RULE != 'alpha_beta'):
+                return tc.TcVggMixed(ws, bs, cfg, self.device, rule=self.RULE)
+            return tc.TcVggEngine(ws, bs, cfg, self.device, precision=self.precision, rule=self.RULE)
+        return self._caches["engine"].get(list(enc.parameters()) + list(enc.buffers()), build)
 
     def encode_images(self, imgs):
         """Encoder forward -> (features (B,P,C) fp32 pixel-major, feature map size, encoder state)."""
@@ -648,41 +644,32 @@ class ExplainGridTDAttention(object):
         return fmap.flatten(2).transpose(1, 2).contiguous(), (h, w), None
 
     def _explainer_weights(self, quirk_double_bias_ih=True):
-        """Concatenated / re-laid-out weights of the fused explainer forward, cached until a parameter changes
-        (the cache key holds every source tensor's data pointer and in-place version counter)."""
+        """Concatenated / re-laid-out weights of the fused explainer forward, cached until a parameter changes."""
         m = self.model
         cell, L, xg, hg = m.AdaLSTM.lstm_cell, m.LanguageLSTM, m.AdaLSTM.x_gate, m.AdaLSTM.h_gate
+        H = m.hidden_dim
+
+        def build():
+            # x1 = [h2, glob, emb] (:975): recurrent part [h2 | h1] -> (4H gates | sentinel gate), input part [glob | emb]
+            W1_rec = torch.cat((torch.cat((cell.weight_ih[:, :H], cell.weight_hh), 1),
+                                torch.cat((xg.weight[:, :H], hg.weight), 1)), 0).t().contiguous()          # (2H, 5H)
+            W1_in = torch.cat((cell.weight_ih[:, H:], xg.weight[:, H:]), 0).t().contiguous()               # (2E, 5H)
+            b1 = torch.cat((cell.bias_ih + cell.bias_hh, xg.bias + hg.bias)).contiguous()
+            W2 = torch.cat((L.weight_ih, L.weight_hh), 1).t().contiguous()                                 # (3H, 4H)
+            b2 = (L.bias_ih + (L.bias_ih if quirk_double_bias_ih else L.bias_hh)).contiguous()            # Q3 (:789)
+            return ops.lstm_prep_weights(W1_rec, 5), W1_in, b1, ops.lstm_prep_weights(W2, 4), b2
         src = [cell.weight_ih, cell.weight_hh, cell.bias_ih, cell.bias_hh, xg.weight, xg.bias, hg.weight, hg.bias,
                L.weight_ih, L.weight_hh, L.bias_ih, L.bias_hh]
-        key = (quirk_double_bias_ih,) + tuple((t.data_ptr(), t._version) for t in src)
-        if getattr(self, "_expl_w_key", None) != key:
-            H = m.hidden_dim
-            with torch.no_grad():
-                # x1 = [h2, glob, emb] (:975): recurrent part [h2 | h1] -> (4H gates | sentinel gate), input part [glob | emb]
-                W1_rec = torch.cat((torch.cat((cell.weight_ih[:, :H], cell.weight_hh), 1),
-                                    torch.cat((xg.weight[:, :H], hg.weight), 1)), 0).t().contiguous()      # (2H, 5H)
-                W1_in = torch.cat((cell.weight_ih[:, H:], xg.weight[:, H:]), 0).t().contiguous()           # (2E, 5H)
-                b1 = torch.cat((cell.bias_ih + cell.bias_hh, xg.bias + hg.bias)).contiguous()
-                W2 = torch.cat((L.weight_ih, L.weight_hh), 1).t().contiguous()                             # (3H, 4H)
-                b2 = (L.bias_ih + (L.bias_ih if quirk_double_bias_ih else L.bias_hh)).contiguous()        # Q3 (:789)
-                self._expl_w = (ops.lstm_prep_weights(W1_rec, 5), W1_in, b1, ops.lstm_prep_weights(W2, 4), b2)
-            self._expl_w_key = key
-        return self._expl_w
+        return self._caches["expl_w"].get(src, build, (quirk_double_bias_ih,))
 
     def _lx(self, name, weight, bias=None, derive=None):
-        """Cached tensor-core Linear for the explainer forwards: ``weight`` (out, in) and ``bias`` are (views of) model
-        parameters; ``derive()`` (optional) builds the actual (weight, bias) from them (concatenations, transposes) and
-        is re-run only when a source tensor changes (data pointer / in-place version)."""
+        """Cached Linear layer ``name`` of the explainer forwards: ``weight`` (out, in) and ``bias`` are (views of) model
+        parameters, or lists of the parameters ``derive()`` builds the actual (weight, bias) from (concatenations,
+        transposes); rebuilt when one of these source tensors changes."""
         src = [t for t in (weight if isinstance(weight, (list, tuple)) else [weight]) if t is not None]
         src += [t for t in (bias if isinstance(bias, (list, tuple)) else [bias]) if t is not None]
-        key = tuple((t.data_ptr(), t._version) for t in src)
-        cache = self.__dict__.setdefault("_lx_cache", {})
-        hit = cache.get(name)
-        if hit is None or hit[0] != key:
-            with torch.no_grad():
-                w, b = derive() if derive is not None else (weight.detach(), None if bias is None else bias.detach())
-            hit = cache[name] = (key, self._linear(w, b), (w, b))
-        return hit[1]
+        make = derive or (lambda: (weight.detach(), None if bias is None else bias.detach()))
+        return self._caches["lx", name].get(src, lambda: self._linear(*make()))
 
     def _linear(self, weight, bias):
         """A Linear layer of the explainer forward.  precision 'bf16' (the throughput mode): ``ops.LinearX3`` — the
@@ -693,34 +680,19 @@ class ExplainGridTDAttention(object):
             return ops.LinearX3(weight, bias)
         return lambda x: torch.addmm(bias, x, weight.t()) if bias is not None else x @ weight.t()
 
-    def _linears(self):
-        """The explainer forward's Linear layers on the tensor-core GEMM (built once, rebuilt when a source parameter
-        changes): 1x1 projector, global projection, W_v, the input-side gate pre-activations, the two attention
-        projections as one block-diagonal layer, the vocabulary projection."""
-        m = self.model
-        att, cell, xg = m.AdaAttention, m.AdaLSTM.lstm_cell, m.AdaLSTM.x_gate
-        src = [m.img_projector.weight, m.img_projector.bias, m.global_img_feature_proj.weight, att.W_v_proj.weight,
-               att.W_g_proj.weight, att.W_s_proj.weight, att.W_s_proj.bias, m.fc.weight, m.fc.bias, cell.weight_ih,
-               cell.bias_ih, cell.bias_hh, xg.weight, xg.bias]
-        key = tuple((t.data_ptr(), t._version) for t in src)
-        if getattr(self, "_lin_key", None) != key:
-            H, K = m.hidden_dim, att.num_pixel
-            dev = m.fc.weight.device
-            _, W1_in, b1, _, _ = self._explainer_weights()
-            with torch.no_grad():
-                Wa = torch.zeros(2 * K, 2 * H, device=dev)                 # (out, in): rows 0..K-1 <- h1, K..2K-1 <- s
-                Wa[:K, :H] = att.W_g_proj.weight
-                Wa[K:, H:] = att.W_s_proj.weight
-                ba = torch.cat((torch.zeros(K, device=dev), att.W_s_proj.bias))
-                Wp = m.img_projector.weight.detach().reshape(H, -1)
-                W1t = W1_in.t().contiguous()
-            L = self._linear
-            self._lin = dict(proj=L(Wp, m.img_projector.bias.detach()),
-                             glob=L(m.global_img_feature_proj.weight.detach(), m.global_img_feature_proj.bias.detach()),
-                             wv=L(att.W_v_proj.weight.detach(), att.W_v_proj.bias.detach()), pre1=L(W1t, b1), att=L(Wa, ba),
-                             fc=L(m.fc.weight.detach(), m.fc.bias.detach()))
-            self._lin_key = key
-        return self._lin
+    def _attention_layer(self):
+        """[h | s] @ blockdiag(W_g^T, W_s^T) + [0 | b_s]: both attention projections of a step as one Linear layer
+        (computing them inside the attention kernel re-reads 0.8 MB of weights per image and step: measured slower)."""
+        att = self.model.AdaAttention
+        H, K = att.hidden_dim, att.num_pixel
+        dev = att.W_s_proj.weight.device
+
+        def derive():
+            Wa = torch.zeros(2 * K, 2 * H, device=dev)           # (out, in): rows 0..K-1 <- h, K..2K-1 <- s
+            Wa[:K, :H] = att.W_g_proj.weight
+            Wa[K:, H:] = att.W_s_proj.weight
+            return Wa, torch.cat((torch.zeros(K, device=dev), att.W_s_proj.bias))
+        return self._lx("att", [att.W_g_proj.weight, att.W_s_proj.weight], att.W_s_proj.bias, derive)
 
     def explainer_forward(self, feat, tokens, quirk_double_bias_ih=True, want_gates=False):
         """The explainer's teacher-forced forward (reference :941-1012) batched over images.
@@ -747,24 +719,26 @@ class ExplainGridTDAttention(object):
         att = m.AdaAttention
         K = att.num_pixel
         new = lambda *shape: torch.empty(*shape, device=dev, dtype=torch.float32)
-        lin = self._linears()         # the forward's GEMMs on the tcgen05 kernels (bf16x3: fp32 accuracy), no library GEMM
+        cell, xg, hg = m.AdaLSTM.lstm_cell, m.AdaLSTM.x_gate, m.AdaLSTM.h_gate
         with torch.no_grad():
             feat = feat.contiguous()
             avg = feat.mean(1)
-            A_pre = lin["proj"](feat.view(B * P, C)).view(B, P, H)
+            # every GEMM of this forward runs on the tcgen05 kernels (ops.LinearX3: bf16x3, fp32 accuracy)
+            ipw = m.img_projector.weight
+            A_pre = self._lx("proj", ipw, m.img_projector.bias,
+                             lambda: (ipw.detach().reshape(H, C), m.img_projector.bias.detach()))(feat.view(B * P, C)).view(B, P, H)
             A = A_pre.clamp(min=0)
-            glob_pre = lin["glob"](avg)
+            glob_pre = self._lx("glob", m.global_img_feature_proj.weight, m.global_img_feature_proj.bias)(avg)
             glob = glob_pre.clamp(min=0)
-            img_proj = lin["wv"](A.view(B * P, H)).view(B, P, K)                     # (B,P,K)
-            cell, L = m.AdaLSTM.lstm_cell, m.LanguageLSTM
+            img_proj = self._lx("wv", att.W_v_proj.weight, att.W_v_proj.bias)(A.view(B * P, H)).view(B, P, K)   # (B,P,K)
             W1p, W1_in, b1, W2p, b2 = self._explainer_weights(quirk_double_bias_ih)
-            # both attention projections as ONE GEMM per step: [h1 | s] @ blockdiag(W_g^T, W_s^T) + [0 | b_s]
-            # (computing them inside the attention kernel re-reads 0.8 MB of weights per image and step: measured slower)
+            att_lin = self._attention_layer()
             w_h = att.w_h.weight.reshape(-1).contiguous()
             # ---- state-independent halves for all T steps at once
             emb = m.embedding(tokens[:, :T])                                                     # (B,T,E)
             xin = torch.cat((glob.unsqueeze(1).expand(B, T, E), emb), -1)                        # (B,T,2E)
-            pre1 = lin["pre1"](xin.transpose(0, 1).reshape(T * B, 2 * E)).view(T, B, 5 * H)
+            pre1 = self._lx("pre1", [cell.weight_ih, xg.weight], [cell.bias_ih, cell.bias_hh, xg.bias, hg.bias],
+                            lambda: (W1_in.t().contiguous(), b1))(xin.transpose(0, 1).reshape(T * B, 2 * E)).view(T, B, 5 * H)
             # ---- saved state
             h1, c1, h2, c2 = (torch.zeros(B, T + 1, H, device=dev) for _ in range(4))
             g1, i1, f1, g2, i2, f2, st, ctx, ctx_hat = (new(B, T, H) for _ in range(9))
@@ -782,13 +756,13 @@ class ExplainGridTDAttention(object):
                 ops.lstm_step(hcat[p], W1p, pre1[t], 5, c1[:, t], h1[:, t + 1], c1[:, t + 1], g1[:, t], i1[:, t],
                               f1[:, t], s=st[:, t], h_copy0=hcat[q][:, H:], h_copy1=x2c[p][:, H:2 * H],
                               h_copy2=hs[:, :H], s_copy=hs[:, H:], o=row(o1, t), sg=row(sg, t))
-                hsp = lin["att"](hs)                                                              # (B,2K)
+                hsp = att_lin(hs)                                                                 # (B,2K)
                 ops.adaptive_attention(A, img_proj, hsp, w_h, st[:, t], ctx[:, t], ctx_hat[:, t], alpha[:, t],
                                        beta[:, t], ctx_hat_copy=x2c[p][:, :H])
                 # LanguageLSTM from [ctx_hat_t | h1_{t+1} | h2_t]                                             :984-990
                 ops.lstm_step(x2c[p], W2p, b2, 4, c2[:, t], h2[:, t + 1], c2[:, t + 1], g2[:, t], i2[:, t], f2[:, t],
                               h_copy0=hcat[q][:, :H], h_copy1=x2c[q][:, 2 * H:], o=row(o2, t))
-            pred = lin["fc"]((ctx_hat + h2[:, 1:]).view(B * T, H)).view(B, T, m.vocab_size)
+            pred = self._lx("fc", m.fc.weight, m.fc.bias)((ctx_hat + h2[:, 1:]).view(B * T, H)).view(B, T, m.vocab_size)
             x1 = torch.cat((h2[:, :T], xin), -1)
             x2 = torch.cat((ctx_hat, h1[:, 1:]), -1)
             st_ = dict(x1=x1, x2=x2, g1=g1, i1=i1, f1=f1, g2=g2, i2=i2, f2=f2, st=st, ctx=ctx, ctx_hat=ctx_hat,
@@ -884,33 +858,43 @@ class ExplainGridTDAttention(object):
         self._state, self._enc_state, self._feat_hw = st, est, (fh, fw)
         self.caption_length = len(tokens) - 1
         self.num_pixels = feat.shape[1]
-        # attributes the reference exposes (read by evaluation.py: .predictions .alphas .betas ...)
+        self.image_features = feat[0].t().reshape(1, feat.shape[2], fh, fw)
+        self._expose_state(st)
+
+    def _expose_state(self, st):
+        """attributes the reference exposes (read by evaluation.py: .predictions .alphas .betas ...)"""
         self.predictions, self.alphas, self.betas = st["pred"][0], st["alpha"][0], st["beta"][0]
         self.x1t, self.x2t = st["x1"][0], st["x2"][0]
         self.h1t, self.c1t, self.h2t, self.c2t = st["h1"][0], st["c1"][0], st["h2"][0], st["c2"][0]
         self.g1t, self.i1t_act, self.f1t_act = st["g1"][0], st["i1"][0], st["f1"][0]
         self.g2t, self.i2t_act, self.f2t_act = st["g2"][0], st["i2"][0], st["f2"][0]
         self.st, self.context, self.context_hat = st["st"][0], st["ctx"][0], st["ctx_hat"][0]
-        C = feat.shape[2]
-        self.image_features = feat[0].t().reshape(1, C, fh, fw)
         self.avg_feature = st["avg"][0]
 
-    def _decoder_lrp(self, ts):
+    def _decode(self, st, req_img, req_t, req_word, tc_gemm, head_idx=0, ws_cache=None):
+        """The decoder kernels of this explainer for the (image, word) requests on the explainer forward's state ``st``:
+        -> ((Q,P,C) relevance or gradient of the encoder output, (Q,T) word relevances).  ``head_idx``: the attention
+        head an AoA explanation follows; ``ws_cache``: ops._decoder_workspace (the relevance decoders)."""
+        return ops.gridtd_decoder_lrp(st, self._lrp_weights(), req_img, req_t, req_word, tc_gemm=tc_gemm,
+                                      ws_cache=ws_cache)
+
+    def _decode_words(self, ts, head_idx=0):
+        """``_decode`` for the words ``ts`` of the caption ``_set_state`` saved"""
+        i32 = lambda v: torch.tensor(v, dtype=torch.int32, device=self.device)
         toks = self.beam_caption_encode
-        dev = self.device
-        req_t = torch.tensor(ts, dtype=torch.int32, device=dev)
-        req_word = torch.tensor([toks[t + 1] for t in ts], dtype=torch.int32, device=dev)
-        req_img = torch.zeros(len(ts), dtype=torch.int32, device=dev)
-        return ops.gridtd_decoder_lrp(self._state, self._lrp_weights(), req_img, req_t, req_word,
-                                      tc_gemm=(self.precision in ('bf16', 'mixed')))
+        return self._decode(self._state, i32([0] * len(ts)), i32(list(ts)), i32([toks[t + 1] for t in ts]),
+                            self.tc_gemm, head_idx)
 
     def explain_caption_wordt(self, t):
-        """reference :1014-1135 -> (r_img_feature (1,C,h,w), r_words (t+1,))."""
+        """reference :1014-1135 -> (r_img_feature (1,C,h,w), r_words (t+1,)); the gradient classes: the image
+        feature's gradient."""
+        return self._explain_word(t)
+
+    def _explain_word(self, t, head_idx=0):
         assert t < self.caption_length
-        r_feat, r_words = self._decoder_lrp([t])
+        r_feat, r_words = self._decode_words([t], head_idx)
         fh, fw = self._feat_hw
-        r_img_feature = r_feat[0].t().reshape(1, -1, fh, fw)
-        return r_img_feature, r_words[0, :t + 1]
+        return r_feat[0].t().reshape(1, -1, fh, fw), r_words[0, :t + 1]
 
     def explain_cnn(self, r_img_feature):
         """reference :1137-1139: relevance of the encoder output -> relevance of the image (1,3,H,W)."""
@@ -922,30 +906,37 @@ class ExplainGridTDAttention(object):
             lrp_wrapper.add_lrp(enc)
         return enc.compute_lrp(self.img, target=r_img_feature, precision='simt')
 
+    def _explain_image(self, r_feat):
+        """explain_cnn for each of the (Q,P,C) encoder-output relevances of the saved image -> (Q,3,H,W)"""
+        if self.uses_tc:
+            return self.engine().relevance(self._enc_state, r_feat,
+                                           torch.zeros(r_feat.shape[0], dtype=torch.int32, device=self.device))
+        enc = self.model.img_encoder.encoder
+        lrp_wrapper.add_lrp(enc)
+        fh, fw = self._feat_hw
+        return torch.cat([lrp_wrapper.compute_lrp(enc, self.img.detach().clone(), precision='simt',
+                                                  target=r_feat[t].t().reshape(1, -1, fh, fw)) for t in range(r_feat.shape[0])])
+
     def explain_caption(self, img_filepath, t_list=None):
         """reference :1141-1156 -> (relevance_imgs [T x (1,3,H,W)], relevance_preceeding_words [T x (t+1,)]).
         All words of the caption are explained in one batched decoder call + one batched encoder chain."""
+        return self._explain_caption(img_filepath, 0, t_list)
+
+    def _explain_caption(self, img_filepath, head_idx, t_list):
         self.img_filepath = img_filepath
         self.get_hidden_parameters(img_filepath)
         T = self.caption_length
         if T == 0:
             return [], []
-        r_feat, r_words = self._decoder_lrp(list(range(T)))
-        if self.uses_tc:
-            rows = torch.zeros(T, dtype=torch.int32, device=self.device)
-            heat = self.engine().relevance(self._enc_state, r_feat, rows)
-        else:
-            enc = self.model.img_encoder.encoder
-            lrp_wrapper.add_lrp(enc)
-            fh, fw = self._feat_hw
-            heat = torch.cat([lrp_wrapper.compute_lrp(enc, self.img.detach().clone(), precision='simt',
-                                                      target=r_feat[t].t().reshape(1, -1, fh, fw)) for t in range(T)])
+        r_feat, r_words = self._decode_words(range(T), head_idx)
+        heat = self._explain_image(r_feat)
         if self.ACCUMULATE_LIKE_REFERENCE:
             heat = torch.cumsum(heat, 0)
         relevance_imgs = [heat[t:t + 1] for t in range(T)]
         relevance_preceeding_words = [r_words[t, :t + 1] for t in range(T)]
         self.visualize_explanations(relevance_imgs, t=t_list)
-        self.save_linguistic_explanation(relevance_preceeding_words)
+        if self.SAVE_LINGUISTIC:
+            self.save_linguistic_explanation(relevance_preceeding_words)
         return relevance_imgs, relevance_preceeding_words
 
     def save_linguistic_explanation(self, relevance_preceeding_words):
@@ -982,37 +973,16 @@ class ExplainGridTDGradient(GradientFamily, ExplainGridTDAttention):
         ExplainGridTDAttention.__init__(self, args, word_map, model=model, precision=precision)
         self._check_encoder()
 
-    def _grad_weights(self):
-        return self._cached_grad_weights(gridtd_grad_weights)
+    _GRAD_WEIGHTS = staticmethod(gridtd_grad_weights)
+    SAVE_LINGUISTIC = False               # like the reference's gridTD gradient explainers
 
-    def _set_state(self, img, tokens, enc=None):
-        ExplainGridTDAttention._set_state(self, img, tokens, enc)
-        if self._state is not None:
-            st = self._state
-            self.o1t_act, self.o2t_act, self.sen_gate = st["o1"][0], st["o2"][0], st["sg"][0]
+    def _expose_state(self, st):
+        ExplainGridTDAttention._expose_state(self, st)
+        self.o1t_act, self.o2t_act, self.sen_gate = st["o1"][0], st["o2"][0], st["sg"][0]
 
-    def _decoder_grad(self, ts):
-        toks = self.beam_caption_encode
-        i32 = lambda v: torch.tensor(v, dtype=torch.int32, device=self.device)
-        return ops.gridtd_decoder_grad(self._state, self._grad_weights(), i32([0] * len(ts)), i32(list(ts)),
-                                       i32([toks[t + 1] for t in ts]), guided=self.GUIDED_DECODER,
-                                       tc_gemm=(self.precision in ('bf16', 'mixed')))
-
-    def explain_caption_wordt(self, t):
-        """reference :1424-1508 (guided: :1588-1675) -> (d_img_feature (1,C,h,w), r_words (t+1,))."""
-        assert t < self.caption_length
-        d_feat, r_words = self._decoder_grad([t])
-        fh, fw = self._feat_hw
-        return d_feat[0].t().reshape(1, -1, fh, fw), r_words[0, :t + 1]
-
-    def explain_caption(self, img_filepath, t_list=None):
-        """reference :1525-1539: every word of the caption in one batched decoder call + one batched encoder pass."""
-        self.img_filepath = img_filepath
-        self.get_hidden_parameters(img_filepath)
-        if self.caption_length == 0:
-            return [], []
-        d_feat, r_words = self._decoder_grad(list(range(self.caption_length)))
-        return self._explain_all(d_feat, r_words)
+    def _decode(self, st, req_img, req_t, req_word, tc_gemm, head_idx=0, ws_cache=None):
+        return ops.gridtd_decoder_grad(st, self._grad_weights(), req_img, req_t, req_word, guided=self.GUIDED_DECODER,
+                                       tc_gemm=tc_gemm)
 
 
 class ExplainiGridTDGuidedGradient(ExplainGridTDGradient):

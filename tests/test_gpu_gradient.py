@@ -178,7 +178,7 @@ def test_encoder_gradient_vs_oracle(precision, guided):
         ws = [sd[k] for k in sd if k.endswith("weight")]
         bs = [sd[k] for k in sd if k.endswith("bias")]
         rule = "guided" if guided else "gradient"
-        eng = (tc.TcVggGradientHybrid(ws, bs, cfg, DEV, rule=rule) if precision == "bf16" else
+        eng = (tc.TcVggMixed(ws, bs, cfg, DEV, rule=rule) if precision == "bf16" else
                tc.TcVggEngine(ws, bs, cfg, DEV, precision=precision, rule=rule))
         st = eng.forward(x.to(DEV))
         assert_close(eng.features(st, "nchw"), feat, rtol=1e-4, atol=2e-5 * float(feat.abs().max()), what="features")
@@ -199,7 +199,7 @@ def test_encoder_gradient_vs_oracle(precision, guided):
         assert_close(got / scale, want / scale, rtol=1e-4, atol=1e-5, what="simt gradient")
     elif precision == "fp32":
         assert _rel_l2(got, want) < (3e-3 if guided else 3e-2) and spearman(got, want) > 0.999
-    else:       # bf16 chain on the fp32-accurate forward's masks (TcVggGradientHybrid): the mask flips dominate, as above
+    else:       # bf16 chain on the fp32-accurate forward's masks (TcVggMixed): the mask flips dominate, as above
         assert _rel_l2(got, want) < (5e-3 if guided else 4e-2) and spearman(got, want) > 0.999
 
 

@@ -457,3 +457,94 @@ def test_decoder_workspace_cache_keyed_on_weights(monkeypatch):
     W["W_a"].sub_(1.0)
     _, e3, k3 = ops._decoder_workspace(cache, "gridtd", (1, 2, 3), 100, "cuda", True, W)
     assert e3 == 0 and k3 not in (None, key, k2)
+
+
+_DECODERS = ("gridtd_decoder_lrp", "aoa_decoder_lrp", "adaptive_decoder_lrp", "gridtd_decoder_grad", "aoa_decoder_grad",
+             "adaptive_decoder_grad")
+
+
+@pytest.fixture(scope="module")
+def small_models():
+    from models import gridTDmodel as G, aoamodel as A, adaptiveattention as AA
+    torch.manual_seed(0)
+    V, H, E = 30, 64, 32
+    return {"gridtd": G.GridTDModel(E, H, V, "vgg16"), "aoa": A.AOAModel(E, H, 8, V, "vgg16"),
+            "adaptive": AA.AdaptiveAttentionCaptioningModel(H, H, V, "vgg16")}
+
+
+@pytest.mark.parametrize("cls_name", [
+    "gridTDmodel.ExplainGridTDAttention", "gridTDmodel.ExplainGridTDGradient", "gridTDmodel.ExplainiGridTDGuidedGradient",
+    "gridTDmodel.ExplainGridTDGradCam", "gridTDmodel.ExplainGridTDGuidedGradCam",
+    "aoamodel.ExplainAOAAttention", "aoamodel.ExplainAOAGradient", "aoamodel.ExplainAOAGuidedGradient",
+    "aoamodel.ExplainAOAGradCam", "aoamodel.ExplainAOAGuidedGradCam",
+    "adaptiveattention.ExplainAdaptiveAttention", "adaptiveattention.ExplainAdaptiveGradient",
+    "adaptiveattention.ExplainiAdaptiveGuidedGradient", "adaptiveattention.ExplainAdaptiveGradCam",
+    "adaptiveattention.ExplainAdaptiveGuidedGradCam"])
+def test_explainer_decode_reaches_its_decoder(small_models, tmp_path, monkeypatch, cls_name):
+    """``_decode`` of each of the 15 explainer classes calls the batched decoder entry point of its family and kind with
+    the class's cached weights, the AoA head count and per-request head, the gridTD guided flag and (relevance
+    decoders only) the caller's workspace cache; ``_decode_words`` turns caption positions into image-0 requests."""
+    import importlib
+    from lrpx import ops
+    mod_name, name = cls_name.split(".")
+    cls = getattr(importlib.import_module("models." + mod_name), name)
+    family = {"gridTDmodel": "gridtd", "aoamodel": "aoa", "adaptiveattention": "adaptive"}[mod_name]
+    model = small_models[family]
+    args = argparse.Namespace(embed_dim=model.embed_dim, hidden_dim=model.hidden_dim, num_head=8, encoder="vgg16",
+                              height=224, width=224, save_path=str(tmp_path), dataset="syn", weight="")
+    ex = cls(args, synth.word_map(model.vocab_size), model=model)
+    calls = []
+    for fn in _DECODERS:
+        monkeypatch.setattr(ops, fn, lambda *a, _fn=fn, **kw: calls.append((_fn, a, kw)) or ("r_feat", "r_words"))
+    kind = "grad" if ex.GRADIENT else "lrp"
+    assert ex.GRADIENT == ("Attention" not in name)
+    W = ex._grad_weights() if ex.GRADIENT else ex._lrp_weights()
+    st, ws = {"feat": None}, {}
+    i32 = lambda v: torch.tensor(v, dtype=torch.int32)
+    req_img, req_t, req_word = i32([0, 1]), i32([2, 0]), i32([5, 6])
+    assert ex._decode(st, req_img, req_t, req_word, True, 3, ws) == ("r_feat", "r_words")
+    (fn, a, kw), = calls
+    assert fn == f"{family}_decoder_{kind}"
+    assert a[0] is st and a[1] is W and kw["tc_gemm"] is True
+    reqs = a[3:] if family == "aoa" else a[2:]
+    assert [r.tolist() for r in reqs[:3]] == [[0, 1], [2, 0], [5, 6]]
+    if family == "aoa":
+        assert a[2] == 8 and reqs[3].tolist() == [3, 3]
+    else:
+        assert len(reqs) == 3
+    if kind == "lrp":
+        assert kw["ws_cache"] is ws and set(kw) == {"tc_gemm", "ws_cache"}
+    elif family == "gridtd":
+        assert kw["guided"] is ex.GUIDED_DECODER and set(kw) == {"tc_gemm", "guided"}
+        assert ex.GUIDED_DECODER == ("Guided" in name)
+    else:
+        assert set(kw) == {"tc_gemm"}
+    # the per-image path: requests of image 0 for the words of the saved caption, tc_gemm from the precision
+    calls.clear()
+    ex._state, ex.beam_caption_encode = st, [1, 7, 8, 9]
+    ex._decode_words([0, 2], 1)
+    (fn, a, kw), = calls
+    reqs = a[3:] if family == "aoa" else a[2:]
+    assert [r.tolist() for r in reqs[:3]] == [[0, 0], [0, 2], [7, 9]] and kw["tc_gemm"] is False
+    assert family != "aoa" or reqs[3].tolist() == [1, 1]
+
+
+def test_weight_cache_rebuilds_on_weight_or_key_change():
+    """ops.WeightCache: the same object while the sources and the extra key are unchanged; rebuilt (under no_grad) after
+    an in-place update, a replaced tensor or another extra key."""
+    from lrpx import ops
+    p = torch.nn.Parameter(torch.ones(3))
+    q = torch.zeros(2)
+    cache, built = ops.WeightCache(), []
+
+    def build():
+        built.append(1)
+        return p * 2
+    first = cache.get([p, q], build, (1,))
+    assert cache.get([p, q], build, (1,)) is first and len(built) == 1 and not first.requires_grad
+    with torch.no_grad():
+        p.add_(1.0)
+    second = cache.get([p, q], build, (1,))
+    assert second is not first and torch.equal(second, torch.full((3,), 4.0)) and len(built) == 2
+    assert cache.get([p, q], build, (2,)) is not second and len(built) == 3
+    assert cache.get([p, torch.zeros(2)], build, (2,)) is not second and len(built) == 4
