@@ -380,6 +380,12 @@ int lrpx_grad_cam_f32(const float* feat, const float* grads, const int32_t* req_
 int lrpx_cam_expand_mul_f32(const float* g, const float* cam, const float* Kh, const float* Kw, float* out, int Q, int C,
                             int h, int w, int H, int W, void* stream);
 
+/* Guided Grad-CAM's expansion along y (gridTDmodel.py:1826-1828), the first half of Kh cam_q Kw^T:
+ *   out[q][y][j] = sum_i Kh[y][i] * cam[q][i][j]   (fmaf over i = 0..h-1, lrpx_cam_expand_mul_f32's order)
+ * cam (Q,h,w), Kh (H,h), out (Q,H,w).  The tensor-core chain's INPUT3 epilogue applies the x half (cam_rows / cam_kw
+ * of lrpx_tc_conv_args) where it forms the image gradient, so the guided gradient is never stored un-multiplied. */
+int lrpx_cam_expand_rows_f32(const float* cam, const float* Kh, float* out, int Q, int h, int w, int H, void* stream);
+
 /* lrp_tune weights, batched (gridTDmodel.py:549-578, aoamodel.py:597-626, utils.py:55-64):
  *   w = argmax logits[b]; if is_stop[w] -> weights 1; else r = fc-row eps rule, split to h / ctx,
  *   weights = r / max|r| + 1.   No host synchronisation; is_stop is a device byte mask (V). */
@@ -583,7 +589,10 @@ enum {
    * 6..7: zero) holds, K-ordered (filter row dy, channel), the weights of filter tap (dy, dx); the kernel adds the
    * three column-shifted partial sums in its epilogue.  Same output as LRPX_TC_EPI_INPUT (3x3 only).
    * gain_mode selects the delivery format of the heat-map: 0 = fp32 (n, 3, h, w), 1 = channel mean fp32 (n, h, w)
-   * (evaluation.py:134,411,503 reduce every heat-map with torch.mean(relevance, dim=(0,1)) first), 2 = fp16 (n, 3, h, w). */
+   * (evaluation.py:134,411,503 reduce every heat-map with torch.mean(relevance, dim=(0,1)) first), 2 = fp16 (n, 3, h, w).
+   * With cam_rows set (guided rule only) every pixel's three values are first multiplied by Guided Grad-CAM's expanded map
+   *   v[e][y][x] = sum_j cam_kw[x][j] * cam_rows[e][y][j]   (fmaf over j = 0..cam_w-1, lrpx_cam_expand_mul_f32's order)
+   * so format 0 equals lrpx_cam_expand_mul_f32 of the un-multiplied output bit for bit, and 1 / 2 are its formats. */
   LRPX_TC_EPI_INPUT3 = 8,
   /* General relevance epilogue (any alpha/beta, the epsilon rule, bf16 or fp32-accurate storage):
    *   for group j < groups:  v_j = acc[p][n] * gain_j[img(p)][rem(p)][n]
@@ -673,6 +682,10 @@ typedef struct {
   int out_pitch;        /* STORE_F32: floats per row of `out` (0 = ncol) and                                */
   int n_valid;          /*            the columns that exist (<= ncol; the weight rows beyond are padding);
                          *            `bias` (n_valid floats) is added when given                           */
+  /* ---- Guided Grad-CAM factor of INPUT3 with rule 3 (NULL cam_rows: no factor) */
+  const float* cam_rows;  /* fp32 (n_img, h, cam_w): lrpx_cam_expand_rows_f32 of each block's Grad-CAM map       */
+  const float* cam_kw;    /* fp32 (w, cam_w): the expansion along x (the Kw of lrpx_cam_expand_mul_f32)          */
+  int cam_w;              /* width of the Grad-CAM map, 1..64                                                    */
 } lrpx_tc_conv_args;
 
 int lrpx_tc_conv(const lrpx_tc_conv_args* args, void* stream);

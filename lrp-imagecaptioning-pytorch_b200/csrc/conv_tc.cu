@@ -124,6 +124,9 @@ struct TcParams {
   const float* x1;
   void* out;
   void* out2;
+  const float* cam_rows;   // INPUT3, guided rule: Guided Grad-CAM's map expanded along y (n_img, h, cam_w), or nullptr
+  const float* cam_kw;     // (w, cam_w): its expansion along x
+  int cam_w;
 };
 
 // ------------------------------------------------------------------------------------------ PTX wrappers
@@ -613,6 +616,7 @@ __device__ __forceinline__ void epi_release(const TcParams& p, uint32_t release_
 // Neighbouring rows are neighbouring TMEM lanes = neighbouring threads: warp shuffles, plus a 48-byte exchange through
 // shared memory at the three warp boundaries of a 128-row block.  The first and last row of a block have no neighbour,
 // so the M halves of a tile start 126 rows apart and a tile yields 252 output rows.
+template <bool CAM>
 __device__ __forceinline__ void epi_input3(const TcParams& p, const RowInfo& r, uint32_t taddr, uint32_t release_bar,
                                            float* scratch /* [4 quarters][2][8] of this (buffer, half) */, int quarter,
                                            int bar_id, uint32_t full_bar, uint32_t full_parity) {
@@ -627,6 +631,15 @@ __device__ __forceinline__ void epi_input3(const TcParams& p, const RowInfo& r, 
   if (writes)
 #pragma unroll
     for (int c = 0; c < 3; ++c) xin[c] = __ldg(p.x + ((size_t)img * 3 + c) * hw + pix);
+  // Guided Grad-CAM: this pixel's factor (Kw cam_rows^T)[y][x], formed in lrpx_cam_expand_mul_f32's fmaf order; its loads
+  // and sum run, like the input values', before the accumulator wait
+  float cam_v = 1.f;
+  if (CAM && writes) {
+    const float* t = p.cam_rows + ((size_t)r.e * p.h + (r.a - 1)) * p.cam_w;
+    const float* kw = p.cam_kw + (size_t)(r.b - 1) * p.cam_w;
+    cam_v = 0.f;
+    for (int j = 0; j < p.cam_w; ++j) cam_v = fmaf(__ldg(kw + j), __ldg(t + j), cam_v);
+  }
   // only now wait for the tile's accumulator: the row arithmetic and the two dependent loads above (request -> image, image
   // -> pixel values) used to start AFTER the wait and sat, with the integer divisions of tile_coords, on the pass's critical
   // path — the layer's tile time is the latency of one such pass (two warp sets alternate), not its bytes or its MMAs
@@ -673,6 +686,10 @@ __device__ __forceinline__ void epi_input3(const TcParams& p, const RowInfo& r, 
     // rules 2 / 3 (gradient family): the gradient with respect to the image itself, no multiplication by x
     res[c] = p.rule >= 2 ? cp : fmaxf(xv, 0.f) * cp + fminf(xv, 0.f) * cn;
   }
+  // a rounded product (never contracted into the channel mean's additions): the same value lrpx_cam_expand_mul_f32 stores
+  if (CAM)
+#pragma unroll
+    for (int c = 0; c < 3; ++c) res[c] = __fmul_rn(res[c], cam_v);
   // delivery format (gain_mode): 0 = fp32 (Q,3,h,w), the reference's return value; 1 = channel mean fp32 (Q,h,w) — what
   // every consumer in evaluation.py reduces a heat-map to first (:134,:411,:503: torch.mean(relevance, dim=(0,1)));
   // 2 = fp16 (Q,3,h,w)
@@ -1082,10 +1099,13 @@ constexpr int TC_EPI_FWDX_SIMPLE = 12;
 constexpr int TC_EPI_MUL_FOLD = 15;         // MUL with the three filter COLUMNS folded into N (64-channel layers, epi_mul_fold)
 constexpr int TC_EPI_MULX_S = 13, TC_EPI_MULX_UNPOOL_S = 14;      // MULX / MULX_UNPOOL with one gain group, no addend (epi_mulx)
 constexpr int TC_EPI_FWDX_SPLIT_ADD = 16;   // FWDX with split rows and a residual operand (idn / hd): epi_fwdx<true>
+constexpr int TC_EPI_INPUT3_CAM = 17;       // INPUT3 with Guided Grad-CAM's factor (cam_rows): epi_input3<true>, on its own so
+                                            // that the factor's loop does not cost the plain first layer registers
+__host__ __device__ constexpr bool is_input3(int epi) { return epi == LRPX_TC_EPI_INPUT3 || epi == TC_EPI_INPUT3_CAM; }
 
 // number of 32-column units per (lane quarter, M half) of a tile
 __device__ __forceinline__ int epi_units_per_half(const TcParams& p, int epi) {
-  if (epi == LRPX_TC_EPI_INPUT || epi == LRPX_TC_EPI_INPUT3) return 1;
+  if (epi == LRPX_TC_EPI_INPUT || is_input3(epi)) return 1;
   if (epi == TC_EPI_MUL_FOLD) return 4;                   // four units of 16 output channels (`c` counts 32 per unit: c >> 1)
   if (epi == TC_EPI_FWDX_SIMPLE) return p.half >> 4;      // 16-column units (run_epilogue_tile: c = u << 4)
   const int ncols = (epi == LRPX_TC_EPI_FWD_GAIN || epi == LRPX_TC_EPI_FWDX || epi == TC_EPI_FWDX_SIMPLE ||
@@ -1102,15 +1122,15 @@ __device__ __forceinline__ void epi_unit(const TcParams& p, const RowInfo& r0, u
                                          float* scratch = nullptr, int quarter = 0, int bar_id = 0, uint32_t full_bar = 0,
                                          uint32_t full_parity = 0) {
   if (p.debug_flags & 16) {             // timing experiment: only hands the accumulator back
-    if (EPI == LRPX_TC_EPI_INPUT3) { mbar_wait_ns(full_bar, full_parity, (uint32_t)p.sleep_ns); tc_fence_after(); }
+    if (is_input3(EPI)) { mbar_wait_ns(full_bar, full_parity, (uint32_t)p.sleep_ns); tc_fence_after(); }
     epi_release(p, release_bar);
     return;
   }
   RowInfo r = r0;
   if (p.debug_flags & 1) { r.in_range = false; r.valid = false; }
   const int n0 = n_tile * p.bn;
-  if (EPI == LRPX_TC_EPI_INPUT3) {
-    epi_input3(p, r, taddr, release_bar, scratch, quarter, bar_id, full_bar, full_parity);
+  if (is_input3(EPI)) {
+    epi_input3<EPI == TC_EPI_INPUT3_CAM>(p, r, taddr, release_bar, scratch, quarter, bar_id, full_bar, full_parity);
   } else if (EPI == TC_EPI_MUL_FOLD) {
     epi_mul_fold(p, r0, taddr, c >> 1, release_bar, scratch, quarter, bar_id);
   } else if (EPI == LRPX_TC_EPI_MULX) {
@@ -1291,13 +1311,13 @@ __device__ __forceinline__ void run_epilogue_tile(const TcParams& p, int row_bas
   // LATENCY of one epilogue pass.  Warps 0,1 of a quarter therefore take the even tiles and warps 2,3 the odd ones, so
   // the passes of the two accumulator buffers overlap.
   int set = 0;
-  if ((EPI == LRPX_TC_EPI_INPUT || EPI == LRPX_TC_EPI_INPUT3) && n_units <= 2) {
+  if ((EPI == LRPX_TC_EPI_INPUT || is_input3(EPI)) && n_units <= 2) {
     set = it & 1;
     sub = set ? sub - 2 : sub;
     if (sub < 0 || sub >= 2) sub = n_units;          // not this warp's tile
   }
   if (sub >= n_units) {                 // nothing to read for this warp: hand the buffer back at once
-    if (EPI == LRPX_TC_EPI_INPUT3) { mbar_wait_ns(full_bar, full_parity, (uint32_t)p.sleep_ns); tc_fence_after(); }
+    if (is_input3(EPI)) { mbar_wait_ns(full_bar, full_parity, (uint32_t)p.sleep_ns); tc_fence_after(); }
     epi_release(p, release_bar);
     return;
   }
@@ -1310,12 +1330,12 @@ __device__ __forceinline__ void run_epilogue_tile(const TcParams& p, int row_bas
   RowInfo r{};
   for (int u = sub; u < n_units; u += step) {
     const int h = u >= uph ? 1 : 0, c = (u - h * uph) << (EPI == TC_EPI_FWDX_SIMPLE ? 4 : 5);      // mh <= 2
-    const int hr = (EPI == LRPX_TC_EPI_INPUT3) ? p.half_rows : TC_BM;
+    const int hr = (is_input3(EPI)) ? p.half_rows : TC_BM;
     if (h != h_cached) {
       r = row_info(p, row_base + h * hr);
       h_cached = h;
       // walk mode: the tiles are tile_stride (< tile_out_rows) rows apart; rows past the stride belong to the next tile
-      if (EPI == LRPX_TC_EPI_INPUT3 && p.walk && h * hr + quarter * 32 + (int)(threadIdx.x & 31) - p.fold >= p.tile_stride)
+      if (is_input3(EPI) && p.walk && h * hr + quarter * 32 + (int)(threadIdx.x & 31) - p.fold >= p.tile_stride)
         r.valid = false;
     }
     if (pf_row_base >= 0) epi_prefetch_unit<EPI>(p, pf_row_base + h * TC_BM, n_tile, c);
@@ -1659,7 +1679,7 @@ tc_conv_slab_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_const
       mbar_init(smem_u32(&tmem_full_bar[b]), p.n_issuers);
       // pair: the leader's issuers wait for the epilogue warps of BOTH CTAs (the peer's arrive remotely)
       // (first-layer epilogues: only the 4 * mh warps of the tile's set read the buffer, see the epilogue loop)
-      mbar_init(smem_u32(&tmem_empty_bar[b]), (EPI == LRPX_TC_EPI_INPUT || EPI == LRPX_TC_EPI_INPUT3)
+      mbar_init(smem_u32(&tmem_empty_bar[b]), (EPI == LRPX_TC_EPI_INPUT || is_input3(EPI))
                                                   ? 4 * p.mh : (PAIR ? 2 * TC_EPI_WARPS : TC_EPI_WARPS));
     }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -1843,7 +1863,7 @@ tc_conv_slab_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_const
     // warp walks ONLY its own set's tiles — a tile of that layer costs the SM ~5300 warp instructions, it is bound by
     // instruction issue, and a third of them were the other set's (and the unit-less warps') trips through this loop just to
     // hand the buffer back; the buffer's "empty" barrier counts the 4 * mh warps that actually read it.
-    constexpr bool kSets = EPI == LRPX_TC_EPI_INPUT || EPI == LRPX_TC_EPI_INPUT3;
+    constexpr bool kSets = EPI == LRPX_TC_EPI_INPUT || is_input3(EPI);
     const int sub0 = (warp - 2) >> 2;
     int it = 0, it_step = 1;
     bool idle = false;
@@ -1859,7 +1879,7 @@ tc_conv_slab_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_const
       const uint32_t acc_phase = (it >> p.nbuf_log2) & 1;
       int m_tile, n_tile;
       tile_coords(p, tile, m_tile, n_tile);
-      if (EPI != LRPX_TC_EPI_INPUT3) {          // INPUT3 waits inside its epilogue, after its loads are in flight
+      if (!is_input3(EPI)) {                    // INPUT3 waits inside its epilogue, after its loads are in flight
         mbar_wait_ns(smem_u32(&tmem_full_bar[buf]), acc_phase, (uint32_t)p.sleep_ns);
         tc_fence_after();
       }
@@ -1873,8 +1893,8 @@ tc_conv_slab_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_const
       if (PAIR) rel_bar = mapa_u32(rel_bar, 0);          // shared::cluster address of the LEADER's barrier (both ranks)
       run_epilogue_tile<EPI>(p, m_tile * tile_rows - p.fold + quarter * 32 + lane, taddr, n_tile, (warp - 2) >> 2, p.mh,
                              pf_row, rel_bar, stage, &tmO,
-                             EPI == LRPX_TC_EPI_INPUT3 ? &in3_scratch[it & 1][(it >> 1) & 1][0]
-                                                       : (EPI == TC_EPI_MUL_FOLD ? &in3_scratch[it & 1][0][0] : nullptr),
+                             is_input3(EPI) ? &in3_scratch[it & 1][(it >> 1) & 1][0]
+                                            : (EPI == TC_EPI_MUL_FOLD ? &in3_scratch[it & 1][0][0] : nullptr),
                              quarter, it, smem_u32(&tmem_full_bar[buf]), acc_phase);
     }
     if (EPI == LRPX_TC_EPI_MUL && p.store_off) {      // the staging block must outlive the last tile store's read
@@ -2149,6 +2169,10 @@ extern "C" int lrpx_tc_conv(const lrpx_tc_conv_args* a, void* stream) {
   p.add = a->add; p.add_pitch = a->add_pitch; p.gain3 = a->gain3; p.gain4 = a->gain4;
   p.bn_w = a->bn_w; p.bn_b = a->bn_b; p.idn = a->idn; p.hd = a->hd; p.out4 = a->out4; p.out5 = a->out5;
   p.fwd_flags = a->fwd_flags;
+  LRPX_CHECK_ARG(!a->cam_rows || (epi == LRPX_TC_EPI_INPUT3 && a->rule == 3),
+                 "cam_rows: Guided Grad-CAM's factor needs the INPUT3 epilogue and the guided rule (3)");
+  LRPX_CHECK_ARG(!a->cam_rows || (a->cam_kw && a->cam_w > 0 && a->cam_w <= 64), "cam_rows needs cam_kw and 0 < cam_w <= 64");
+  p.cam_rows = a->cam_rows; p.cam_kw = a->cam_kw; p.cam_w = a->cam_w;
 
   if (epi == LRPX_TC_EPI_FWDX) {
     LRPX_CHECK_ARG(a->out2 && a->n_acc >= 1 && a->n_acc <= 3 && a->ncol % a->n_acc == 0, "FWDX: out2 and n_acc in 1..3");
@@ -2380,7 +2404,9 @@ extern "C" int lrpx_tc_conv(const lrpx_tc_conv_args* a, void* stream) {
           return launch_tc_slab<LRPX_TC_EPI_MUL>(ma0, ma1, mb, mbh, mo, p, grid, st);
         case LRPX_TC_EPI_MUL_UNPOOL: return launch_tc_slab<LRPX_TC_EPI_MUL_UNPOOL>(ma0, ma1, mb, mbh, mo, p, grid, st);
         case LRPX_TC_EPI_INPUT: return launch_tc_slab<LRPX_TC_EPI_INPUT>(ma0, ma1, mb, mbh, mo, p, grid, st);
-        case LRPX_TC_EPI_INPUT3: return launch_tc_slab<LRPX_TC_EPI_INPUT3>(ma0, ma1, mb, mbh, mo, p, grid, st);
+        case LRPX_TC_EPI_INPUT3:
+          if (p.cam_rows) return launch_tc_slab<TC_EPI_INPUT3_CAM>(ma0, ma1, mb, mbh, mo, p, grid, st);
+          return launch_tc_slab<LRPX_TC_EPI_INPUT3>(ma0, ma1, mb, mbh, mo, p, grid, st);
         case LRPX_TC_EPI_MULX:
           if (p.mulx_simple) return launch_tc_slab<TC_EPI_MULX_S>(ma0, ma1, mb, mbh, mo, p, grid, st);
           return launch_tc_slab<LRPX_TC_EPI_MULX>(ma0, ma1, mb, mbh, mo, p, grid, st);

@@ -470,6 +470,20 @@ __global__ void __launch_bounds__(256) cam_expand_mul_kernel(const float* __rest
   }
 }
 
+// the y half of that expansion on its own, with the first loop's fmaf order: out[q][y][j] = sum_i Kh[y][i] * cam[q][i][j].
+// One thread per output value.
+__global__ void __launch_bounds__(256) cam_expand_rows_kernel(const float* __restrict__ cam, const float* __restrict__ Kh,
+                                                              float* __restrict__ out, long long n, int h, int w, int H) {
+  const long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= n) return;
+  const int j = (int)(k % w);
+  const int y = (int)((k / w) % H);
+  const long long q = k / ((long long)w * H);
+  float s = 0.f;
+  for (int i = 0; i < h; ++i) s = fmaf(Kh[(size_t)y * h + i], cam[((size_t)q * h + i) * w + j], s);
+  out[k] = s;
+}
+
 }  // namespace lrpx
 
 using namespace lrpx;
@@ -649,6 +663,16 @@ int lrpx_cam_expand_mul_f32(const float* g, const float* cam, const float* Kh, c
   LRPX_CHECK_ARG((size_t)w * sizeof(float) <= 48 * 1024 && H <= 65535 && Q <= 65535, "map too large");
   if (Q == 0) return LRPX_OK;
   cam_expand_mul_kernel<<<dim3(H, Q), 256, (size_t)w * sizeof(float), as_stream(stream)>>>(g, cam, Kh, Kw, out, C, h, w, H, W);
+  LRPX_CHECK_LAUNCH();
+  return LRPX_OK;
+}
+
+int lrpx_cam_expand_rows_f32(const float* cam, const float* Kh, float* out, int Q, int h, int w, int H, void* stream) {
+  LRPX_CHECK_ARG(cam && Kh && out && Q >= 0 && h > 0 && w > 0 && H > 0, "bad argument");
+  const long long n = (long long)Q * H * w;
+  LRPX_CHECK_ARG((n + 255) / 256 <= 0x7fffffffLL, "map too large");
+  if (n == 0) return LRPX_OK;
+  cam_expand_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, as_stream(stream)>>>(cam, Kh, out, n, h, w, H);
   LRPX_CHECK_LAUNCH();
   return LRPX_OK;
 }

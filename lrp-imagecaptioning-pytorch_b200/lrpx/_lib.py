@@ -85,7 +85,8 @@ class TcConvArgs(C.Structure):
                [(n, C.c_int) for n in ("a_phys", "groups", "split", "n_acc", "rule", "zbias")] + \
                [("alpha", C.c_float), ("beta", C.c_float)] + \
                [(n, _P) for n in ("add", "gain3", "gain4", "bn_w", "bn_b", "idn", "hd", "out4", "out5")] + \
-               [("add_pitch", C.c_int), ("fwd_flags", C.c_int), ("out_pitch", C.c_int), ("n_valid", C.c_int)]
+               [("add_pitch", C.c_int), ("fwd_flags", C.c_int), ("out_pitch", C.c_int), ("n_valid", C.c_int)] + \
+               [("cam_rows", _P), ("cam_kw", _P), ("cam_w", C.c_int)]
 
 
 _LL = C.c_longlong
@@ -170,6 +171,7 @@ SYMBOLS = {
     "lrpx_adaptive_decoder_grad_f32": (_i, [C.POINTER(AdaptiveGradArgs), _P, _sz, _P]),
     "lrpx_grad_cam_f32": (_i, [_P, _P, _P, _P, _i, _i, _i, _P]),
     "lrpx_cam_expand_mul_f32": (_i, [_P, _P, _P, _P, _P, _i, _i, _i, _i, _i, _i, _P]),
+    "lrpx_cam_expand_rows_f32": (_i, [_P, _P, _P, _i, _i, _i, _i, _P]),
     "lrpx_aoa_decoder_workspace_bytes": (_sz, [C.POINTER(AoaArgs)]),
     "lrpx_aoa_decoder_lrp_f32": (_i, [C.POINTER(AoaArgs), _P, _sz, _P]),
     "lrpx_adaptive_decoder_workspace_bytes": (_sz, [C.POINTER(AdaptiveArgs)]),

@@ -22,7 +22,10 @@ from . import ops
 class AblationExperiments:
     def __init__(self, explainer, num_delete_patches=20, patch_size=8, num_delete_words=3, chunk=128):
         """explainer: ExplainGridTDAttention / ExplainAOAAttention / ExplainAdaptiveAttention with precision='bf16'
-        (VGG encoder on the tensor-core engine).  Defaults: evaluation.py:55-56, :241."""
+        (VGG encoder on the tensor-core engine).  Defaults: evaluation.py:55-56, :241.
+        The heat-maps come from the caller, typically ``lrpx.pipeline.BatchExplainer(...).explain`` or ``explain_images``
+        of any image-resolution method: LRP, the gradient, guided backpropagation or Guided Grad-CAM (its maps have the
+        same (Q,3,H,W) shape and delivery formats).  Grad-CAM's (Q, P) maps of the encoder output are not image-sized."""
         if not getattr(explainer, "uses_tc", False):
             raise ValueError("AblationExperiments drives the tensor-core encoder: it needs a VGG-style encoder and "
                              "precision='fp32' or 'bf16'")

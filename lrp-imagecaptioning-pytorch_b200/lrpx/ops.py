@@ -532,16 +532,19 @@ def adaptive_decoder_grad(state: dict, weights: dict, req_img, req_t, req_word, 
         dict(req_img=req_img, req_t=req_t, req_word=req_word), want_raw, "d_feat")
 
 
-def grad_cam(feat, grads, req_img=None):
+def grad_cam(feat, grads, req_img=None, out=None):
     """grad_cam (gridTDmodel.py:1760-1771) for Q requests: feat (B,P,C) encoder output, grads (Q,P,C) its gradient,
-    both pixel-major; req_img (Q,) int32 or None (identity).  Returns (Q,P) maps in [0, 1]."""
+    both pixel-major; req_img (Q,) int32 or None (identity).  Returns (Q,P) maps in [0, 1] (in ``out`` when given)."""
     feat, grads = _f32(feat, "feat"), _f32(grads, "grads")
     Q, P, Cc = grads.shape
     if req_img is not None:
         req_img = req_img.to(device=feat.device, dtype=torch.int32).contiguous()
     elif Q != feat.shape[0]:
         raise _lib.LrpxError("grad_cam: req_img is required when requests and images differ in number")
-    out = torch.empty(Q, P, device=feat.device, dtype=torch.float32)
+    if out is None:
+        out = torch.empty(Q, P, device=feat.device, dtype=torch.float32)
+    elif tuple(out.shape) != (Q, P) or out.dtype != torch.float32 or not out.is_contiguous():
+        raise _lib.LrpxError(f"grad_cam: out must be a contiguous fp32 ({Q}, {P}) tensor")
     check(lib().lrpx_grad_cam_f32(_ptr(feat), _ptr(grads), _ptr(req_img), _ptr(out), Q, P, Cc, _stream()),
           "lrpx_grad_cam_f32")
     return out
@@ -558,6 +561,20 @@ def cam_expand_mul(g, cam, Kh, Kw, out=None):
     out = torch.empty_like(g) if out is None else out
     check(lib().lrpx_cam_expand_mul_f32(_ptr(g), _ptr(cam), _ptr(Kh), _ptr(Kw), _ptr(out), Q, Cc, h, w, H, W, _stream()),
           "lrpx_cam_expand_mul_f32")
+    return out
+
+
+def cam_expand_rows(cam, Kh):
+    """The y half of cam_expand_mul's expansion: (Q,H,w) = Kh (H,h) @ cam (Q,h,w), in its fmaf order.  With the x half
+    (Kw) it is the Guided Grad-CAM factor the tensor-core chain applies in its last epilogue (TcVggEngine.relevance's
+    ``cam``)."""
+    cam, Kh = _f32(cam, "cam"), _f32(Kh, "Kh")
+    Q, h, w = cam.shape
+    H = Kh.shape[0]
+    if Kh.shape[1] != h:
+        raise _lib.LrpxError("cam_expand_rows: shapes do not match")
+    out = torch.empty(Q, H, w, device=cam.device, dtype=torch.float32)
+    check(lib().lrpx_cam_expand_rows_f32(_ptr(cam), _ptr(Kh), _ptr(out), Q, h, w, H, _stream()), "lrpx_cam_expand_rows_f32")
     return out
 
 

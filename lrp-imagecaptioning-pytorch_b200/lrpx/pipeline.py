@@ -15,7 +15,7 @@ from dataclasses import dataclass
 
 import torch
 
-from . import _graph
+from . import _graph, ops
 
 
 @dataclass
@@ -36,19 +36,27 @@ class BatchExplainer:
     def __init__(self, explainer, chunk=128, use_graph=False, tc_gemm=None, head_idx=0, deliver="full"):
         """explainer: models.gridTDmodel.ExplainGridTDAttention, models.aoamodel.ExplainAOAAttention or
         models.adaptiveattention.ExplainAdaptiveAttention on a VGG encoder with precision 'fp32' (fp32-accurate chain),
-        'bf16' or 'mixed', or on a Bottleneck-ResNet encoder with precision 'bf16' or 'mixed'; ``head_idx``: the attention head an AoA explanation follows (aoamodel.py:1165,
-        ``explain_caption(img, head_idx)``); ``deliver``: format of the heat-maps (TcVggEngine.heat_shape): 'full' =
-        fp32 (Q,3,H,W) like the reference, 'channel_mean' = fp32 (Q,H,W), 'fp16'; ``tc_gemm``: decoder GEMMs as bf16x3
-        on tensor cores (default: with precision 'bf16') or on fp32 CUDA cores."""
+        'bf16' or 'mixed', or on a Bottleneck-ResNet encoder with precision 'bf16' or 'mixed'; or one of their
+        gradient-family twins (models/_gradient.py: gradient, guided backpropagation, Grad-CAM, Guided Grad-CAM; on a
+        ResNet in 'bf16' / 'mixed' only Grad-CAM).  ``head_idx``: the attention head an AoA explanation follows
+        (aoamodel.py:1165, ``explain_caption(img, head_idx)``); ``deliver``: format of the heat-maps
+        (TcVggEngine.heat_shape): 'full' = fp32 (Q,3,H,W) like the reference, 'channel_mean' = fp32 (Q,H,W), 'fp16';
+        ``tc_gemm``: decoder GEMMs as bf16x3 on tensor cores (default: with precision 'bf16') or on fp32 CUDA cores.
+        Grad-CAM classes explain with their (Q, P) maps of the encoder output (what explain_cnn returns per word; the
+        encoder chain does not run), so they take deliver='full' only.  Guided Grad-CAM runs the guided chain with the
+        expanded Grad-CAM map applied in its last layer's epilogue, in every delivery format."""
         if not getattr(explainer, "uses_tc", False):
             raise ValueError("BatchExplainer drives the tensor-core chain: it needs a VGG-style encoder with "
                              "precision 'fp32', 'bf16' or 'mixed', or a Bottleneck ResNet with 'bf16' or 'mixed'")
         self.ex = explainer
         # gradient-family explainers (models/_gradient.py): same pipeline, the decoder-gradient kernels and the chain's
-        # 'gradient' / 'guided' rule instead of the relevance ones
+        # 'gradient' / 'guided' rule instead of the relevance ones; CAM = 'cam' (Grad-CAM) | 'guided' (Guided Grad-CAM)
         self.is_gradient = explainer.GRADIENT
-        if self.is_gradient and explainer.CAM:
-            raise ValueError("BatchExplainer covers the gradient and guided-backpropagation explainers, not the CAM variants")
+        self.cam = explainer.CAM if self.is_gradient else None
+        if self.cam == "cam" and deliver != "full":
+            raise ValueError("Grad-CAM explains with (Q, P) maps of the encoder output: they have no channels to reduce "
+                             "or store in another format, use deliver='full'")
+        self._cam_px = {}         # Grad-CAM: feature-map pixels P by image size (H, W)
         self.eng = self.W = None
         self._dec_ws = {}         # persistent decoder workspaces holding the prepared copies of self.W (ops._decoder_workspace)
         self._graphs = {}
@@ -88,19 +96,34 @@ class BatchExplainer:
         return req_img, req_t
 
     def _run(self, imgs, tokens, req_img, req_t, heat, host=None):
+        """-> (r_words, the Guided Grad-CAM operands the launches read: they must outlive a graph capturing them)"""
         est = self.eng.forward(imgs)
-        return self._explain_encoded(est, self.eng.features(est, "pixel"), tokens, req_img, req_t, heat, host)[0]
+        r_words, _, cam = self._explain_encoded(est, self.eng.features(est, "pixel"), tokens, req_img, req_t, heat, host)
+        return r_words, cam
 
     def _explain_encoded(self, est, feat, tokens, req_img, req_t, heat, host=None):
         """Everything after the encoder forward: explainer forward on ``feat`` (the pixel-major features of the encoder
-        state ``est``), decoder kernels, relevance chain into ``heat``.  -> (r_words, the explainer forward's logits)."""
+        state ``est``), decoder kernels, relevance chain (or Grad-CAM maps) into ``heat``.  -> (r_words, the explainer
+        forward's logits, Guided Grad-CAM's (maps, T, Kh, Kw) or None)."""
         st = self.ex.explainer_forward(feat, tokens)
         req_word = tokens[req_img.long(), req_t.long() + 1].to(torch.int32)       # the word each request explains
         # on the explainer's cached decoder weights: the self.W of the last _sync_weights
         r_feat, r_words = self.ex._decode(st, req_img, req_t, req_word, self.tc_gemm, self.head_idx, self._dec_ws)
+        cam = None
+        if self.cam == "cam":                                  # explain_cnn's (Q, P) maps: no encoder chain
+            ops.grad_cam(st["feat"], r_feat, req_img, out=heat)
+        elif self.cam == "guided":
+            # the map expanded along y here; along x, and the product, in the first layer's epilogue of the guided chain
+            fh, fw = est.feat_hw
+            maps = ops.grad_cam(st["feat"], r_feat, req_img).view(-1, fh, fw)
+            Kh, Kw = self.ex._expand_ops(fh, fw, int(est.x.shape[2]), int(est.x.shape[3]))
+            cam = (maps, ops.cam_expand_rows(maps, Kh), Kh, Kw)
+        chain = self.cam != "cam"
+        fused = {} if cam is None else dict(cam=(cam[1], cam[3]))     # (TcResNetEngine has no CAM factor)
         if host is None:
-            self.eng.relevance(est, r_feat, req_img, chunk=self.chunk, out=heat, deliver=self.deliver)
-            return r_words, st["pred"]
+            if chain:
+                self.eng.relevance(est, r_feat, req_img, chunk=self.chunk, out=heat, deliver=self.deliver, **fused)
+            return r_words, st["pred"], cam
         # results go to pinned host buffers: the copy of chunk i runs on a side stream under the kernels of chunk i+1
         host_heat, host_words = host
         main = torch.cuda.current_stream()
@@ -118,9 +141,13 @@ class BatchExplainer:
         side.wait_stream(main)
         with torch.cuda.stream(side):
             host_words.copy_(r_words, non_blocking=True)
-        self.eng.relevance(est, r_feat, req_img, chunk=self.chunk, out=heat, on_chunk=on_chunk, deliver=self.deliver)
+            if not chain:
+                host_heat.copy_(heat, non_blocking=True)
+        if chain:
+            self.eng.relevance(est, r_feat, req_img, chunk=self.chunk, out=heat, on_chunk=on_chunk, deliver=self.deliver,
+                               **fused)
         main.wait_stream(side)
-        return r_words, st["pred"]
+        return r_words, st["pred"], cam
 
     def explain(self, imgs, tokens, out=None, host_out=None, words_per_image=None):
         """imgs (B,3,H,W) fp32 (CUDA, or pinned host memory), tokens (B,T+1) long with column 0 = <start>.
@@ -142,7 +169,7 @@ class BatchExplainer:
             imgs, tokens = imgs.to(dev, non_blocking=True), tokens.to(dev, non_blocking=True)
             req_img, req_t = self._requests(B, T, dev, wpi)
             heat = out if out is not None else torch.empty(shp, device=dev, dtype=dt)
-            return heat, self._run(imgs, tokens, req_img, req_t, heat, host_out)
+            return heat, self._run(imgs, tokens, req_img, req_t, heat, host_out)[0]
         key = (tuple(imgs.shape), tuple(tokens.shape), wpi,
                None if host_out is None else (host_out[0].data_ptr(), host_out[1].data_ptr()))
         g = self._graphs.get(key)
@@ -158,9 +185,10 @@ class BatchExplainer:
             torch.cuda.synchronize()
             graph = torch.cuda.CUDAGraph()
             with _graph.capture(graph):
-                r_words = self._run(s_imgs, s_toks, req_img, req_t, heat, host_out)
-            # everything the captured kernels point at must outlive the graph (incl. the request index tensors)
-            g = self._graphs[key] = (graph, s_imgs, s_toks, heat, r_words, req_img, req_t)
+                r_words, cam = self._run(s_imgs, s_toks, req_img, req_t, heat, host_out)
+            # everything the captured kernels point at must outlive the graph (incl. the request index tensors and the
+            # Guided Grad-CAM maps and operators)
+            g = self._graphs[key] = (graph, s_imgs, s_toks, heat, r_words, req_img, req_t, cam)
         graph, s_imgs, s_toks, heat, r_words = g[:5]
         if imgs.is_cuda:
             s_imgs.copy_(imgs, non_blocking=True)
@@ -200,7 +228,7 @@ class BatchExplainer:
         start = ex.word_map['<start>']
         tokens = torch.tensor([[start] + c + [0] * (T - len(c)) for c in captions], dtype=torch.long, device=dev)
         req_img, req_t = self._requests(B, T, dev, wpi)
-        shp, dt = self._heat_shape(imgs, Q)
+        shp, dt = self._heat_shape(imgs, Q, est)
         if Q == 0:                                               # nothing to explain: explain's empty results
             heat, r_words = torch.empty(shp, device=dev, dtype=dt), torch.empty(0, T, device=dev)
             pred = torch.empty(B, T, ex.model.fc.out_features, device=dev)
@@ -210,13 +238,22 @@ class BatchExplainer:
                 raise ValueError(f"out / host_out hold fewer than the {Q} requests of {T} words found")
             heat = torch.empty(shp, device=dev, dtype=dt) if out is None else out[:Q]
             host = None if host_out is None else (host_out[0][:Q], host_out[1][:Q, :T])
-            r_words, pred = self._explain_encoded(est, feat, tokens, req_img, req_t, heat, host)
+            r_words, pred, _ = self._explain_encoded(est, feat, tokens, req_img, req_t, heat, host)
         return ImageExplanation(captions, tokens, wpi, req_img, req_t, heat, r_words, pred)
 
-    def _heat_shape(self, imgs, Q):
+    def _heat_shape(self, imgs, Q, est=None):
         """(shape, dtype) of Q heat-maps in the delivery format (the engine's image size is known after its first
-        forward; before that it is the size of these images)"""
+        forward; before that it is the size of these images).  Grad-CAM: (Q, P) with P the encoder output's pixels,
+        taken from the encoder state ``est`` of these images or, without one, from a forward of one image of this size
+        (once per size)."""
         H, W = int(imgs.shape[2]), int(imgs.shape[3])
+        if self.cam == "cam":
+            if est is not None:
+                self._cam_px[(H, W)] = est.feat_hw[0] * est.feat_hw[1]
+            elif (H, W) not in self._cam_px:
+                fh, fw = self.eng.forward(torch.zeros(1, 3, H, W, device=self.ex.device)).feat_hw
+                self._cam_px[(H, W)] = fh * fw
+            return (Q, self._cam_px[(H, W)]), torch.float32
         shp = (Q, H, W) if self.deliver == "channel_mean" else (Q, 3, H, W)
         return shp, (torch.float16 if self.deliver == "fp16" else torch.float32)
 

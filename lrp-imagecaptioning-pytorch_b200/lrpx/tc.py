@@ -47,13 +47,14 @@ def pf_rows(n, h, w):
 def tc_conv(a, wt, n_img, h, w, cin, ncol, ksize, epilogue, out, out2=None, bias=None, gain=None, row_img=None,
             pool_idx=None, x=None, gain_mode=0, gain2=None, out3=None, a_phys=0, groups=1, split=0, n_acc=0, rule=0,
             zbias=0, alpha=1.0, beta=0.0, add=None, add_pitch=0, gain3=None, gain4=None, bn_w=None, bn_b=None, idn=None,
-            hd=None, out4=None, out5=None, fwd_flags=0):
+            hd=None, out4=None, out5=None, fwd_flags=0, cam_rows=None, cam_kw=None, cam_w=0):
     """Thin wrapper of lrpx_tc_conv (all tensors preallocated by the caller)."""
     args = TcConvArgs(n_img=n_img, h=h, w=w, cin=cin, ncol=ncol, ksize=ksize, epilogue=epilogue, gain_mode=gain_mode,
                       a_phys=a_phys, groups=groups, split=split, n_acc=n_acc, rule=rule, zbias=zbias, alpha=alpha,
-                      beta=beta, add_pitch=add_pitch, fwd_flags=fwd_flags)
+                      beta=beta, add_pitch=add_pitch, fwd_flags=fwd_flags, cam_w=cam_w)
     for name, t in (("gain2", gain2), ("out3", out3), ("add", add), ("gain3", gain3), ("gain4", gain4), ("bn_w", bn_w),
-                    ("bn_b", bn_b), ("idn", idn), ("hd", hd), ("out4", out4), ("out5", out5)):
+                    ("bn_b", bn_b), ("idn", idn), ("hd", hd), ("out4", out4), ("out5", out5), ("cam_rows", cam_rows),
+                    ("cam_kw", cam_kw)):
         setattr(args, name, t.data_ptr() if t is not None else None)
     args.a, args.wt = a.data_ptr(), wt.data_ptr()
     args.bias = bias.data_ptr() if bias is not None else None
@@ -428,19 +429,24 @@ class TcVggEngine:
         return (Q, 3, H, W), (torch.float16 if deliver == "fp16" else torch.float32)
 
     def relevance(self, st: VggState, r_feat: torch.Tensor, row_img: Optional[torch.Tensor] = None,
-                  chunk: int = 128, out: Optional[torch.Tensor] = None, on_chunk=None, deliver: str = "full") -> torch.Tensor:
+                  chunk: int = 128, out: Optional[torch.Tensor] = None, on_chunk=None, deliver: str = "full",
+                  cam=None) -> torch.Tensor:
         """Image relevance for Q requests.  r_feat: fp32 (Q, h*w, C) pixel-major relevance of the encoder
         output (what the decoder kernels emit); row_img: int32 (Q,) image of each request (None = identity).
         Returns fp32 (Q, 3, H, W).  ``on_chunk(q0, q1)`` is called after the launches that produce out[q0:q1]
         have been enqueued (used to overlap the device->host copy of finished heat-maps with the next chunk).
+        ``cam=(T, Kw)`` (rule 'guided' only): Guided Grad-CAM — every request's image gradient is multiplied by its
+        expanded Grad-CAM map in the last layer's epilogue, T = ops.cam_expand_rows(cam maps, Kh) (Q, H, w) and Kw the
+        (W, w) expansion along x; the 'full' result equals ops.cam_expand_mul of the plain one bit for bit.
         = ``relevance_tail(relevance_head(...))`` per group of at most ``GROUP`` requests (the stage-1 buffers of a
         group stay within their memory budget however many requests a call brings)."""
         Q = r_feat.shape[0]
         if deliver not in self.DELIVER:
             raise _lib.LrpxError(f"deliver must be one of {sorted(self.DELIVER)}")
+        self._check_cam(cam, Q)
         if Q <= self.GROUP:
             head = self.relevance_head(st, r_feat, row_img, chunk)
-            return self.relevance_tail(st, head, out=out, on_chunk=on_chunk, deliver=deliver)
+            return self.relevance_tail(st, head, out=out, on_chunk=on_chunk, deliver=deliver, cam=cam)
         _need_cuda(r_feat, "r_feat")
         if row_img is None:
             if Q != st.n:
@@ -454,8 +460,24 @@ class TcVggEngine:
             g1 = min(Q, g0 + group)
             head = self.relevance_head(st, r_feat[g0:g1], row_img[g0:g1], chunk)
             cb = None if on_chunk is None else (lambda q0, q1, g0=g0: on_chunk(g0 + q0, g0 + q1))
-            self.relevance_tail(st, head, out=out[g0:g1], on_chunk=cb, deliver=deliver)
+            self.relevance_tail(st, head, out=out[g0:g1], on_chunk=cb, deliver=deliver,
+                                cam=None if cam is None else (cam[0][g0:g1], cam[1]))
         return out
+
+    def _check_cam(self, cam, Q):
+        """``cam=(T, Kw)`` of relevance / relevance_tail: the guided rule of the general chain, (Q, H, w) and (W, w) fp32"""
+        if cam is None:
+            return
+        if not self.general or self.rule != "guided":
+            raise _lib.LrpxError("cam= (Guided Grad-CAM's factor) needs the 'guided' rule of the general chain")
+        T, Kw = cam
+        H, W = self.convs[0].h, self.convs[0].w
+        w = Kw.shape[-1]
+        if (tuple(T.shape) != (Q, H, w) or tuple(Kw.shape) != (W, w) or T.dtype != torch.float32
+                or Kw.dtype != torch.float32 or not T.is_contiguous() or not Kw.is_contiguous()):
+            raise _lib.LrpxError(f"cam must be ((Q, H, w), (W, w)) contiguous fp32 tensors with Q={Q}, H={H}, W={W}")
+        _need_cuda(T, "cam rows")
+        _need_cuda(Kw, "cam Kw")
 
     GROUP = 2048          # requests per stage-1 group
 
@@ -537,10 +559,12 @@ class TcVggEngine:
         return dict(Q=Q, chunk=chunk, split=split, s_all=s_all, r_feat=r_feat, row_img=row_img)
 
     def relevance_tail(self, st: VggState, head: dict, out: Optional[torch.Tensor] = None, on_chunk=None,
-                       deliver: str = "full") -> torch.Tensor:
+                       deliver: str = "full", cam=None) -> torch.Tensor:
         """Stage 2 of ``relevance``: the high-resolution layers chunk by chunk, ping-ponging two buffers sized for the
-        largest layer of a chunk, so that finished heat-maps can leave for the host while the next chunk runs."""
+        largest layer of a chunk, so that finished heat-maps can leave for the host while the next chunk runs.
+        ``cam``: as in ``relevance``."""
         Q, chunk, split, s_all, r_feat, row_img = (head[k] for k in ("Q", "chunk", "split", "s_all", "r_feat", "row_img"))
+        self._check_cam(cam, Q)
         dev = r_feat.device
         fh, fw = st.feat_hw
         shp, dt = self.heat_shape(Q, deliver)
@@ -571,7 +595,9 @@ class TcVggEngine:
             c0 = self.convs[0]
             if self.general:
                 tc_conv(s, c0.w_rel3, nq, c0.h, c0.w, c0.cout * self.km, 24, 3, EPI_INPUT3, out[q0:q1], row_img=rimg,
-                        x=st.x, a_phys=c0.cout * self.rm if self.split else 0, gain_mode=dmode, rule=self.rule_id)
+                        x=st.x, a_phys=c0.cout * self.rm if self.split else 0, gain_mode=dmode, rule=self.rule_id,
+                        cam_rows=None if cam is None else cam[0][q0:q1], cam_kw=None if cam is None else cam[1],
+                        cam_w=0 if cam is None else cam[1].shape[1])
             elif c0.w_rel3 is not None:
                 tc_conv(s, c0.w_rel3, nq, c0.h, c0.w, c0.cout, 24, 3, EPI_INPUT3, out[q0:q1], row_img=rimg, x=st.x,
                         gain_mode=dmode)

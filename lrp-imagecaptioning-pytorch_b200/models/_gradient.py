@@ -98,8 +98,9 @@ class GradientFamily:
         return self._caches["grad"].get(self.model.parameters(), lambda: self._GRAD_WEIGHTS(self._state_dict()))
 
     def _check_encoder(self):
-        # Bottleneck ResNets: the fp32 CUDA-core path only (LRPtools.lrp_wrapper.encoder_gradient_simt)
-        if getattr(self, "is_resnet", False) and self.precision in ("bf16", "mixed"):
+        # Bottleneck ResNets: the fp32 CUDA-core path only (LRPtools.lrp_wrapper.encoder_gradient_simt), except for Grad-CAM,
+        # which needs the encoder's forward and no gradient chain (the tensor-core forward of lrpx.tc_resnet)
+        if getattr(self, "is_resnet", False) and self.precision in ("bf16", "mixed") and self.CAM != "cam":
             raise NotImplementedError(f"precision={self.precision!r}: on a ResNet encoder the gradient-family explainers "
                                       "support precision 'fp32' and 'simt' (the fp32 CUDA-core kernels)")
 
@@ -130,12 +131,13 @@ class GradientFamily:
         cam = ops.grad_cam(self._pix(img_feature), self._pix(grads))[0]
         return cam.view(img_feature.shape[2], img_feature.shape[3]) if self.CAM == "guided" else cam
 
-    def _expand_ops(self):
-        fh, fw = self._feat_hw
-        key = (fh, fw, self.img.shape[2], self.img.shape[3])
+    def _expand_ops(self, fh, fw, H, W):
+        """(Kh (H, fh), Kw (W, fw)): pyramid_expand of an (fh, fw) Grad-CAM map to an (H, W) image as two operators, built
+        once per size"""
+        key = (fh, fw, H, W)
         if getattr(self, "_expand_key", None) != key:
-            up = self.img.shape[2] // fh
-            if (fh * up, fw * up) != tuple(self.img.shape[2:]):
+            up = H // fh
+            if (fh * up, fw * up) != (H, W):
                 raise NotImplementedError("guided Grad-CAM needs an image size that is a multiple of the feature map's")
             to = lambda a: torch.tensor(a, dtype=torch.float32, device=self.device)
             self._expand = (to(expand_operator(fh, up)), to(expand_operator(fw, up)))
@@ -149,7 +151,7 @@ class GradientFamily:
         g = self._encoder_gradient(d_pix, rows)
         if self.CAM == "guided":
             fh, fw = self._feat_hw
-            Kh, Kw = self._expand_ops()
+            Kh, Kw = self._expand_ops(fh, fw, self.img.shape[2], self.img.shape[3])
             g = ops.cam_expand_mul(g, self._cam(d_pix, rows).view(-1, fh, fw), Kh, Kw)
         return g
 
